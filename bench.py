@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — decoded MP/s and images/s of rocJpegDecodeBatched on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one rocJpegDecodeBatched pass over one batch of synthetic JPEGs (seeded, encoded
 here at quality 90 — rocjpeg_b200/datagen.py). Default workload = BASELINE.json configs[2]
@@ -22,6 +22,8 @@ Our arm prints ONE JSON line:
                this box's host cores — the baseline BASELINE.json prescribes, because the
                reference has no CPU decode path (src/rocjpeg_decoder.cpp:87-88)
 `--impl reference` times that CPU baseline alone and prints it in the same shape.
+`--dump-outputs DIR` writes the pixels the last timed step of `value` decoded (the inputs are seeded: the same arguments
+decode the same files), so that two builds can be compared output for output.
 Multi-GPU: one process per GPU (torchrun), every rank decodes its own full batch (weak
 scaling, images are independent — no data-path collective); time = max over ranks.
 """
@@ -38,6 +40,7 @@ sys.path.insert(0, ROOT)
 
 METRIC = "decoded_MP_per_s_rocJpegDecodeBatched"
 UNIT = "MP/s"
+DUMP_BYTES = 56 << 20   # float32 pixels of --dump-outputs: with the row indices and the .npy headers the files stay under 64 MB
 WORKLOAD_DESC = {
     "c2": "single 1920x1080 4:2:0 q90 baseline JPEG, no DRI -> RGB (BASELINE configs[1])",
     "c3": "256 x 500x375 q90 baseline JPEGs, 4:4:4/4:2:2/4:2:0 round-robin, no DRI -> RGB_PLANAR (BASELINE configs[2])",
@@ -203,6 +206,38 @@ def run_cpu_baseline(datas, fmt, budget_s=12.0, threads=None):
     return mp * passes / el / 1e6, len(datas) * passes / el, threads, sample
 
 
+def sample_outputs(torch, keep):
+    """The valid rows x bytes of every output channel of every picture, copied to the host as uint8: (name, pixels, rows kept).
+    When the batch holds more than DUMP_BYTES / 4 samples, each channel keeps the same share of its rows, chosen by a fixed
+    seed (rows kept = their indices, else None): the same arguments give the same rows, so two builds of the library can be
+    compared output for output."""
+    import numpy as np
+
+    total = sum(rows * rb for _, _, chans in keep for rows, rb in chans)
+    share = min(1.0, DUMP_BYTES / 4 / total)
+    rng = np.random.default_rng(0)
+    out = []
+    for i, (bufs, pitches, chans) in enumerate(keep):
+        for c, (b, p, (rows, rb)) in enumerate(zip(bufs, pitches, chans)):
+            plane, kept = b[:rows * p].view(rows, p)[:, :rb], None
+            if share < 1.0:
+                kept = np.sort(rng.choice(rows, max(1, int(rows * share)), replace=False))
+                plane = plane[torch.from_numpy(kept).to(plane.device)]
+            out.append((f"image{i:04d}_ch{c}", plane.cpu().numpy(), kept))
+    return out
+
+
+def write_outputs(path, arrays):
+    """<name>.npy = the pixels; where rows were sampled, <name>_rows.npy = the index of each of them in the channel."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, a, kept in arrays:
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float32))
+        if kept is not None:
+            np.save(os.path.join(path, name + "_rows.npy"), kept.astype(np.float32))
+
+
 def measure_inlib(api, torch, workload, args, ndev, dev0, ready):
     """One parse + rocJpegDecodeBatched per step, sharded by the library over `ndev` GPUs (ROCJPEG_B200_DEVICES); see main().
     `ready` = the already built single-GPU objects of the same workload (or None: build them, incl. the 1-GPU time)."""
@@ -306,7 +341,13 @@ def main():
                          "(ROCJPEG_B200_DEVICES); reported under `inlib` (under torchrun rank 0 does this with all N GPUs)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: every rank decodes a full batch; strong: one batch sharded over the ranks by scan bytes")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the pixels the last timed step decoded to DIR/image<i>_ch<c>.npy (float32, "
+                         f"rank 0; where the whole batch would take more than {DUMP_BYTES >> 20} MiB, a seeded sample of rows, "
+                         "whose indices go to image<i>_ch<c>_rows.npy)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path decodes; the reference arm has no such outputs")
     if args.warmup < 3:
         sys.stderr.write(f"bench.py: --warmup {args.warmup} is below the 3 warm-up steps the timing rules require; using 3\n")
         args.warmup = 3
@@ -387,7 +428,7 @@ def main():
         if fmt == "yuv_planar" and css in ("422", "420"):
             pitches[2] = pitches[1]
         bufs = [torch.empty(rows * p + 64, dtype=torch.uint8, device="cuda") for (rows, _), p in zip(chans, pitches)]
-        keep.append(bufs)
+        keep.append((bufs, pitches, chans))
         dests.append([(b.data_ptr(), p) for b, p in zip(bufs, pitches)])
     params = api.make_params(fmt)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
@@ -421,6 +462,7 @@ def main():
         launches += st.kernel_launches
     barrier()
     resident_wall = time.perf_counter() - wall0
+    dumped = sample_outputs(torch, keep) if args.dump_outputs and rank == 0 else None
     resident_ms = sum(step_ms) / len(step_ms)
     stats = dec.stats()
     # per-stage device times for the roofline: the same resident batch on ONE pipeline lane, so that the
@@ -580,7 +622,7 @@ def main():
     achieved = stage_bytes[dom] / dom_ms / 1e6 if dom_ms > 0 else 0.0
     k1_ms = stage_ms[2] + stage_ms[3]
     line = {
-        "metric": METRIC, "value": round(value, 1), "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
+        "metric": METRIC, "value": round(value, 1), "unit": UNIT, "n_gpus": world, "steps": len(step_ms), "warmup": args.warmup,
         "ms_per_step": round(resident_ms, 4), "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None,
         "dtype": "u8 / int16 coefficients / int32 IDCT / fp32 colour", "data": "synthetic", "config": config,
         "images_per_s": round(images_total / (resident_ms / 1e3), 1),
@@ -631,6 +673,8 @@ def main():
         mps, ips, threads, sample = run_cpu_baseline(datas, fmt, args.cpu_budget)
         line["cpu_baseline"] = {"value": round(mps, 2), "unit": UNIT, "images_per_s": round(ips, 1), "cores": threads, "kind": "port",
                                 "sample": sample, "host_cpus": os.cpu_count()}
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     print(json.dumps(line))
     rdist.finalize()
 
