@@ -10,6 +10,7 @@
  *   - a split prepare/run form of rocJpegDecodeBatched (api/rocjpeg.h:331) so the
  *     device-resident throughput ("inputs already in HBM") can be timed apart
  *     from the host->device copy;
+ *   - decodes at 1/2, 1/4 and 1/8 scale (reduced-size IDCT, as libjpeg's scale_denom);
  *   - per-stage CUDA-event timings and batch statistics for the roofline report;
  *   - parser taps (host only; usable without a GPU).
  * Plain C ABI: pointers and sizes only.
@@ -68,6 +69,28 @@ RocJpegStatus rocJpegB200Prepare(RocJpegHandle handle, RocJpegStreamHandle *jpeg
                                  const RocJpegDecodeParams *decode_params, RocJpegImage *destinations);
 RocJpegStatus rocJpegB200Run(RocJpegHandle handle);
 
+/* Decode at reduced size. Denominator d in {1, 2, 4, 8} per picture: the picture is decoded with libjpeg's reduced
+ * inverse DCTs (jidctred.c; an 8x8 block becomes an (8/d)x(8/d) block), so the entropy decode is the same and the
+ * transform and everything after it do 1/d^2 of the work. The output is ceil(W/d) x ceil(H/d) luma samples (libjpeg's
+ * output_width / output_height for scale_num 1, scale_denom d); every RocJpegImage layout rule of rocJpegDecodeBatched
+ * applies to that size, and the crop rectangle is given in its coordinates. Every component is transformed at the same
+ * reduced size, so chroma keeps its coded ratio (libjpeg-turbo decodes 4:2:0 chroma with the next larger transform
+ * instead, to save upsampling; the results of the two differ in 4:2:0 chroma only). d = 1 is rocJpegDecodeBatched
+ * itself. A denominator outside {1, 2, 4, 8} returns ROCJPEG_STATUS_INVALID_PARAMETER. RocJpegDecodeParams'
+ * target_dimension keeps the meaning it has for rocJpegDecodeBatched (none).
+ *   rocJpegB200GetScaledImageInfo: the sizes a decode at 1/scale_denom writes (the rocJpegGetImageInfo rules applied to
+ *     ceil(W/d) x ceil(H/d));
+ *   rocJpegB200DecodeBatchedScaled: rocJpegDecodeBatched with one denominator per picture (scale_denoms NULL: all 1);
+ *   rocJpegB200PrepareScaled: rocJpegB200Prepare with denominators; rocJpegB200Run is unchanged.
+ * After a scaled decode rocJpegB200GetPlanes returns the scaled planes: component c is (blocks_w[c] * 8/d) x
+ * (blocks_h[c] * 8/d) samples; rocJpegB200GetCoefficients is unchanged. */
+RocJpegStatus rocJpegB200GetScaledImageInfo(RocJpegHandle handle, RocJpegStreamHandle jpeg_stream_handle, int scale_denom, uint8_t *num_components,
+                                            RocJpegChromaSubsampling *subsampling, uint32_t *widths, uint32_t *heights);
+RocJpegStatus rocJpegB200DecodeBatchedScaled(RocJpegHandle handle, RocJpegStreamHandle *jpeg_stream_handles, int batch_size,
+                                             const RocJpegDecodeParams *decode_params, const int32_t *scale_denoms, RocJpegImage *destinations);
+RocJpegStatus rocJpegB200PrepareScaled(RocJpegHandle handle, RocJpegStreamHandle *jpeg_stream_handles, int batch_size,
+                                       const RocJpegDecodeParams *decode_params, const int32_t *scale_denoms, RocJpegImage *destinations);
+
 /* Timing-harness helper: exactly the caller's loop of the reference's batched sample - rocJpegStreamParse(datas[i],
  * lengths[i], handles[i]) for every image, then one rocJpegDecodeBatched - issued from C. *parse_seconds (optional) = wall
  * time of the parse loop. */
@@ -87,7 +110,8 @@ RocJpegStatus rocJpegB200StreamLoadFiles(RocJpegStreamHandle *jpeg_stream_handle
                                          int io_threads, RocJpegStatus *per_file_status);
 
 /* Stage taps for image `index` of the last decoded batch. Layout = the oracle's: component-major,
- * each component an MCU-padded raster of blocks (64 int16, natural order) / samples (u8). */
+ * each component an MCU-padded raster of blocks (64 int16, natural order) / samples (u8; at scale 1/d
+ * (8/d)x(8/d) samples per block, see rocJpegB200DecodeBatchedScaled). */
 RocJpegStatus rocJpegB200GetCoefficients(RocJpegHandle handle, int index, int16_t *host_out, size_t count);
 RocJpegStatus rocJpegB200GetPlanes(RocJpegHandle handle, int index, uint8_t *host_out, size_t count);
 

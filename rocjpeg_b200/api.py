@@ -101,7 +101,9 @@ EXT_EXPORTS = (
     "rocJpegB200PlanShards", "rocJpegB200GetDeviceCount", "rocJpegB200StreamHostScan",
     "rocJpegB200GetScanStatus", "rocJpegB200GetDeviceSegment", "rocJpegB200ParseAndDecodeBatched",
     "rocJpegB200PlanShardsPinned", "rocJpegB200GetImageStatus", "rocJpegB200StreamLoadFiles",
+    "rocJpegB200GetScaledImageInfo", "rocJpegB200DecodeBatchedScaled", "rocJpegB200PrepareScaled",
 )
+SCALES = (1, 2, 4, 8)   # denominators of the reduced-size decodes
 
 _lib = None
 
@@ -137,6 +139,9 @@ def load_library() -> C.CDLL:
     L.rocJpegB200GetStats.argtypes = [vp, C.POINTER(Stats)]
     L.rocJpegB200Prepare.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(RocJpegDecodeParams), C.POINTER(RocJpegImage)]
     L.rocJpegB200Run.argtypes = [vp]
+    L.rocJpegB200GetScaledImageInfo.argtypes = [vp, vp, i32, C.POINTER(C.c_uint8), C.POINTER(i32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]
+    L.rocJpegB200DecodeBatchedScaled.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(RocJpegDecodeParams), C.POINTER(C.c_int32), C.POINTER(RocJpegImage)]
+    L.rocJpegB200PrepareScaled.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(RocJpegDecodeParams), C.POINTER(C.c_int32), C.POINTER(RocJpegImage)]
     L.rocJpegB200GetCoefficients.argtypes = [vp, i32, vp, C.c_size_t]
     L.rocJpegB200GetPlanes.argtypes = [vp, i32, vp, C.c_size_t]
     L.rocJpegB200StreamGetInfo.argtypes = [vp, C.POINTER(StreamInfo)]
@@ -318,6 +323,25 @@ class Decoder:
         _check(self.lib.rocJpegGetImageInfo(self.handle, stream.handle, C.byref(n), C.byref(css), w, h), "rocJpegGetImageInfo")
         return n.value, css.value, list(w), list(h)
 
+    def scaled_image_info(self, stream: JpegStream, scale_denom: int):
+        """rocJpegB200GetScaledImageInfo: (num_components, subsampling, widths, heights) of a decode at 1/scale_denom."""
+        n = C.c_uint8()
+        css = C.c_int()
+        w = (C.c_uint32 * 4)()
+        h = (C.c_uint32 * 4)()
+        _check(self.lib.rocJpegB200GetScaledImageInfo(self.handle, stream.handle, scale_denom, C.byref(n), C.byref(css), w, h),
+               "rocJpegB200GetScaledImageInfo")
+        return n.value, css.value, list(w), list(h)
+
+    @staticmethod
+    def _scales(scales, n):
+        """int32 array of denominators (a ready ctypes array passes through), or None (all 1)."""
+        if scales is None or isinstance(scales, C.Array):
+            return scales
+        if len(scales) != n:
+            raise ValueError(f"{len(scales)} scale denominators for {n} pictures")
+        return (C.c_int32 * n)(*[int(d) for d in scales])
+
     @staticmethod
     def _images(dests):
         arr = (RocJpegImage * len(dests))()
@@ -342,6 +366,12 @@ class Decoder:
         hs, imgs, n, _ = streams if dests is None else self.make_batch(streams, dests)
         return self.lib.rocJpegDecodeBatched(self.handle, hs, n, C.byref(params), imgs)
 
+    def decode_batched_scaled(self, streams, params: RocJpegDecodeParams, dests, scales) -> int:
+        """rocJpegB200DecodeBatchedScaled: picture i decoded at 1/scales[i] (scales None: all full size). dests and the crop
+        rectangle are in scaled units (scaled_image_info). Returns RocJpegStatus."""
+        hs, imgs, n, _ = streams if dests is None else self.make_batch(streams, dests)
+        return self.lib.rocJpegB200DecodeBatchedScaled(self.handle, hs, n, C.byref(params), self._scales(scales, n), imgs)
+
     def make_sources(self, addresses, lengths):
         """Argument arrays (data pointers, lengths) for parse_and_decode_batched."""
         n = len(addresses)
@@ -357,10 +387,13 @@ class Decoder:
         return st, sec.value
 
     # ---- extension taps -------------------------------------------------
-    def prepare(self, streams, params, dests) -> int:
+    def prepare(self, streams, params, dests, scales=None) -> int:
+        """rocJpegB200Prepare, or rocJpegB200PrepareScaled when `scales` (one denominator per picture) is given."""
         hs = (C.c_void_p * len(streams))(*[s.handle for s in streams])
         imgs = self._images(dests)
-        return self.lib.rocJpegB200Prepare(self.handle, hs, len(streams), C.byref(params), imgs)
+        if scales is None:
+            return self.lib.rocJpegB200Prepare(self.handle, hs, len(streams), C.byref(params), imgs)
+        return self.lib.rocJpegB200PrepareScaled(self.handle, hs, len(streams), C.byref(params), self._scales(scales, len(streams)), imgs)
 
     def run(self) -> int:
         return self.lib.rocJpegB200Run(self.handle)

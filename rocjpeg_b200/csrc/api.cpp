@@ -49,7 +49,21 @@ inline rjb::DecodeParams ToParams(const RocJpegDecodeParams* p) {
     return d;
 }
 
-static_assert(sizeof(rjb::DestImage) == sizeof(RocJpegImage), "RocJpegImage layout");
+// The decoder's destinations: the caller's RocJpegImage plus the picture's scale denominator (scale_denoms NULL: all 1).
+// INVALID_PARAMETER for a denominator other than 1, 2, 4 or 8.
+int ToDests(const RocJpegImage* images, int n, const int32_t* scale_denoms, std::vector<rjb::DestImage>* out) {
+    out->resize(size_t(n));
+    for (int i = 0; i < n; i++) {
+        rjb::DestImage& d = (*out)[size_t(i)];
+        for (int c = 0; c < 4; c++) {
+            d.channel[c] = images[i].channel[c];
+            d.pitch[c] = images[i].pitch[c];
+        }
+        d.scale_denom = scale_denoms ? scale_denoms[i] : 1;
+        if (!rjb::ValidScale(d.scale_denom)) return ROCJPEG_STATUS_INVALID_PARAMETER;
+    }
+    return ROCJPEG_STATUS_SUCCESS;
+}
 static_assert(ROCJPEG_B200_STAGE_COUNT == rjb::kStageCount, "stage count");
 
 int CollectStreams(RocJpegStreamHandle* handles, int n, std::vector<const rjb::StreamParser*>* out) {
@@ -149,6 +163,25 @@ RocJpegStatus ROCJPEGAPI rocJpegGetImageInfo(RocJpegHandle handle, RocJpegStream
     }
 }
 
+RocJpegStatus rocJpegB200GetScaledImageInfo(RocJpegHandle handle, RocJpegStreamHandle jpeg_stream_handle, int scale_denom, uint8_t* num_components,
+                                            RocJpegChromaSubsampling* subsampling, uint32_t* widths, uint32_t* heights) {
+    if (handle == nullptr || jpeg_stream_handle == nullptr || num_components == nullptr || subsampling == nullptr || widths == nullptr ||
+        heights == nullptr || !rjb::ValidScale(scale_denom))
+        return ROCJPEG_STATUS_INVALID_PARAMETER;
+    auto h = static_cast<DecoderHandle*>(handle);
+    try {
+        int32_t css = 0;
+        int st = h->decoder->GetImageInfo(static_cast<StreamHandle*>(jpeg_stream_handle)->parser.get(), num_components, &css, widths, heights,
+                                          scale_denom);
+        *subsampling = RocJpegChromaSubsampling(css);
+        return RocJpegStatus(st);
+    } catch (const std::exception& e) {
+        h->CaptureError(e.what());
+        ERR(e.what());
+        return ROCJPEG_STATUS_RUNTIME_ERROR;
+    }
+}
+
 RocJpegStatus ROCJPEGAPI rocJpegDecode(RocJpegHandle handle, RocJpegStreamHandle jpeg_stream_handle, const RocJpegDecodeParams* decode_params,
                                        RocJpegImage* destination) {
     if (handle == nullptr || decode_params == nullptr || destination == nullptr) return ROCJPEG_STATUS_INVALID_PARAMETER;
@@ -156,7 +189,9 @@ RocJpegStatus ROCJPEGAPI rocJpegDecode(RocJpegHandle handle, RocJpegStreamHandle
     auto h = static_cast<DecoderHandle*>(handle);
     try {
         const rjb::StreamParser* s = static_cast<StreamHandle*>(jpeg_stream_handle)->parser.get();
-        int st = h->decoder->Decode(&s, 1, ToParams(decode_params), reinterpret_cast<const rjb::DestImage*>(destination));
+        std::vector<rjb::DestImage> dsts;
+        ToDests(destination, 1, nullptr, &dsts);
+        int st = h->decoder->Decode(&s, 1, ToParams(decode_params), dsts.data());
         if (st != 0) h->CaptureError(h->decoder->last_error());
         return RocJpegStatus(st);
     } catch (const std::exception& e) {
@@ -168,6 +203,11 @@ RocJpegStatus ROCJPEGAPI rocJpegDecode(RocJpegHandle handle, RocJpegStreamHandle
 
 RocJpegStatus ROCJPEGAPI rocJpegDecodeBatched(RocJpegHandle handle, RocJpegStreamHandle* jpeg_stream_handles, int batch_size,
                                               const RocJpegDecodeParams* decode_params, RocJpegImage* destinations) {
+    return rocJpegB200DecodeBatchedScaled(handle, jpeg_stream_handles, batch_size, decode_params, nullptr, destinations);
+}
+
+RocJpegStatus rocJpegB200DecodeBatchedScaled(RocJpegHandle handle, RocJpegStreamHandle* jpeg_stream_handles, int batch_size,
+                                             const RocJpegDecodeParams* decode_params, const int32_t* scale_denoms, RocJpegImage* destinations) {
     if (handle == nullptr || jpeg_stream_handles == nullptr || decode_params == nullptr || destinations == nullptr)
         return ROCJPEG_STATUS_INVALID_PARAMETER;
     auto h = static_cast<DecoderHandle*>(handle);
@@ -176,7 +216,10 @@ RocJpegStatus ROCJPEGAPI rocJpegDecodeBatched(RocJpegHandle handle, RocJpegStrea
         std::vector<const rjb::StreamParser*> streams;
         int st = CollectStreams(jpeg_stream_handles, batch_size, &streams);
         if (st != 0) return RocJpegStatus(st);
-        st = h->decoder->Decode(streams.data(), batch_size, ToParams(decode_params), reinterpret_cast<const rjb::DestImage*>(destinations));
+        std::vector<rjb::DestImage> dsts;
+        st = ToDests(destinations, batch_size, scale_denoms, &dsts);
+        if (st != 0) return RocJpegStatus(st);
+        st = h->decoder->Decode(streams.data(), batch_size, ToParams(decode_params), dsts.data());
         if (st != 0) h->CaptureError(h->decoder->last_error());
         return RocJpegStatus(st);
     } catch (const std::exception& e) {
@@ -243,6 +286,11 @@ RocJpegStatus rocJpegB200GetStats(RocJpegHandle handle, RocJpegB200Stats* stats)
 
 RocJpegStatus rocJpegB200Prepare(RocJpegHandle handle, RocJpegStreamHandle* jpeg_stream_handles, int batch_size,
                                  const RocJpegDecodeParams* decode_params, RocJpegImage* destinations) {
+    return rocJpegB200PrepareScaled(handle, jpeg_stream_handles, batch_size, decode_params, nullptr, destinations);
+}
+
+RocJpegStatus rocJpegB200PrepareScaled(RocJpegHandle handle, RocJpegStreamHandle* jpeg_stream_handles, int batch_size,
+                                       const RocJpegDecodeParams* decode_params, const int32_t* scale_denoms, RocJpegImage* destinations) {
     if (handle == nullptr || jpeg_stream_handles == nullptr || decode_params == nullptr || destinations == nullptr || batch_size <= 0)
         return ROCJPEG_STATUS_INVALID_PARAMETER;
     auto h = static_cast<DecoderHandle*>(handle);
@@ -250,8 +298,10 @@ RocJpegStatus rocJpegB200Prepare(RocJpegHandle handle, RocJpegStreamHandle* jpeg
         std::vector<const rjb::StreamParser*> streams;
         int st = CollectStreams(jpeg_stream_handles, batch_size, &streams);
         if (st != 0) return RocJpegStatus(st);
-        return RocJpegStatus(h->decoder->Prepare(streams.data(), batch_size, ToParams(decode_params),
-                                                 reinterpret_cast<const rjb::DestImage*>(destinations)));
+        std::vector<rjb::DestImage> dsts;
+        st = ToDests(destinations, batch_size, scale_denoms, &dsts);
+        if (st != 0) return RocJpegStatus(st);
+        return RocJpegStatus(h->decoder->Prepare(streams.data(), batch_size, ToParams(decode_params), dsts.data()));
     } catch (const std::exception& e) {
         h->CaptureError(e.what());
         ERR(e.what());

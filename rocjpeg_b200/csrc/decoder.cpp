@@ -238,6 +238,7 @@ int Decoder::Initialize() {
     RJB_CUDA(PreloadK0());
     RJB_CUDA(PreloadK1());
     RJB_CUDA(PreloadK2());
+    RJB_CUDA(PreloadK2Scaled());
     RJB_CUDA(PreloadK3());
     RJB_CUDA(PreloadK23());
     for (int l = 1; l < 4; l++) {   // the lanes a call uses by default; the others (ROCJPEG_B200_LANES > 4) are created on demand
@@ -347,14 +348,15 @@ void PlanShardsPinned(const uint64_t* cost, const int* fixed, int n, int ndev, i
 }
 
 // src/rocjpeg_decoder.cpp:307-358
-int Decoder::GetImageInfo(const StreamParser* s, uint8_t* ncomp, int32_t* css, uint32_t* widths, uint32_t* heights) {
+int Decoder::GetImageInfo(const StreamParser* s, uint8_t* ncomp, int32_t* css, uint32_t* widths, uint32_t* heights, int scale_denom) {
     std::lock_guard<std::mutex> lock(mutex_);
-    if (!s || !ncomp || !css || !widths || !heights) return kInvalidParameter;
+    if (!s || !ncomp || !css || !widths || !heights || !ValidScale(scale_denom)) return kInvalidParameter;
     const ParsedJpeg& p = s->parsed();
     *ncomp = uint8_t(p.ncomp);
     *css = p.css;
-    widths[0] = uint32_t(p.width);
-    heights[0] = uint32_t(p.height);
+    // at scale 1/d the picture is ceil(W/d) x ceil(H/d) (libjpeg's output_width / output_height), the rules below apply to that
+    widths[0] = uint32_t((p.width + scale_denom - 1) / scale_denom);
+    heights[0] = uint32_t((p.height + scale_denom - 1) / scale_denom);
     widths[3] = heights[3] = 0;
     switch (p.css) {
         case CSS_444: widths[1] = widths[2] = widths[0]; heights[1] = heights[2] = heights[0]; break;
@@ -396,6 +398,8 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     h_img_dctile0_.assign(size_t(n) + 1, 0);
     h_k2_tile0_.assign(size_t(n) + 1, 0);
     h_k3_tile0_.assign(size_t(n) + 1, 0);
+    for (auto& v : h_k2s_tile0_) v.assign(size_t(n) + 1, 0);
+    h_scale_.assign(size_t(n), 1);
     h_fused_.clear();
     h_tile_img_.clear();
     h_tile_img_w_.clear();
@@ -444,6 +448,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     k2_needed_ = false;
     uint64_t scan_off = 0, raw_off = 0, blk = 0, plane_off = 0, ent = 0, sub = 0;
     uint32_t dctile = 0, k2tile = 0, k3tile = 0, max_pairs = 1, max_sub = 0, k0tile = 0, nseg_total = 0;
+    uint32_t k2stile[kScaledKernels] = {};
     all_pinned_ = true;
     // Upload plan. Streams that lie close together in ONE page-locked allocation (the caller's arena of files, or
     // the staging pool's slab) are uploaded by a single copy that takes the few bytes between them along: the copy
@@ -496,6 +501,11 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     for (int i = 0; i < n; i++) {
         const ParsedJpeg& p = streams[i]->parsed();
         ImageDesc& im = h_images_[size_t(i)];
+        // scale 1/d: the output is ceil(W/d) x ceil(H/d); crop rectangle and destinations are in those units
+        const int d = dsts[i].scale_denom;
+        if (!ValidScale(d)) return Fail(kInvalidParameter, "scale denominator must be 1, 2, 4 or 8");
+        h_scale_[size_t(i)] = d;
+        const int out_w = (p.width + d - 1) / d, out_h = (p.height + d - 1) / d;
         im.width = p.width; im.height = p.height; im.ncomp = p.ncomp; im.css = p.css;
         im.mcus_x = p.mcus_x; im.mcus_y = p.mcus_y; im.bpm = p.bpm; im.restart_interval = p.restart_interval;
         im.total_mcus = p.mcus_x * p.mcus_y;
@@ -587,9 +597,9 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
         {
             const uint32_t cw = uint32_t(int(params.crop_right) - int(params.crop_left));
             const uint32_t chh = uint32_t(int(params.crop_bottom) - int(params.crop_top));
-            if (p.restart_interval > 0 && cw > 0 && chh > 0 && cw <= uint32_t(p.width) && chh <= uint32_t(p.height) &&
-                params.crop_top >= 0 && params.crop_bottom <= p.height && im.mcus_y > 0) {
-                const int mcu_h = 8 * std::max(1, p.ncomp == 1 ? 1 : p.vmax);
+            if (p.restart_interval > 0 && cw > 0 && chh > 0 && cw <= uint32_t(out_w) && chh <= uint32_t(out_h) &&
+                params.crop_top >= 0 && params.crop_bottom <= out_h && im.mcus_y > 0) {
+                const int mcu_h = 8 * std::max(1, p.ncomp == 1 ? 1 : p.vmax) / d;   // MCU rows in output rows
                 const uint64_t row_lo = uint64_t(params.crop_top / mcu_h), row_hi = uint64_t((params.crop_bottom - 1) / mcu_h);
                 const uint64_t ri = uint64_t(p.restart_interval);
                 const uint64_t k_lo = row_lo * uint64_t(im.mcus_x) / ri, k_hi = ((row_hi + 1) * uint64_t(im.mcus_x) - 1) / ri;
@@ -612,23 +622,27 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
         h_img_dctile0_[size_t(i)] = dctile;
         dctile += uint32_t((im.total_mcus + kDcTileMcus - 1) / kDcTileMcus);
         // planes + IDCT tiles
+        // (a picture at scale 1/d has planes of (blocks_w * 8/d) x (blocks_h * 8/d) samples and its tiles in the kernel of that scale)
         h_k2_tile0_[size_t(i)] = k2tile;
+        for (int s = 0; s < kScaledKernels; s++) h_k2s_tile0_[s][size_t(i)] = k2stile[s];
+        uint32_t& idct_tiles = d == 1 ? k2tile : k2stile[ScaleIndex(d)];
+        const int bs = 8 / d;   // samples per block row and column
         for (int c = 0; c < p.ncomp; c++) {
-            im.plane_pitch[c] = uint32_t(AlignUp(size_t(p.blocks_w[c]) * 8, 64));
+            im.plane_pitch[c] = uint32_t(AlignUp(size_t(p.blocks_w[c]) * bs, 64));
             im.plane_off[c] = plane_off;
-            plane_off += AlignUp(size_t(im.plane_pitch[c]) * size_t(p.blocks_h[c]) * 8, 256);
-            k2tile += uint32_t((p.blocks_w[c] + 31) / 32) * uint32_t(p.blocks_h[c]);
-            stats_.plane_bytes += uint64_t(p.blocks_w[c]) * p.blocks_h[c] * 64;
+            plane_off += AlignUp(size_t(im.plane_pitch[c]) * size_t(p.blocks_h[c]) * bs, 256);
+            idct_tiles += uint32_t((p.blocks_w[c] + 31) / 32) * uint32_t(p.blocks_h[c]);
+            stats_.plane_bytes += uint64_t(p.blocks_w[c]) * p.blocks_h[c] * uint64_t(bs * bs);
         }
         // output job. ROI rule: src/rocjpeg_decoder.cpp:126-131 (unsigned widths).
         OutputDesc& od = h_outputs_[size_t(i)];
         const uint32_t rw = uint32_t(int(params.crop_right) - int(params.crop_left));
         const uint32_t rh = uint32_t(int(params.crop_bottom) - int(params.crop_top));
         od.x0 = od.y0 = 0;
-        od.w = p.width;
-        od.h = p.height;
-        if (rw > 0 && rh > 0 && rw <= uint32_t(p.width) && rh <= uint32_t(p.height)) {
-            if (params.crop_left < 0 || params.crop_top < 0 || params.crop_right > p.width || params.crop_bottom > p.height)
+        od.w = out_w;
+        od.h = out_h;
+        if (rw > 0 && rh > 0 && rw <= uint32_t(out_w) && rh <= uint32_t(out_h)) {
+            if (params.crop_left < 0 || params.crop_top < 0 || params.crop_right > out_w || params.crop_bottom > out_h)
                 return Fail(kInvalidParameter, "crop rectangle lies outside the picture");
             od.x0 = params.crop_left; od.y0 = params.crop_top; od.w = int32_t(rw); od.h = int32_t(rh);
         }
@@ -639,18 +653,19 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
         }
         // Planar formats without a crop need no output stage: the IDCT stage stores the planes straight
         // into the caller's channels (4:2:2 / 4:2:0 NATIVE are interleaved surfaces and keep their tiles).
-        const bool whole = od.x0 == 0 && od.y0 == 0 && od.w == p.width && od.h == p.height;
+        const bool whole = od.x0 == 0 && od.y0 == 0 && od.w == out_w && od.h == out_h;
         const bool planar = od.fmt == FMT_Y || od.fmt == FMT_YUV_PLANAR ||
                             (od.fmt == FMT_NATIVE && (p.css == CSS_444 || p.css == CSS_440 || p.css == CSS_411 || p.css == CSS_400));
         od.direct = (whole && planar && direct_ok && !(remote && remote[i])) ? 1 : 0;
         // Whole-picture RGB / RGB_PLANAR: IDCT and colour conversion in one kernel, the planes never leave shared memory
-        od.fused = (whole && fuse_ok && (od.fmt == FMT_RGB || od.fmt == FMT_RGB_PLANAR) && h_fused_.size() < 65535) ? 1 : 0;
+        // (full size only: a scaled picture goes reduced-size IDCT -> plane arena -> output stage)
+        od.fused = (d == 1 && whole && fuse_ok && (od.fmt == FMT_RGB || od.fmt == FMT_RGB_PLANAR) && h_fused_.size() < 65535) ? 1 : 0;
         const bool tiles = !od.direct && !od.fused;
         od.tiles_x = tiles ? uint32_t((od.w + kK3TileW - 1) / kK3TileW) : 0u;
         od.tiles_y = tiles ? uint32_t((od.h + kK3TileH - 1) / kK3TileH) : 0u;
         any_direct_ = any_direct_ || od.direct || od.fused || !whole;   // the plane arena is then incomplete: the tap re-runs the IDCT
         needs_planes_ = needs_planes_ || tiles;
-        k2_needed_ = k2_needed_ || !od.fused;
+        k2_needed_ = k2_needed_ || (!od.fused && d == 1);
         if (od.fused) {
             FusedImage fi = {};
             fi.ent0 = im.ent0; fi.blk0 = im.blk0; fi.ent_cap = im.ent_cap;
@@ -698,6 +713,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     h_k0_tile0_[size_t(n)] = k0tile;
     h_img_dctile0_[size_t(n)] = dctile;
     h_k2_tile0_[size_t(n)] = k2tile;
+    for (int s = 0; s < kScaledKernels; s++) h_k2s_tile0_[s][size_t(n)] = k2stile[s];
     h_k3_tile0_[size_t(n)] = k3tile;
     scan_bytes_ = scan_off;
     raw_bytes_ = raw_off;
@@ -743,6 +759,11 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     k2_ = K2Args{};
     k2_.nimages = n;
     k2_.total_tiles = k2tile;
+    for (int s = 0; s < kScaledKernels; s++) {
+        k2s_[s] = K2Args{};
+        k2s_[s].nimages = n;
+        k2s_[s].total_tiles = k2stile[s];
+    }
     k3_ = K3Args{};
     k3_.nimages = n;
     k3_.total_tiles = k3tile;
@@ -755,7 +776,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
 
 // Descriptor block: one pinned host buffer mirrored by one device buffer, one copy.
 struct Lane::Layout {
-    size_t images, outputs, cta0, k0tile0, dctile0, k2tile0, k3tile0, fused, tile_img, tile_img_w, gather, luts, qtables, total;
+    size_t images, outputs, cta0, k0tile0, dctile0, k2tile0, k2stile0[kScaledKernels], k3tile0, fused, tile_img, tile_img_w, gather, luts, qtables, total;
 };
 
 int Lane::Upload(cudaStream_t up, UploadTurn turn) {
@@ -771,6 +792,7 @@ int Lane::Upload(cudaStream_t up, UploadTurn turn) {
     L.k0tile0 = place((n + 1) * 4);
     L.dctile0 = place((n + 1) * 4);
     L.k2tile0 = place((n + 1) * 4);
+    for (int s = 0; s < kScaledKernels; s++) L.k2stile0[s] = place((n + 1) * 4);
     L.k3tile0 = place((n + 1) * 4);
     L.fused = place(h_fused_.size() * sizeof(FusedImage));
     L.tile_img = place(h_tile_img_.size() * 4);
@@ -787,6 +809,7 @@ int Lane::Upload(cudaStream_t up, UploadTurn turn) {
     std::memcpy(h + L.k0tile0, h_k0_tile0_.data(), (n + 1) * 4);
     std::memcpy(h + L.dctile0, h_img_dctile0_.data(), (n + 1) * 4);
     std::memcpy(h + L.k2tile0, h_k2_tile0_.data(), (n + 1) * 4);
+    for (int s = 0; s < kScaledKernels; s++) std::memcpy(h + L.k2stile0[s], h_k2s_tile0_[s].data(), (n + 1) * 4);
     std::memcpy(h + L.k3tile0, h_k3_tile0_.data(), (n + 1) * 4);
     std::memcpy(h + L.fused, h_fused_.data(), h_fused_.size() * sizeof(FusedImage));
     std::memcpy(h + L.tile_img, h_tile_img_.data(), h_tile_img_.size() * 4);
@@ -852,6 +875,12 @@ int Lane::Upload(cudaStream_t up, UploadTurn turn) {
     k2_.entries = k1_.entries;
     k2_.blk_rec = k1_.blk_rec;
     k2_.planes = needs_planes_ ? d_planes_.as<uint8_t>() : nullptr;
+    for (int s = 0; s < kScaledKernels; s++) {
+        const uint32_t tiles = k2s_[s].total_tiles;
+        k2s_[s] = k2_;
+        k2s_[s].img_tile0 = reinterpret_cast<const uint32_t*>(d + L.k2stile0[s]);
+        k2s_[s].total_tiles = tiles;
+    }
     k3_.images = k1_.images;
     k3_.outputs = reinterpret_cast<const OutputDesc*>(d + L.outputs);
     k3_.img_tile0 = reinterpret_cast<const uint32_t*>(d + L.k3tile0);
@@ -976,12 +1005,16 @@ int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up, Upload
     RJB_CUDA(mark(4));
     RJB_CUDA(LaunchDcScan(k1_, stream_));
     RJB_CUDA(mark(5));
-    if (k2_needed_) RJB_CUDA(LaunchK2Idct(k2_, stream_));
+    uint32_t idct_launches = 0;
+    {
+        const int st = LaunchIdct(false, &idct_launches);
+        if (st != kSuccess) return st;
+    }
     RJB_CUDA(mark(6));
     RJB_CUDA(LaunchK23Fused(k23_, stream_));
     RJB_CUDA(LaunchK3Output(k3_, stream_));
     RJB_CUDA(mark(7));
-    stats_.kernel_launches += (k1_fused ? 1u : uint32_t(rounds) + (k1_.inline_scan ? 1u : 2u)) + (k1_.dc_image ? 1 : 3) + (k2_needed_ ? 1 : 0) + (k23_.total_tiles ? 1 : 0) + (k23_.total_tiles_w ? 1 : 0) +
+    stats_.kernel_launches += (k1_fused ? 1u : uint32_t(rounds) + (k1_.inline_scan ? 1u : 2u)) + (k1_.dc_image ? 1 : 3) + idct_launches + (k23_.total_tiles ? 1 : 0) + (k23_.total_tiles_w ? 1 : 0) +
                               (k3_.total_tiles ? 1 : 0);   // sync rounds, (scan +) write, 1 or 3 DC kernels, IDCT, fused IDCT + output, output
     RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
     RJB_CUDA(cudaMemcpyAsync(h_counters_.data() + 256, k0_.status, h_images_.size() * sizeof(ScanStatus), cudaMemcpyDeviceToHost, stream_));
@@ -989,6 +1022,23 @@ int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up, Upload
     if (ev_trace_[2]) RJB_CUDA(cudaEventRecord(ev_trace_[2], stream_));
     host_ms_[2] = NowMs();
     exit_guard.ok = true;
+    return kSuccess;
+}
+
+int Lane::LaunchIdct(bool force_planes, uint32_t* launches) {
+    // (force_planes: the plane tap's re-run, which transforms every picture - fused ones included - into the arena)
+    K2Args k2 = k2_;
+    k2.force_planes = force_planes ? 1 : 0;
+    if (k2_needed_ || force_planes) {
+        RJB_CUDA(LaunchK2Idct(k2, stream_));
+        if (k2.total_tiles) (*launches)++;
+    }
+    for (int s = 0; s < kScaledKernels; s++) {
+        K2Args ks = k2s_[s];
+        ks.force_planes = k2.force_planes;
+        RJB_CUDA(LaunchK2Scaled(ks, 2 << s, stream_));
+        if (ks.total_tiles) (*launches)++;
+    }
     return kSuccess;
 }
 
@@ -1018,7 +1068,9 @@ int Lane::Finish(int profiling_) {
         RJB_CUDA(LaunchK1ClearShort(k1_, stream_));   // ... and may have reported pictures short that are not
         RJB_CUDA(LaunchK1Write(k1_, stream_));
         RJB_CUDA(LaunchDcScan(k1_, stream_));
-        if (k2_needed_) RJB_CUDA(LaunchK2Idct(k2_, stream_));
+        uint32_t idct_launches = 0;
+        const int st = LaunchIdct(false, &idct_launches);
+        if (st != kSuccess) return st;
         RJB_CUDA(LaunchK23Fused(k23_, stream_));
         RJB_CUDA(LaunchK3Output(k3_, stream_));
         RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
@@ -1117,10 +1169,13 @@ int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodePar
                 std::cerr << "[ERR]  {Decode}  The JPEG image (chroma subsampling / layout / size) is not supported!" << std::endl;
             return Fail(p.support_status, "unsupported or inconsistent JPEG");
         }
+        const int d = dsts[i].scale_denom;
+        if (!ValidScale(d)) return Fail(kInvalidParameter, "scale denominator must be 1, 2, 4 or 8");
+        const int out_w = (p.width + d - 1) / d, out_h = (p.height + d - 1) / d;   // the crop rectangle is in output units
         const uint32_t rw = uint32_t(int(params.crop_right) - int(params.crop_left));
         const uint32_t rh = uint32_t(int(params.crop_bottom) - int(params.crop_top));
-        if (rw > 0 && rh > 0 && rw <= uint32_t(p.width) && rh <= uint32_t(p.height) &&
-            (params.crop_left < 0 || params.crop_top < 0 || params.crop_right > p.width || params.crop_bottom > p.height))
+        if (rw > 0 && rh > 0 && rw <= uint32_t(out_w) && rh <= uint32_t(out_h) &&
+            (params.crop_left < 0 || params.crop_top < 0 || params.crop_right > out_w || params.crop_bottom > out_h))
             return Fail(kInvalidParameter, "crop rectangle lies outside the picture");
     }
     if (params.output_format < FMT_NATIVE || params.output_format > FMT_RGB_PLANAR)
@@ -1503,22 +1558,24 @@ int Lane::CopyCoefficients(int image, int16_t* host_out, size_t count) {
 int Lane::CopyPlanes(int image, uint8_t* host_out, size_t count) {
     if (image < 0 || size_t(image) >= h_images_.size() || !host_out) return kInvalidParameter;
     const ImageDesc& im = h_images_[size_t(image)];
+    const size_t bs = size_t(8 / h_scale_[size_t(image)]);   // samples per block row and column
     size_t need = 0;
-    for (int c = 0; c < im.ncomp; c++) need += size_t(im.blocks_w[c]) * im.blocks_h[c] * 64;
+    for (int c = 0; c < im.ncomp; c++) need += size_t(im.blocks_w[c]) * im.blocks_h[c] * bs * bs;
     if (count < need) return kInvalidParameter;
     if (any_direct_) {   // the planes of this batch went straight to the caller: produce them in the arena for the tap
         RJB_CUDA(cudaStreamSynchronize(stream_));
         RJB_CUDA(d_planes_.Reserve(plane_bytes_ + 512));
         k2_.planes = d_planes_.as<uint8_t>();
         k3_.planes = k2_.planes;
-        K2Args k2 = k2_;
-        k2.force_planes = 1;
-        RJB_CUDA(LaunchK2Idct(k2, stream_));
+        for (K2Args& k : k2s_) k.planes = k2_.planes;
+        uint32_t launches = 0;
+        const int st = LaunchIdct(true, &launches);
+        if (st != kSuccess) return st;
         RJB_CUDA(cudaStreamSynchronize(stream_));
     }
     size_t base = 0;
     for (int c = 0; c < im.ncomp; c++) {
-        const size_t w = size_t(im.blocks_w[c]) * 8, h = size_t(im.blocks_h[c]) * 8;
+        const size_t w = size_t(im.blocks_w[c]) * bs, h = size_t(im.blocks_h[c]) * bs;
         RJB_CUDA(cudaMemcpy2D(host_out + base, w, d_planes_.as<uint8_t>() + im.plane_off[c], im.plane_pitch[c], w, h,
                               cudaMemcpyDeviceToHost));
         base += w * h;

@@ -37,7 +37,11 @@ struct DecodeParams {
 struct DestImage {
     uint8_t* channel[4];
     uint32_t pitch[4];
+    int32_t scale_denom;   // 1, 2, 4 or 8: the picture is decoded at 1/scale_denom of its size (reduced-size IDCT)
 };
+constexpr int kScaledKernels = 3;   // reduced-size IDCT kernels: scale 1/2, 1/4, 1/8
+inline bool ValidScale(int d) { return d == 1 || d == 2 || d == 4 || d == 8; }
+inline int ScaleIndex(int d) { return d == 2 ? 0 : d == 4 ? 1 : 2; }   // d > 1: index of its reduced-size kernel
 
 class DeviceBuffer {
   public:
@@ -60,7 +64,7 @@ enum StageId {
     kStageSync,         // all k1_sync rounds
     kStageWrite,        // (k1_scan +) k1_write
     kStageDc,           // dc_image, or dc_sums + dc_scan + dc_apply
-    kStageIdct,         // k2_idct
+    kStageIdct,         // k2_idct and the reduced-size k2_idct_4x4 / 2x2 / 1x1
     kStageOutput,       // k3_output
     kStageCount
 };
@@ -153,6 +157,8 @@ class Lane {
   private:
     struct Layout;   // byte layout of the descriptor block
     int Fail(int status, const std::string& why);
+    // the IDCT stage: k2_idct for the full-size pictures, a reduced-size kernel per scale present; returns the launches
+    int LaunchIdct(bool force_planes, uint32_t* launches);
 
     bool created_ = false;
     std::string err_;
@@ -167,6 +173,8 @@ class Lane {
     std::vector<ImageDesc> h_images_;
     std::vector<OutputDesc> h_outputs_;
     std::vector<uint32_t> h_img_cta0_, h_img_dctile0_, h_k2_tile0_, h_k3_tile0_, h_k0_tile0_, h_needed_segments_;
+    std::vector<uint32_t> h_k2s_tile0_[kScaledKernels];   // first tile of each image in the reduced-size kernel of its scale
+    std::vector<int> h_scale_;                             // scale denominator of each image
     uint32_t truncated_images_ = 0;
     std::vector<GatherItem> h_gather_;
     struct CopyRun {
@@ -185,6 +193,7 @@ class Lane {
     K0Args k0_ = {};
     K1Args k1_ = {};
     K2Args k2_ = {};
+    K2Args k2s_[kScaledKernels] = {};   // reduced-size IDCT: the pictures of scale 1/2, 1/4, 1/8
     K3Args k3_ = {};
     K23Args k23_ = {};
     bool k2_needed_ = true;       // some image of the lane is not served by the fused kernel
@@ -222,7 +231,8 @@ class Decoder {
     Decoder(int backend, int device_id);
     ~Decoder();
     int Initialize();   // RocJpegStatus
-    int GetImageInfo(const StreamParser* s, uint8_t* ncomp, int32_t* css, uint32_t* widths, uint32_t* heights);
+    // scale_denom > 1: the sizes a decode at that scale writes (rocJpegB200GetScaledImageInfo)
+    int GetImageInfo(const StreamParser* s, uint8_t* ncomp, int32_t* css, uint32_t* widths, uint32_t* heights, int scale_denom = 1);
     int Decode(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts);
 
     // Extension entry points (include/rocjpeg_b200_ext.h)

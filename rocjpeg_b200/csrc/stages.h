@@ -6,7 +6,8 @@
 //                       handling VCN does on the slice it is given
 //   K1 (k1_huffman.cu)  the Huffman decode done by VCN fixed function in the
 //                       reference (src/rocjpeg_vaapi_decoder.cpp:677-689, 816-828)
-//   K2 (k2_idct.cu)     the dequantise + IDCT done by VCN fixed function (same call sites)
+//   K2 (k2_idct.cu)     the dequantise + IDCT done by VCN fixed function (same call sites);
+//      (k2_scaled.cu)   its reduced-size forms for decodes at 1/2, 1/4 and 1/8 scale
 //   K3 (k3_output.cu)   the post-processing kernels and copies of
 //                       src/rocjpeg_hip_kernels.cpp / src/rocjpeg_decoder.cpp:372-636
 #pragma once
@@ -163,6 +164,10 @@ struct K2Args {
     uint32_t total_tiles;
 };
 cudaError_t LaunchK2Idct(const K2Args& a, cudaStream_t stream);
+// Reduced-size IDCT (k2_scaled.cu) for the pictures decoded at scale 1 / scale_denom (2, 4 or 8): every block yields an
+// (8 / scale_denom)-sample square. Same tiles and arguments as LaunchK2Idct; planes, pitches, crop rectangle and the
+// caller's channels are in scaled units.
+cudaError_t LaunchK2Scaled(const K2Args& a, int scale_denom, cudaStream_t stream);
 
 // K2 + K3 in one kernel for whole-picture RGB / RGB_PLANAR outputs (OutputDesc::fused): coefficients in, pixels out.
 struct K23Args {
@@ -191,6 +196,7 @@ cudaError_t LaunchK3Output(const K3Args& a, cudaStream_t stream);
 // Load the stages' kernels now instead of at their first launch.
 cudaError_t PreloadK1();
 cudaError_t PreloadK2();
+cudaError_t PreloadK2Scaled();
 cudaError_t PreloadK3();
 
 }  // namespace rjb
