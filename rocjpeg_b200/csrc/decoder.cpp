@@ -829,7 +829,8 @@ int Lane::Upload(cudaStream_t up, UploadTurn turn) {
                  o_tile_carry = carve(size_t(k0_.total_tiles) * 16), o_status = carve(n * sizeof(ScanStatus)), o_entries = carve(entry_count_ * 4),
                  o_blkrec = carve(coef_blocks_ * sizeof(BlockRec)), o_nnz = carve(nsub_total_ * 4), o_state = carve(nsub_total_ * 4),
                  o_used = carve(nsub_total_ * 4), o_subseg = carve(nsub_total_ * 4), o_cta_entries = carve(size_t(k1_.total_ctas) * 4),
-                 o_cta_partial = carve(size_t(k1_.total_ctas) * 8), o_cta_carry = carve(size_t(k1_.total_ctas) * 8), o_cta_flag = carve(size_t(k1_.total_ctas) * 4 + 4),
+                 o_cta_partial = carve(size_t(k1_.total_ctas) * 8), o_cta_carry = carve(size_t(k1_.total_ctas) * 8), o_cta_flag = carve(size_t(k1_.total_ctas) * 8 + 4),
+                 o_cta_dc = carve(size_t(k1_.total_ctas) * 32),
                  o_dc_partial = carve(size_t(k1_.total_dc_tiles) * 12), o_dc_carry = carve(size_t(k1_.total_dc_tiles) * 12),
                  o_end = carve(0);
     (void)o_end;
@@ -862,6 +863,7 @@ int Lane::Upload(cudaStream_t up, UploadTurn turn) {
     k1_.dc_carry = reinterpret_cast<int3*>(base + o_dc_carry);
     k1_.cta_carry = reinterpret_cast<uint2*>(base + o_cta_carry);
     k1_.cta_flag = reinterpret_cast<uint32_t*>(base + o_cta_flag);
+    k1_.cta_dc = reinterpret_cast<int4*>(base + o_cta_dc);
     // the batch's counter set is picked at launch time (LaunchAll): the sets alternate
     k1_.entries = reinterpret_cast<uint32_t*>(base + o_entries);
     k1_.blk_rec = reinterpret_cast<BlockRec*>(base + o_blkrec);
@@ -983,7 +985,12 @@ int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up, Upload
     // k1_fused); ROCJPEG_B200_NO_K1_FUSE=1 or an explicit ROCJPEG_B200_SYNC_ROUNDS keep the separate kernels.
     const bool k1_fuse_ok = EnvInt("ROCJPEG_B200_NO_K1_FUSE", 0) == 0 && std::getenv("ROCJPEG_B200_SYNC_ROUNDS") == nullptr;
     const bool k1_fused = k1_fuse_ok && k1_.fusable && k1_.total_ctas != 0;
-    if (k1_fused) RJB_CUDA(cudaMemsetAsync(k1_.cta_flag, 0, size_t(k1_.total_ctas) * 4 + 4, stream_));   // "published" flags of the CTAs + the ticket counter
+    // ... and, for pictures small enough for dc_image, it integrates the DC differences itself (no DC launch behind it;
+    // ROCJPEG_B200_NO_K1_DC=1 keeps it). Not for larger ones: a CTA waits there for the picture's earlier CTAs to finish
+    // writing, and with the many CTAs of 4K pictures those waits hold SM slots the next wave needs (c4_dri 3.29 -> 3.65 ms)
+    k1_.k1_dc = k1_fused && k1_.dc_image && EnvInt("ROCJPEG_B200_NO_K1_DC", 0) == 0 ? 1 : 0;
+    // "published" flags of the CTAs, the ticket counter, the CTAs' DC flags
+    if (k1_fused) RJB_CUDA(cudaMemsetAsync(k1_.cta_flag, 0, size_t(k1_.total_ctas) * 8 + 4, stream_));
     // K0: end of slice, destuffing, restart intervals -> clean stream + segment table, all on the device
     if (!(include_upload && tiles_reduced_)) {   // cudaMemcpy upload, or a resident batch run again: the reduction is its own launch
         RJB_CUDA(LaunchK0Reduce(k0_, stream_));
@@ -1003,7 +1010,7 @@ int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up, Upload
         RJB_CUDA(LaunchK1Write(k1_, stream_));
     }
     RJB_CUDA(mark(4));
-    RJB_CUDA(LaunchDcScan(k1_, stream_));
+    if (!k1_.k1_dc) RJB_CUDA(LaunchDcScan(k1_, stream_));
     RJB_CUDA(mark(5));
     uint32_t idct_launches = 0;
     {
@@ -1014,8 +1021,9 @@ int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up, Upload
     RJB_CUDA(LaunchK23Fused(k23_, stream_));
     RJB_CUDA(LaunchK3Output(k3_, stream_));
     RJB_CUDA(mark(7));
-    stats_.kernel_launches += (k1_fused ? 1u : uint32_t(rounds) + (k1_.inline_scan ? 1u : 2u)) + (k1_.dc_image ? 1 : 3) + idct_launches + (k23_.total_tiles ? 1 : 0) + (k23_.total_tiles_w ? 1 : 0) +
-                              (k3_.total_tiles ? 1 : 0);   // sync rounds, (scan +) write, 1 or 3 DC kernels, IDCT, fused IDCT + output, output
+    stats_.kernel_launches += (k1_fused ? 1u : uint32_t(rounds) + (k1_.inline_scan ? 1u : 2u)) + (k1_.k1_dc ? 0 : k1_.dc_image ? 1 : 3) + idct_launches +
+                              (k23_.total_tiles ? 1 : 0) + (k23_.total_tiles_w ? 1 : 0) +
+                              (k3_.total_tiles ? 1 : 0);   // sync rounds, (scan +) write, 0, 1 or 3 DC kernels, IDCT, fused IDCT + output, output
     RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
     RJB_CUDA(cudaMemcpyAsync(h_counters_.data() + 256, k0_.status, h_images_.size() * sizeof(ScanStatus), cudaMemcpyDeviceToHost, stream_));
     stats_.d2h_bytes = 256 + h_images_.size() * sizeof(ScanStatus);

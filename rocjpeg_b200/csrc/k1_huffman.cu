@@ -37,6 +37,8 @@
 //                     32-bit (int16 value, zig-zag index) entry per symbol with
 //                     magnitude bits, eight per 256-bit store) and one 8-byte record
 //                     per block {where its entries end, DC difference}.
+//   k1_fused          counting and write pass in one kernel; for pictures dc_image would take, each CTA then also
+//                     integrates the DC of its share of the picture's blocks (IntegrateDc) and no DC kernel runs.
 //   dc_image          pictures up to a few thousand MCUs: per-component, per-restart-
 //                     interval prefix sum of the DC differences, one CTA per picture,
 //                     one launch; the integrated DC replaces the difference in the
@@ -611,6 +613,18 @@ __global__ void __launch_bounds__(kScanThreads) k1_scan(K1Args a) {
 
 // ---------------------------------------------------------------- k1_write
 
+// k1_fused's DC integration splits a picture's blocks among its CTAs at the block each CTA's first own subsequence starts
+// in: the block in progress there for a subsequence inside a restart interval (`excl` = blocks the interval ended
+// before it), the interval's end for one behind the interval's data, the picture's end for one behind the picture.
+// Clamped so that the split points never decrease, whatever a damaged stream made of the counts.
+constexpr int kDcPosSlot = 32;   // K1Smem::scratch words holding the range (IntegrateDc)
+__device__ __forceinline__ uint32_t BlockPos(const K1Args& a, const ImageDesc& im, const Sub& s, uint32_t excl) {
+    if (!s.in_range) return im.nblocks;
+    const SegmentDesc& sd = a.segments[s.seg];
+    const uint32_t p = sd.blk_first + (!s.active ? sd.blk_count : s.first ? 0u : min(excl, sd.blk_count));
+    return min(p, im.nblocks);
+}
+
 // The write pass behind the staging: `st`, `my_nnz`, `key` = the thread's synchronised end state, entry count and start
 // state. FUSED (k1_fused): the same CTA has just synchronised - what enters it from the picture's earlier CTAs is read
 // from their partials as soon as each has published them (`cta_flag`), and the state handed over at the CTA boundary is
@@ -866,9 +880,15 @@ __global__ void __launch_bounds__(T) k1_write(K1Args a) {
 // write. What the verifying round of k1_sync checks is checked here by the CTA itself: the state its halo threads
 // derived for its first subsequence must be the one the owner (the CTA before it) ended on; every mismatch is counted
 // in counters[0], and the host then falls back to the separate kernels for the batch (none on the benchmark batches,
-// forced in tests with ROCJPEG_B200_HALO=1).
+// forced in tests with ROCJPEG_B200_HALO=1). With K1Args::k1_dc the CTA then turns the DC differences of its share of the
+// picture's blocks into absolute DC values (IntegrateDc), and no DC kernel follows.
 template <int S>
-__global__ void __launch_bounds__(T) k1_fused(K1Args a, int max_iters) {
+__device__ void IntegrateDc(const K1Args& a, uint32_t* scratch, uint32_t img, uint32_t cta);
+
+// (the register cap replaces __launch_bounds__(T), which cannot be combined with it: the DC integration behind the write
+// loop would otherwise raise the kernel from the decode loops' 46 registers to 48)
+template <int S>
+__global__ void __maxnreg__(46) k1_fused(K1Args a, int max_iters) {
     PdlEntry();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint32_t* const lut = reinterpret_cast<uint32_t*>(smem_raw);
@@ -876,11 +896,12 @@ __global__ void __launch_bounds__(T) k1_fused(K1Args a, int max_iters) {
     const int tid = threadIdx.x;
     // Which CTA's work this is: a ticket, not blockIdx - the waits below are for lower indices, and a ticket holder
     // knows that every lower ticket has been drawn by a CTA that is running (whatever order the grid is dispatched in).
-    __shared__ uint32_t s_ticket;
+    __shared__ uint32_t s_ticket, s_img;
     if (tid == 0) s_ticket = atomicAdd(a.cta_flag + a.total_ctas, 1u);
     __syncthreads();
     const uint32_t cta = s_ticket;
     SyncOut so = SyncBody<S, true>(a, sm, lut, 0, max_iters, cta);
+    if (tid == 0) s_img = so.img;
     // this CTA's counts and states are in global memory: let the picture's later CTAs see them
     __threadfence();
     __syncthreads();
@@ -899,6 +920,15 @@ __global__ void __launch_bounds__(T) k1_fused(K1Args a, int max_iters) {
     Sub me = so.me;
     if (tid < H) me.active = false;   // halo slots belong to the previous CTA
     WriteBody<S, true>(a, sm, so.lv, so.img, im, me, me.active ? so.state : 0u, me.active ? so.nnz : 0u, so.used, cta);
+    if (a.k1_dc) {
+        // (ticket and picture re-read from shared memory: kept in registers across the write loop they cost two)
+        const uint32_t c = *static_cast<volatile uint32_t*>(&s_ticket);
+        // this CTA's records are written: the next CTA may read the DC difference its first block got from here
+        __threadfence();
+        __syncthreads();
+        if (tid == 0) asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(a.cta_flag + c), "r"(2u) : "memory");
+        IntegrateDc<S>(a, sm.scratch, *static_cast<volatile uint32_t*>(&s_img), c);
+    }
 }
 
 // ---------------------------------------------------------------- DC prediction
@@ -967,6 +997,150 @@ __device__ __forceinline__ int64_t LastReset(int64_t m0, int64_t m1, int ri) {
     if (ri <= 0) return m0 == 0 ? 0 : -1;
     const int64_t last = ((m1 - 1) / ri) * ri;
     return last >= m0 ? last : -1;
+}
+
+// RecDc through L2: the first block of a range may have got its DC difference from another SM
+__device__ __forceinline__ int LoadDc(const BlockRec* r) {
+    const uint2 v = __ldcg(reinterpret_cast<const uint2*>(r));
+    return v.x == kNoEntry ? 0 : int(int16_t(v.y & 0xFFFFu));
+}
+
+// k1_fused, after its write pass: the DC differences of blocks [lo, hi) of the picture (BlockPos) become absolute DC values,
+// the arithmetic of dc_image on a range that need not start on an MCU. Every record of the range is final once this CTA and
+// the one before it have written theirs: the first block's DC symbol may lie in the previous CTA, every other symbol of the
+// range lies in this one. Each thread sums a contiguous run; a CTA-wide segmented scan and a decoupled look-back over the
+// picture's earlier CTAs (their per-component sums after the last predictor reset, or the predictors leaving them once
+// known) give the predictors entering each run. Every wait is for a lower ticket, i.e. for a running CTA that itself
+// waits only for lower tickets.
+template <int S>
+__device__ void IntegrateDc(const K1Args& a, uint32_t* scratch, uint32_t img, uint32_t cta) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    constexpr int kW = T / 32;
+    const ImageDesc& im = a.images[img];
+    const uint32_t first = __ldg(a.img_cta0 + img);
+    uint32_t* const dc_flag = a.cta_flag + a.total_ctas + 1;
+    const int H = a.halo;
+    if (tid == H || tid == T - 1) {   // the range: where the CTA's first own subsequence starts, and where the next CTA's does
+        // blocks entering the CTA from its restart interval (WriteBody left them in scratch) and, from the CTA's own partial,
+        // those leaving it
+        const uint32_t enter = scratch[3 * kW];
+        const int64_t gi = int64_t(cta) * (T - H) + tid - H;
+        if (tid == H) {
+            scratch[kDcPosSlot] = BlockPos(a, im, Locate<S>(a, im, gi, false), enter);
+        } else {
+            const uint2 part = a.cta_partial[cta];
+            scratch[kDcPosSlot + 1] = BlockPos(a, im, Locate<S>(a, im, gi + 1, false), part.y + (part.x ? 0u : enter));
+        }
+    }
+    if (tid == 0 && cta != first) {
+        uint32_t f;
+        do {
+            asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(f) : "l"(a.cta_flag + cta - 1) : "memory");
+        } while (f != 2u);
+    }
+    __syncthreads();
+    const uint32_t lo = cta == first ? 0u : scratch[kDcPosSlot];
+    const uint32_t hi = max(lo, scratch[kDcPosSlot + 1]);
+    const uint32_t per = (hi - lo + T - 1) / T;
+    const uint32_t b0 = min(lo + uint32_t(tid) * per, hi), b1 = min(b0 + per, hi);
+    BlockRec* const rec = a.blk_rec + im.blk0;
+    const uint32_t bpm = uint32_t(im.bpm), comp_bits = im.comp_bits;
+    const int ri = im.restart_interval;
+    // the run's sums after its last reset (f: it holds one)
+    int s0 = 0, s1 = 0, s2 = 0;
+    uint32_t f = 0;
+    {
+        uint32_t m = b0 / bpm, k = b0 - m * bpm;
+        for (uint32_t b = b0; b < b1; b++) {
+            if (k == 0 && ResetAt(m, ri)) { s0 = s1 = s2 = 0; f = 1; }
+            const int d = LoadDc(rec + b);
+            const uint32_t comp = (comp_bits >> (2 * k)) & 3u;
+            s0 += comp == 0u ? d : 0;
+            s1 += comp == 1u ? d : 0;
+            s2 += comp == 2u ? d : 0;
+            if (++k == bpm) { k = 0; m++; }
+        }
+    }
+    int v0 = s0, v1 = s1, v2 = s2;
+    uint32_t g = f;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int p0 = __shfl_up_sync(0xFFFFFFFFu, v0, d);
+        const int p1 = __shfl_up_sync(0xFFFFFFFFu, v1, d);
+        const int p2 = __shfl_up_sync(0xFFFFFFFFu, v2, d);
+        const uint32_t pg = __shfl_up_sync(0xFFFFFFFFu, g, d);
+        if (lane >= d) {
+            if (!g) { v0 += p0; v1 += p1; v2 += p2; }
+            g |= pg;
+        }
+    }
+    int* const ws = reinterpret_cast<int*>(scratch);   // [4 w + c]: warp w's inclusive sums, [4 w + 3]: it holds a reset
+    int* const carry = ws + 4 * kW;                      // predictors entering the CTA
+    if (lane == 31) { ws[4 * warp] = v0; ws[4 * warp + 1] = v1; ws[4 * warp + 2] = v2; ws[4 * warp + 3] = int(g); }
+    __syncthreads();
+    if (warp == 0) {
+        int t0 = 0, t1 = 0, t2 = 0, tf = 0;   // the CTA's own sums after its last reset
+        for (int w = 0; w < kW; w++) {
+            if (ws[4 * w + 3]) { t0 = ws[4 * w]; t1 = ws[4 * w + 1]; t2 = ws[4 * w + 2]; tf = 1; }
+            else { t0 += ws[4 * w]; t1 += ws[4 * w + 1]; t2 += ws[4 * w + 2]; }
+        }
+        if (lane == 0) {
+            a.cta_dc[2 * cta] = make_int4(t0, t1, t2, tf);
+            __threadfence();
+            asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(dc_flag + cta), "r"(1u) : "memory");
+        }
+        // one lane per earlier CTA of the picture, 32 at a time from the nearest backwards, up to the nearest one whose
+        // outgoing predictors are known or whose range holds a reset
+        int c0 = 0, c1 = 0, c2 = 0;
+        for (int64_t top = int64_t(cta); top > int64_t(first); top -= 32) {
+            const int64_t k = top - 32 + lane;
+            int4 e = make_int4(0, 0, 0, 0);
+            uint32_t fl = 0;
+            if (k >= int64_t(first)) {
+                do {
+                    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(fl) : "l"(dc_flag + k) : "memory");
+                } while (fl == 0u);
+                e = __ldcg(a.cta_dc + 2 * k + (fl == 2u ? 1 : 0));
+            }
+            const uint32_t stop = __ballot_sync(0xFFFFFFFFu, fl == 2u || e.w != 0);
+            const int from = stop ? 31 - __clz(stop) : 0;
+            if (lane >= from) { c0 += e.x; c1 += e.y; c2 += e.z; }
+            if (stop) break;
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            c0 += __shfl_xor_sync(0xFFFFFFFFu, c0, d);
+            c1 += __shfl_xor_sync(0xFFFFFFFFu, c1, d);
+            c2 += __shfl_xor_sync(0xFFFFFFFFu, c2, d);
+        }
+        if (lane == 0) {
+            carry[0] = c0; carry[1] = c1; carry[2] = c2;
+            a.cta_dc[2 * cta + 1] = tf ? make_int4(t0, t1, t2, 0) : make_int4(c0 + t0, c1 + t1, c2 + t2, 0);
+            __threadfence();
+            asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(dc_flag + cta), "r"(2u) : "memory");
+        }
+    }
+    __syncthreads();
+    // predictors entering the run: the warp's exclusive prefix, the earlier warps' sums back to the last reset, the carry
+    int p0 = __shfl_up_sync(0xFFFFFFFFu, v0, 1), p1 = __shfl_up_sync(0xFFFFFFFFu, v1, 1), p2 = __shfl_up_sync(0xFFFFFFFFu, v2, 1);
+    uint32_t open = !__shfl_up_sync(0xFFFFFFFFu, g, 1);
+    if (lane == 0) { p0 = p1 = p2 = 0; open = 1; }
+    for (int w = warp - 1; w >= 0 && open; w--) {
+        p0 += ws[4 * w]; p1 += ws[4 * w + 1]; p2 += ws[4 * w + 2];
+        if (ws[4 * w + 3]) open = 0;
+    }
+    if (open) { p0 += carry[0]; p1 += carry[1]; p2 += carry[2]; }
+    uint32_t m = b0 / bpm, k = b0 - m * bpm;
+    for (uint32_t b = b0; b < b1; b++) {
+        if (k == 0 && ResetAt(m, ri)) p0 = p1 = p2 = 0;
+        const int d = LoadDc(rec + b);
+        const uint32_t comp = (comp_bits >> (2 * k)) & 3u;
+        p0 += comp == 0u ? d : 0;
+        p1 += comp == 1u ? d : 0;
+        p2 += comp == 2u ? d : 0;
+        rec[b].dc = int16_t(comp == 0u ? p0 : comp == 1u ? p1 : p2);
+        if (++k == bpm) { k = 0; m++; }
+    }
 }
 
 __global__ void __launch_bounds__(kDcTileMcus) dc_sums(K1Args a) {

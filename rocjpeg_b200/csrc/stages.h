@@ -117,7 +117,11 @@ struct K1Args {
     uint2* cta_partial;           // per K1 CTA: (has segment start, blocks after the last start)
     uint32_t* cta_entries;        // per K1 CTA: coefficient entries of the CTA's subsequences
     uint2* cta_carry;             // per K1 CTA: (blocks, entries) entering it from the image's earlier CTAs (k1_scan)
-    uint32_t* cta_flag;           // per K1 CTA: k1_fused has published the CTA's counts and states; [total_ctas] = its ticket counter (all zeroed before the launch)
+    uint32_t* cta_flag;           // per K1 CTA: k1_fused has published the CTA's counts and states (1) and written its records (2);
+                                  // [total_ctas] = its ticket counter; [total_ctas + 1 + k] = CTA k has published its DC sums (1) and
+                                  // the predictors leaving it (2) (all zeroed before the launch)
+    int4* cta_dc;                 // per K1 CTA (k1_fused with k1_dc): [2 k] per-component DC sums of its block range after its last
+                                  // predictor reset (.w: the range holds one), [2 k + 1] predictors leaving it
     int3* dc_partial;             // per DC tile: per-component DC sum after the tile's last reset
     int3* dc_carry;               // per DC tile: predictors entering it (dc_scan)
     uint32_t* counters;           // [kMaxSyncRounds] boundary changes per round, then [kMaxSyncRounds] decodes per round
@@ -137,6 +141,7 @@ struct K1Args {
     int fusable;                  // no image has more than 256 K1 CTAs: counting and write pass may run as one kernel (k1_fused)
     int dc_image;                 // no image has more than kDcImageMaxMcus MCUs: one CTA per image integrates its DC
                                   // differences in ONE launch (dc_image) instead of sums / scan / apply
+    int k1_dc;                    // k1_fused integrates the DC differences itself: LaunchDcScan is not needed after it
 };
 
 // Speculative decode + CTA-local synchronisation (round 0) or cross-CTA fix-up (round >= 1).
