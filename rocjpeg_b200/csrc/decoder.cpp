@@ -33,6 +33,12 @@ int TraceLevel() {
     return level;
 }
 
+// ROCJPEG_B200_DEBUG_SYNC=1: synchronise after every stage of a lane and say which one failed
+bool DebugSync() {
+    static const bool on = EnvInt("ROCJPEG_B200_DEBUG_SYNC", 0) != 0;
+    return on;
+}
+
 double NowMs() {
     return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
@@ -103,30 +109,6 @@ void SubmitPool::Run(int n, const std::function<void(int)>& fn) {
     fn(0);
     while (pending_.load(std::memory_order_acquire) != 0) std::this_thread::yield();
 }
-
-namespace {
-// Waits for the submitter's turn on the shared upload stream and passes it on - also when the
-// submitter bails out early, so that the lanes behind it never wait forever.
-struct TurnGuard {
-    UploadTurn t;
-    bool passed = false;
-    explicit TurnGuard(UploadTurn turn) : t(turn) {}
-    void Acquire() const {
-        if (t.turn)
-            while (t.turn->load(std::memory_order_acquire) != t.mine) std::this_thread::yield();
-    }
-    void Release() {
-        if (t.turn && !passed) t.turn->store(t.mine + 1, std::memory_order_release);
-        passed = true;
-    }
-    ~TurnGuard() {
-        if (!passed) {
-            Acquire();
-            Release();
-        }
-    }
-};
-}  // namespace
 
 DeviceBuffer::~DeviceBuffer() {
     if (ptr_) cudaFree(ptr_);
@@ -449,7 +431,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     uint64_t scan_off = 0, raw_off = 0, blk = 0, plane_off = 0, ent = 0, sub = 0;
     uint32_t dctile = 0, k2tile = 0, k3tile = 0, max_pairs = 1, max_sub = 0, k0tile = 0, nseg_total = 0;
     uint32_t k2stile[kScaledKernels] = {};
-    all_pinned_ = true;
+    bool all_pinned = true;
     // Upload plan. Streams that lie close together in ONE page-locked allocation (the caller's arena of files, or
     // the staging pool's slab) are uploaded by a single copy that takes the few bytes between them along: the copy
     // engine moves such a run at the full PCIe rate (48-50 GB/s measured against 33 GB/s for the gather kernel's
@@ -567,7 +549,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
         if (merged) raw_off = plan_off[size_t(i)];
         im.raw_off = raw_off;
         h_gather_[size_t(i)] = GatherItem{src - im.raw_skip, raw_off, up_bytes, 0u};
-        all_pinned_ = all_pinned_ && rs.dev != nullptr;
+        all_pinned = all_pinned && rs.dev != nullptr;
         raw_off += AlignUp(size_t(up_bytes) + 16, 128);   // (merged: the arena's end is taken from the last run below)
         im.k0_tile0 = k0tile;
         h_k0_tile0_[size_t(i)] = k0tile;
@@ -726,6 +708,12 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     stats_.scan_bytes = total_clean;
     stats_.blocks = blk;
     stats_.subsequences = sub;
+    // Many small pictures: one gather kernel reading the parsers' mapped page-locked buffers (a copy call per picture
+    // would cost the host more than the transfer). Few large ones: plain copies, which run on the copy engine at full
+    // PCIe rate without occupying SMs.
+    if (!h_runs_.empty()) upload_by_ = kUploadRuns;
+    else if (all_pinned && n > 4 && raw_bytes_ / size_t(n) < (256u << 10) && EnvInt("ROCJPEG_B200_NO_GATHER", 0) == 0) upload_by_ = kUploadGather;
+    else upload_by_ = kUploadPerPicture;
 
     k1_ = K1Args{};
     k1_.nimages = n;
@@ -735,10 +723,11 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     k0_.nimages = n;
     k0_.total_tiles = k0tile;
     k0_.sub_bytes = S;
+    const bool inline_scan_ok = EnvInt("ROCJPEG_B200_NO_INLINE_SCAN", 0) == 0;
     {
         uint32_t most_tiles = 0;
         for (int i = 0; i < n; i++) most_tiles = std::max(most_tiles, h_k0_tile0_[size_t(i) + 1] - h_k0_tile0_[size_t(i)]);
-        k0_.inline_scan = (most_tiles <= 32u && EnvInt("ROCJPEG_B200_NO_INLINE_SCAN", 0) == 0) ? 1 : 0;
+        k0_.inline_scan = (most_tiles <= 32u && inline_scan_ok) ? 1 : 0;
     }
     k1_.rec_fill_vecs = uint32_t((blk * sizeof(BlockRec) + 15) / 16);   // the slab leaves 256 bytes behind every array
     k1_.lut_smem_bytes = max_pairs * 2u * uint32_t(kFastSize) * 4u + max_sub * 4u;
@@ -747,7 +736,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     {
         uint32_t most = 0;
         for (int i = 0; i < n; i++) most = std::max(most, h_img_cta0_[size_t(i) + 1] - h_img_cta0_[size_t(i)]);
-        k1_.inline_scan = (most <= 32u && EnvInt("ROCJPEG_B200_NO_INLINE_SCAN", 0) == 0) ? 1 : 0;
+        k1_.inline_scan = (most <= 32u && inline_scan_ok) ? 1 : 0;
         k1_.fusable = most <= uint32_t(std::max(0, EnvInt("ROCJPEG_B200_K1_FUSE_CTAS", 256))) ? 1 : 0;
         uint32_t most_mcus = 0;
         for (int i = 0; i < n; i++) most_mcus = std::max(most_mcus, uint32_t(h_images_[size_t(i)].total_mcus));
@@ -756,6 +745,16 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
         const int dc_limit = EnvInt("ROCJPEG_B200_DC_IMAGE_MCUS", n >= 16 ? 2 * kDcImageMaxMcus : kDcImageMaxMcus);
         k1_.dc_image = (most_mcus <= uint32_t(std::max(0, dc_limit)) && EnvInt("ROCJPEG_B200_NO_DC_IMAGE", 0) == 0) ? 1 : 0;
     }
+    // Counting and write pass of the entropy stage in one kernel when no picture has more than 256 K1 CTAs (k1_huffman.cu:
+    // k1_fused); ROCJPEG_B200_NO_K1_FUSE=1 or an explicit ROCJPEG_B200_SYNC_ROUNDS keep the separate kernels, with that
+    // many k1_sync rounds launched up front.
+    const char* rounds_env = std::getenv("ROCJPEG_B200_SYNC_ROUNDS");
+    sync_rounds_ = std::min(std::max((rounds_env && *rounds_env) ? std::atoi(rounds_env) : 2, 1), kMaxSyncRounds);
+    k1_fused_ = !rounds_env && EnvInt("ROCJPEG_B200_NO_K1_FUSE", 0) == 0 && k1_.fusable && k1_.total_ctas != 0;
+    // ... and, for pictures small enough for dc_image, it integrates the DC differences itself (no DC launch behind it;
+    // ROCJPEG_B200_NO_K1_DC=1 keeps it). Not for larger ones: a CTA waits there for the picture's earlier CTAs to finish
+    // writing, and with the many CTAs of 4K pictures those waits hold SM slots the next wave needs (c4_dri 3.29 -> 3.65 ms)
+    k1_.k1_dc = k1_fused_ && k1_.dc_image && EnvInt("ROCJPEG_B200_NO_K1_DC", 0) == 0 ? 1 : 0;
     k2_ = K2Args{};
     k2_.nimages = n;
     k2_.total_tiles = k2tile;
@@ -779,8 +778,7 @@ struct Lane::Layout {
     size_t images, outputs, cta0, k0tile0, dctile0, k2tile0, k2stile0[kScaledKernels], k3tile0, fused, tile_img, tile_img_w, gather, luts, qtables, total;
 };
 
-int Lane::Upload(cudaStream_t up, UploadTurn turn) {
-    TurnGuard guard(turn);
+int Lane::Upload(cudaStream_t up) {
     if (up == nullptr) up = stream_;
     const size_t n = h_images_.size();
     Layout L;
@@ -896,50 +894,41 @@ int Lane::Upload(cudaStream_t up, UploadTurn turn) {
 
     // Uploads of all lanes go through ONE stream, in lane order: the first chunk gets the whole
     // PCIe link and its kernels start while the next chunks are still in flight.
-    guard.Acquire();
     host_ms_[1] = NowMs();
     if (ev_trace_[0]) RJB_CUDA(cudaEventRecord(ev_trace_[0], up));
     RJB_CUDA(cudaMemcpyAsync(d, h, L.total, cudaMemcpyHostToDevice, up));
     stats_.h2d_bytes = L.total;
-    for (const GatherItem& g : h_gather_) stats_.h2d_bytes += g.nbytes;
-    // Many small pictures: one gather kernel reading the parsers' mapped page-locked buffers (a copy call
-    // per picture would cost the host more than the transfer). Few large ones: plain copies, which run on
-    // the copy engine at full PCIe rate without occupying SMs.
-    const bool use_runs = !h_runs_.empty();
-    const bool use_gather = !use_runs && all_pinned_ && h_images_.size() > 4 && raw_bytes_ / h_images_.size() < (256u << 10) &&
-                            EnvInt("ROCJPEG_B200_NO_GATHER", 0) == 0;
-    tiles_reduced_ = use_gather;
-    if (use_gather) {   // ... which also leaves the per-tile prefix elements of the destuffing pass
-        RJB_CUDA(LaunchGatherReduce(k0_, reinterpret_cast<const GatherItem*>(d + L.gather), up));
-        stats_.kernel_launches++;
-    } else if (use_runs) {
-        stats_.h2d_bytes = L.total;
-        for (const CopyRun& r : h_runs_) {
-            RJB_CUDA(cudaMemcpyAsync(const_cast<uint8_t*>(k0_.raw) + r.dst_off, r.src, r.nbytes, cudaMemcpyHostToDevice, up));
-            stats_.h2d_bytes += r.nbytes;
-        }
-    } else {
-        for (size_t i = 0; i < n; i++)
-            RJB_CUDA(cudaMemcpyAsync(const_cast<uint8_t*>(k0_.raw) + h_gather_[i].dst_off, h_gather_[i].src, h_gather_[i].nbytes,
-                                     cudaMemcpyHostToDevice, up));
+    switch (upload_by_) {
+        case kUploadGather:
+            RJB_CUDA(LaunchGatherReduce(k0_, reinterpret_cast<const GatherItem*>(d + L.gather), up, &stats_.kernel_launches));
+            for (const GatherItem& g : h_gather_) stats_.h2d_bytes += g.nbytes;
+            break;
+        case kUploadRuns:
+            for (const CopyRun& r : h_runs_) {
+                RJB_CUDA(cudaMemcpyAsync(const_cast<uint8_t*>(k0_.raw) + r.dst_off, r.src, r.nbytes, cudaMemcpyHostToDevice, up));
+                stats_.h2d_bytes += r.nbytes;
+            }
+            break;
+        case kUploadPerPicture:
+            for (const GatherItem& g : h_gather_) {
+                RJB_CUDA(cudaMemcpyAsync(const_cast<uint8_t*>(k0_.raw) + g.dst_off, g.src, g.nbytes, cudaMemcpyHostToDevice, up));
+                stats_.h2d_bytes += g.nbytes;
+            }
+            break;
     }
     if (ev_trace_[1]) RJB_CUDA(cudaEventRecord(ev_trace_[1], up));
     if (up != stream_) {
         RJB_CUDA(cudaEventRecord(ev_uploaded_, up));
-        guard.Release();
         RJB_CUDA(cudaStreamWaitEvent(stream_, ev_uploaded_, 0));
     }
     return kSuccess;
 }
 
-int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up, UploadTurn turn) {
-    const int rounds = std::min(std::max(EnvInt("ROCJPEG_B200_SYNC_ROUNDS", 2), 1), kMaxSyncRounds);
+int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up) {
     // profiling 1: an event after every stage (they sit between the kernels, so neighbouring stages no longer
     // overlap through programmatic dependent launch); 2: only the first and the last event (total time)
-    // ROCJPEG_B200_DEBUG_SYNC=1: synchronise after every stage and say which one failed
-    static const bool debug_sync = EnvInt("ROCJPEG_B200_DEBUG_SYNC", 0) != 0;
     auto mark = [&](int i) -> cudaError_t {
-        if (debug_sync) {
+        if (DebugSync()) {
             const cudaError_t e = cudaStreamSynchronize(stream_);
             if (e != cudaSuccess) {
                 static const char* const kNames[] = {"(before)", "upload", "destuff", "huffman sync", "huffman write", "dc", "idct", "output"};
@@ -951,20 +940,17 @@ int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up, Upload
         return want ? cudaEventRecord(ev_[i], stream_) : cudaSuccess;
     };
     stats_.kernel_launches = 0;
-    // whatever happens below, the lanes queued behind this one on the upload stream get their turn (the guard passes it on
-    // when this function leaves before Upload() did), and a failure leaves both counter sets clean for the next call
+    // whatever happens below, a failure leaves both counter sets clean for the next call
     struct ExitGuard {
         Lane* lane;
-        TurnGuard turn;
         bool ok = false;
         ~ExitGuard() {
             if (!ok && lane->d_counters_.capacity() >= 512) cudaMemsetAsync(lane->d_counters_.as<uint8_t>(), 0, 512, lane->stream_);
         }
-    } exit_guard{this, TurnGuard(include_upload ? turn : UploadTurn())};
+    } exit_guard{this};
     RJB_CUDA(mark(0));
     if (include_upload) {
-        exit_guard.turn.passed = true;   // Upload() owns the turn from here on (its own guard passes it on)
-        int st = Upload(up, turn);
+        int st = Upload(up);
         if (st != kSuccess) return st;
     }
     RJB_CUDA(mark(1));
@@ -981,55 +967,44 @@ int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up, Upload
         RJB_CUDA(cudaMemsetAsync(k1_.blk_rec, 0xFF, coef_blocks_ * sizeof(BlockRec), stream_));
         RJB_CUDA(cudaMemsetAsync(k1_.counters_next, 0, 256, stream_));
     }
-    // Counting and write pass of the entropy stage in one kernel when no picture has more than 256 K1 CTAs (k1_huffman.cu:
-    // k1_fused); ROCJPEG_B200_NO_K1_FUSE=1 or an explicit ROCJPEG_B200_SYNC_ROUNDS keep the separate kernels.
-    const bool k1_fuse_ok = EnvInt("ROCJPEG_B200_NO_K1_FUSE", 0) == 0 && std::getenv("ROCJPEG_B200_SYNC_ROUNDS") == nullptr;
-    const bool k1_fused = k1_fuse_ok && k1_.fusable && k1_.total_ctas != 0;
-    // ... and, for pictures small enough for dc_image, it integrates the DC differences itself (no DC launch behind it;
-    // ROCJPEG_B200_NO_K1_DC=1 keeps it). Not for larger ones: a CTA waits there for the picture's earlier CTAs to finish
-    // writing, and with the many CTAs of 4K pictures those waits hold SM slots the next wave needs (c4_dri 3.29 -> 3.65 ms)
-    k1_.k1_dc = k1_fused && k1_.dc_image && EnvInt("ROCJPEG_B200_NO_K1_DC", 0) == 0 ? 1 : 0;
     // "published" flags of the CTAs, the ticket counter, the CTAs' DC flags
-    if (k1_fused) RJB_CUDA(cudaMemsetAsync(k1_.cta_flag, 0, size_t(k1_.total_ctas) * 8 + 4, stream_));
+    if (k1_fused_) RJB_CUDA(cudaMemsetAsync(k1_.cta_flag, 0, size_t(k1_.total_ctas) * 8 + 4, stream_));
     // K0: end of slice, destuffing, restart intervals -> clean stream + segment table, all on the device
-    if (!(include_upload && tiles_reduced_)) {   // cudaMemcpy upload, or a resident batch run again: the reduction is its own launch
-        RJB_CUDA(LaunchK0Reduce(k0_, stream_));
-        stats_.kernel_launches++;
-    }
-    RJB_CUDA(LaunchK0Destuff(k0_, stream_));
-    stats_.kernel_launches += k0_.inline_scan ? 1 : 2;
+    if (!(include_upload && upload_by_ == kUploadGather))   // cudaMemcpy upload, or a resident batch run again: the reduction is its own launch
+        RJB_CUDA(LaunchK0Reduce(k0_, stream_, &stats_.kernel_launches));
+    RJB_CUDA(LaunchK0Destuff(k0_, stream_, &stats_.kernel_launches));
     RJB_CUDA(mark(2));
-    if (k1_fused) {
-        RJB_CUDA(LaunchK1Fused(k1_, stream_));
+    if (k1_fused_) {
+        RJB_CUDA(LaunchK1Fused(k1_, stream_, &stats_.kernel_launches));
         stats_.sync_rounds = 1;   // counters[0] = CTA boundaries that did not hold: Finish() then runs the separate kernels
         RJB_CUDA(mark(3));
     } else {
-        for (int r = 0; r < rounds; r++) RJB_CUDA(LaunchK1Sync(k1_, r, stream_));
-        stats_.sync_rounds = uint32_t(rounds);
+        for (int r = 0; r < sync_rounds_; r++) RJB_CUDA(LaunchK1Sync(k1_, r, stream_, &stats_.kernel_launches));
+        stats_.sync_rounds = uint32_t(sync_rounds_);
         RJB_CUDA(mark(3));
-        RJB_CUDA(LaunchK1Write(k1_, stream_));
+        RJB_CUDA(LaunchK1Write(k1_, stream_, &stats_.kernel_launches));
     }
     RJB_CUDA(mark(4));
-    if (!k1_.k1_dc) RJB_CUDA(LaunchDcScan(k1_, stream_));
-    RJB_CUDA(mark(5));
-    uint32_t idct_launches = 0;
-    {
-        const int st = LaunchIdct(false, &idct_launches);
-        if (st != kSuccess) return st;
-    }
-    RJB_CUDA(mark(6));
-    RJB_CUDA(LaunchK23Fused(k23_, stream_));
-    RJB_CUDA(LaunchK3Output(k3_, stream_));
-    RJB_CUDA(mark(7));
-    stats_.kernel_launches += (k1_fused ? 1u : uint32_t(rounds) + (k1_.inline_scan ? 1u : 2u)) + (k1_.k1_dc ? 0 : k1_.dc_image ? 1 : 3) + idct_launches +
-                              (k23_.total_tiles ? 1 : 0) + (k23_.total_tiles_w ? 1 : 0) +
-                              (k3_.total_tiles ? 1 : 0);   // sync rounds, (scan +) write, 0, 1 or 3 DC kernels, IDCT, fused IDCT + output, output
-    RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
-    RJB_CUDA(cudaMemcpyAsync(h_counters_.data() + 256, k0_.status, h_images_.size() * sizeof(ScanStatus), cudaMemcpyDeviceToHost, stream_));
-    stats_.d2h_bytes = 256 + h_images_.size() * sizeof(ScanStatus);
+    const int st = LaunchDownstream(!k1_.k1_dc, mark);
+    if (st != kSuccess) return st;
     if (ev_trace_[2]) RJB_CUDA(cudaEventRecord(ev_trace_[2], stream_));
     host_ms_[2] = NowMs();
     exit_guard.ok = true;
+    return kSuccess;
+}
+
+int Lane::LaunchDownstream(bool integrate_dc, const std::function<cudaError_t(int)>& mark) {
+    if (integrate_dc) RJB_CUDA(LaunchDcScan(k1_, stream_, &stats_.kernel_launches));
+    RJB_CUDA(mark(5));
+    const int st = LaunchIdct(false, &stats_.kernel_launches);
+    if (st != kSuccess) return st;
+    RJB_CUDA(mark(6));
+    RJB_CUDA(LaunchK23Fused(k23_, stream_, &stats_.kernel_launches));
+    RJB_CUDA(LaunchK3Output(k3_, stream_, &stats_.kernel_launches));
+    RJB_CUDA(mark(7));
+    RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
+    RJB_CUDA(cudaMemcpyAsync(h_counters_.data() + 256, k0_.status, h_images_.size() * sizeof(ScanStatus), cudaMemcpyDeviceToHost, stream_));
+    stats_.d2h_bytes = 256 + h_images_.size() * sizeof(ScanStatus);
     return kSuccess;
 }
 
@@ -1037,15 +1012,11 @@ int Lane::LaunchIdct(bool force_planes, uint32_t* launches) {
     // (force_planes: the plane tap's re-run, which transforms every picture - fused ones included - into the arena)
     K2Args k2 = k2_;
     k2.force_planes = force_planes ? 1 : 0;
-    if (k2_needed_ || force_planes) {
-        RJB_CUDA(LaunchK2Idct(k2, stream_));
-        if (k2.total_tiles) (*launches)++;
-    }
+    if (k2_needed_ || force_planes) RJB_CUDA(LaunchK2Idct(k2, stream_, launches));
     for (int s = 0; s < kScaledKernels; s++) {
         K2Args ks = k2s_[s];
         ks.force_planes = k2.force_planes;
-        RJB_CUDA(LaunchK2Scaled(ks, 2 << s, stream_));
-        if (ks.total_tiles) (*launches)++;
+        RJB_CUDA(LaunchK2Scaled(ks, 2 << s, stream_, launches));
     }
     return kSuccess;
 }
@@ -1062,29 +1033,22 @@ int Lane::Finish(int profiling_) {
         for (;;) {
             uint32_t slot = std::min<uint32_t>(last + 1, kMaxSyncRounds - 1);
             RJB_CUDA(cudaMemsetAsync(k1_.counters + slot, 0, 4, stream_));
-            RJB_CUDA(LaunchK1Sync(k1_, int(slot), stream_));
+            RJB_CUDA(LaunchK1Sync(k1_, int(slot), stream_, &stats_.kernel_launches));
             RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
             RJB_CUDA(cudaStreamSynchronize(stream_));
             stats_.sync_rounds++;
-            stats_.kernel_launches++;
             last = slot;
             if (cnt[slot] == 0) break;
             if (++guard > k1_.total_ctas + 2) return Fail(kExecutionFailed, "entropy decoder failed to converge");
         }
         RJB_CUDA(cudaMemsetAsync(k1_.blk_rec, 0xFF, coef_blocks_ * sizeof(BlockRec), stream_));
         RJB_CUDA(cudaMemsetAsync(k1_.counters + 2 * kMaxSyncRounds, 0, 4, stream_));   // the first write pass counted its entries already
-        RJB_CUDA(LaunchK1ClearShort(k1_, stream_));   // ... and may have reported pictures short that are not
-        RJB_CUDA(LaunchK1Write(k1_, stream_));
-        RJB_CUDA(LaunchDcScan(k1_, stream_));
-        uint32_t idct_launches = 0;
-        const int st = LaunchIdct(false, &idct_launches);
+        RJB_CUDA(LaunchK1ClearShort(k1_, stream_, &stats_.kernel_launches));   // ... and may have reported pictures short that are not
+        RJB_CUDA(LaunchK1Write(k1_, stream_, &stats_.kernel_launches));
+        // k1_write leaves DC differences, also where k1_fused had integrated them; no stage events (the host waited in between)
+        const int st = LaunchDownstream(true, [](int) { return cudaSuccess; });
         if (st != kSuccess) return st;
-        RJB_CUDA(LaunchK23Fused(k23_, stream_));
-        RJB_CUDA(LaunchK3Output(k3_, stream_));
-        RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
-        RJB_CUDA(cudaMemcpyAsync(h_counters_.data() + 256, k0_.status, h_images_.size() * sizeof(ScanStatus), cudaMemcpyDeviceToHost, stream_));
         RJB_CUDA(cudaStreamSynchronize(stream_));
-        stats_.kernel_launches += 8;
     }
     stats_.entries = cnt[2 * kMaxSyncRounds];
     // per-image outcome: what the destuffing pass and the entropy stage found in the bytes
@@ -1193,13 +1157,9 @@ int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodePar
         const int st = lanes_[l].Create(device_id_, sm_count_, l < 4);
         if (st != kSuccess) return Fail(st, lanes_[l].last_error());
     }
-    // Optionally one submitter per lane (ROCJPEG_B200_SUBMIT_THREADS=1): the caller's thread takes lane 0,
-    // helper threads the others; uploads are enqueued in lane order, everything else in parallel. Off by
-    // default: it cuts the host's submit time from 0.22 to 0.09 ms on the 256-image batch, but the call is
-    // bound by the device (upload + pipeline), so the wall time does not move (profiles/r01e_e2e.md).
-    const bool threaded = active_lanes_ > 1 && EnvInt("ROCJPEG_B200_SUBMIT_THREADS", 0) != 0;
-    std::atomic<int> turn{0};
-    int status[kMaxLanes] = {};
+    // The lanes are described and enqueued one after the other on the caller's thread, so their uploads reach the shared
+    // upload stream in lane order. A submitter thread per lane would cut the host's submit time (0.22 -> 0.09 ms on the
+    // 256-image batch) but not the wall time: the call is bound by the device (profiles/r01e_e2e.md).
     // Pageable input: the parse only reserved page-locked staging; the bytes are copied now, chunk by chunk ahead of each
     // chunk's upload, by a few helper threads (one core copies 16 GB/s, a third of what the upload moves).
     bool any_pending = false;
@@ -1216,34 +1176,16 @@ int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodePar
             for (int i = first + t; i < first + cnt; i += threads) streams[i]->EnsureStaged();
         });
     };
-    auto submit = [&](int l) {
-        DeviceGuard guard(device_id_);
+    for (int l = 0; l < active_lanes_; l++) {
+        if (any_pending) stage(l);
         Lane& lane = lanes_[l];
         const int first = chunk_first_[l], cnt = chunk_first_[l + 1] - first;
-        UploadTurn ut;
-        ut.turn = threaded ? &turn : nullptr;
-        ut.mine = l;
         lane.set_host_mark(0, NowMs());
         int st = lane.Build(streams + first, cnt, params, dsts + first, remote ? remote + first : nullptr);
-        if (st == kSuccess) st = launch ? lane.LaunchAll(true, profiling_, upload_stream_, ut) : lane.Upload(upload_stream_, ut);
-        else TurnGuard pass(ut);   // never reached the upload: pass the turn on
-        status[l] = st;
-    };
-    if (threaded) {
-        for (int l = 0; l < active_lanes_ && any_pending; l++) stage(l);
-        if (!pool_) pool_.reset(new SubmitPool(kMaxLanes - 1));
-        pool_->Run(active_lanes_, submit);
-    } else {
-        for (int l = 0; l < active_lanes_; l++) {
-            if (any_pending) stage(l);
-            submit(l);
-            if (status[l] != kSuccess) break;
-        }
-    }
-    for (int l = 0; l < active_lanes_; l++) {
-        if (status[l] != kSuccess) {
+        if (st == kSuccess) st = launch ? lane.LaunchAll(true, profiling_, upload_stream_) : lane.Upload(upload_stream_);
+        if (st != kSuccess) {
             for (int k = 0; k < active_lanes_; k++) lanes_[k].Sync();   // do not leave work in flight behind an error (the failed lane's included)
-            return Fail(status[l], lanes_[l].last_error());
+            return Fail(st, lane.last_error());
         }
     }
     return kSuccess;
@@ -1267,25 +1209,28 @@ int Decoder::FinishAll() {
     return status;
 }
 
+void BatchStats::Accumulate(const BatchStats& s) {
+    for (int i = 0; i < kStageCount; i++) stage_ms[i] += s.stage_ms[i];
+    sync_rounds = std::max(sync_rounds, s.sync_rounds);
+    for (int r = 0; r < kMaxSyncRounds; r++) decodes_per_round[r] += s.decodes_per_round[r];
+    scan_bytes += s.scan_bytes;
+    blocks += s.blocks;
+    entries += s.entries;
+    subsequences += s.subsequences;
+    plane_bytes += s.plane_bytes;
+    fused_blocks += s.fused_blocks;
+    output_bytes += s.output_bytes;
+    h2d_bytes += s.h2d_bytes;
+    d2h_bytes += s.d2h_bytes;
+    kernel_launches += s.kernel_launches;
+    sub_bytes = std::max(sub_bytes, s.sub_bytes);
+}
+
 void Decoder::Aggregate() {
     stats_ = BatchStats();
     stats_.lanes = active_lanes_;
     for (int l = 0; l < active_lanes_; l++) {
-        const BatchStats& s = lanes_[l].stats();
-        for (int i = 0; i < kStageCount; i++) stats_.stage_ms[i] += s.stage_ms[i];
-        stats_.sync_rounds = std::max(stats_.sync_rounds, s.sync_rounds);
-        for (int r = 0; r < kMaxSyncRounds; r++) stats_.decodes_per_round[r] += s.decodes_per_round[r];
-        stats_.scan_bytes += s.scan_bytes;
-        stats_.blocks += s.blocks;
-        stats_.entries += s.entries;
-        stats_.subsequences += s.subsequences;
-        stats_.plane_bytes += s.plane_bytes;
-        stats_.fused_blocks += s.fused_blocks;
-        stats_.output_bytes += s.output_bytes;
-        stats_.h2d_bytes += s.h2d_bytes;
-        stats_.d2h_bytes += s.d2h_bytes;
-        stats_.kernel_launches += s.kernel_launches;
-        stats_.sub_bytes = std::max(stats_.sub_bytes, s.sub_bytes);
+        stats_.Accumulate(lanes_[l].stats());
         if (profiling_) {   // wall time on the device: first event of the first lane to the last event of any lane
             float ms = 0;
             if (cudaEventElapsedTime(&ms, lanes_[0].first_event(), lanes_[l].last_event()) == cudaSuccess)
@@ -1405,22 +1350,9 @@ int Decoder::DecodeSharded(const StreamParser* const* streams, int n, const Deco
         const int st = dec->Wait();
         if (st != kSuccess && status == kSuccess) status = Fail(st, dec->last_error());
         const BatchStats& s = dec->stats_;
-        for (int i = 0; i < kStageCount; i++) total.stage_ms[i] += s.stage_ms[i];
+        total.Accumulate(s);
         total.total_ms = std::max(total.total_ms, s.total_ms);
-        total.sync_rounds = std::max(total.sync_rounds, s.sync_rounds);
-        for (int r = 0; r < kMaxSyncRounds; r++) total.decodes_per_round[r] += s.decodes_per_round[r];
-        total.scan_bytes += s.scan_bytes;
-        total.blocks += s.blocks;
-        total.entries += s.entries;
         total.truncated_images += s.truncated_images;
-        total.subsequences += s.subsequences;
-        total.plane_bytes += s.plane_bytes;
-        total.fused_blocks += s.fused_blocks;
-        total.output_bytes += s.output_bytes;
-        total.h2d_bytes += s.h2d_bytes;
-        total.d2h_bytes += s.d2h_bytes;
-        total.kernel_launches += s.kernel_launches;
-        total.sub_bytes = std::max(total.sub_bytes, s.sub_bytes);
         total.lanes += s.lanes;
         total.devices++;
     }

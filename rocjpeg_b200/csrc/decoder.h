@@ -88,11 +88,13 @@ struct BatchStats {
     float host_submit_ms = 0, host_wait_ms = 0;   // host wall time: describing + enqueueing / waiting for the device
     int devices = 1;                    // GPUs the call was sharded over
     uint32_t truncated_images = 0;      // pictures whose scan ended before their last block
+    // adds another lane's or device's counters: sums, and the larger sync_rounds and sub_bytes (not total_ms, lanes,
+    // devices, truncated_images, host_*_ms)
+    void Accumulate(const BatchStats& s);
 };
 
-// Helper threads of one decoder: the lanes of a call are described and enqueued in parallel (kernel
-// launches cost the host ~3 us each and a lane issues about fifteen), the caller's thread taking lane 0.
-// Workers sleep on a condition variable between calls.
+// Helper threads of one decoder: they copy pageable input into page-locked staging, and a sharded call enqueues
+// each device's share from one of them. Workers sleep on a condition variable between calls.
 class SubmitPool {
   public:
     explicit SubmitPool(int workers);
@@ -114,13 +116,6 @@ class SubmitPool {
     bool stop_ = false;
 };
 
-// Order in which concurrent lane submitters may enqueue on the shared upload stream (lane order: the
-// first chunk gets the whole PCIe link, its kernels start while the next chunks are still in flight).
-struct UploadTurn {
-    std::atomic<int>* turn = nullptr;   // null: single submitter, no ordering needed
-    int mine = 0;
-};
-
 // One pipeline lane: a CUDA stream, its device arenas and the description of the
 // (sub-)batch it is decoding. A decode call splits its batch over up to kMaxLanes lanes so
 // that the upload of one chunk overlaps the kernels of another and the latency-bound tails
@@ -135,8 +130,8 @@ class Lane {
     // remote[i] != 0: image i's destination lives on another GPU (stores go over NVLink: rows through the output stage, not the
     // IDCT stage's scattered block stores); nullptr: all local
     int Build(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const uint8_t* remote = nullptr);
-    int Upload(cudaStream_t upload_stream, UploadTurn turn = UploadTurn());   // nullptr: use the lane's own stream
-    int LaunchAll(bool include_upload, int profiling, cudaStream_t upload_stream, UploadTurn turn = UploadTurn());
+    int Upload(cudaStream_t upload_stream);   // nullptr: use the lane's own stream
+    int LaunchAll(bool include_upload, int profiling, cudaStream_t upload_stream);
     int Finish(int profiling);
     int Sync();
     int CopyCoefficients(int image, int16_t* host_out, size_t count);
@@ -157,8 +152,11 @@ class Lane {
   private:
     struct Layout;   // byte layout of the descriptor block
     int Fail(int status, const std::string& why);
-    // the IDCT stage: k2_idct for the full-size pictures, a reduced-size kernel per scale present; returns the launches
+    // the IDCT stage: k2_idct for the full-size pictures, a reduced-size kernel per scale present; counts the launches
     int LaunchIdct(bool force_planes, uint32_t* launches);
+    // Everything after the entropy stage: DC integration (integrate_dc), IDCT, fused IDCT + output, output stage, then
+    // the counters and per-image status back to the host. mark(i) runs after stage i - 1 (LaunchAll's stage events).
+    int LaunchDownstream(bool integrate_dc, const std::function<cudaError_t(int)>& mark);
 
     bool created_ = false;
     std::string err_;
@@ -197,8 +195,12 @@ class Lane {
     K3Args k3_ = {};
     K23Args k23_ = {};
     bool k2_needed_ = true;       // some image of the lane is not served by the fused kernel
-    bool tiles_reduced_ = false;   // the upload kernel left the destuffing pass's per-tile prefix elements
-    bool all_pinned_ = false, any_direct_ = false, needs_planes_ = false;
+    bool any_direct_ = false, needs_planes_ = false;
+    // The kernel schedule, fixed by Build: how the entropy-coded bytes are uploaded (the gather kernel also leaves the
+    // destuffing pass's per-tile prefix elements), and k1_fused or `sync_rounds_` k1_sync rounds up front + k1_write.
+    enum UploadBy { kUploadPerPicture, kUploadRuns, kUploadGather } upload_by_ = kUploadPerPicture;
+    bool k1_fused_ = false;
+    int sync_rounds_ = 2;
     size_t scan_bytes_ = 0, raw_bytes_ = 0, coef_blocks_ = 0, entry_count_ = 0, plane_bytes_ = 0, nsub_total_ = 0;
     uint32_t nseg_total_ = 0;
 
@@ -277,7 +279,7 @@ class Decoder {
     int chunk_first_[kMaxLanes + 1] = {};   // image range of each lane's chunk
     BatchStats stats_;
     // multi-device sharding
-    std::unique_ptr<SubmitPool> pool_;              // lane submitters (ROCJPEG_B200_SUBMIT_THREADS=1)
+    std::unique_ptr<SubmitPool> pool_;              // copiers of pageable input into staging (ROCJPEG_B200_COPY_THREADS)
     std::unique_ptr<SubmitPool> shard_pool_;        // one submitter per peer device
     bool is_peer_ = false;                          // a peer never shards further
     std::vector<std::unique_ptr<Decoder>> peers_;   // decoders on the other devices, owned by the handle's decoder

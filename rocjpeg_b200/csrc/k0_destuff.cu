@@ -516,20 +516,20 @@ __global__ void __launch_bounds__(kThreads) k0_apply(K0Args a) {
 
 }  // namespace
 
-cudaError_t LaunchK0Reduce(const K0Args& a, cudaStream_t stream) {
+cudaError_t LaunchK0Reduce(const K0Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_tiles == 0) return cudaSuccess;
-    return LaunchPdl(k0_reduce, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
+    return LaunchPdl(launches, k0_reduce, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
 }
 
-cudaError_t LaunchGatherReduce(const K0Args& a, const GatherItem* items, cudaStream_t stream) {
+cudaError_t LaunchGatherReduce(const K0Args& a, const GatherItem* items, cudaStream_t stream, uint32_t* launches) {
     if (a.total_tiles == 0) return cudaSuccess;
-    return LaunchPdl(gather_reduce, dim3(min(a.total_tiles, uint32_t(kGatherCtas))), dim3(kThreads), 0, stream, a, items, const_cast<uint8_t*>(a.raw));
+    return LaunchPdl(launches, gather_reduce, dim3(min(a.total_tiles, uint32_t(kGatherCtas))), dim3(kThreads), 0, stream, a, items, const_cast<uint8_t*>(a.raw));
 }
 
-cudaError_t LaunchK0Destuff(const K0Args& a, cudaStream_t stream) {
+cudaError_t LaunchK0Destuff(const K0Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_tiles == 0) return cudaSuccess;
     cudaError_t e = cudaSuccess;
-    if (!a.inline_scan) e = LaunchPdl(k0_scan, dim3(a.nimages), dim3(kThreads), 0, stream, a);
+    if (!a.inline_scan) e = LaunchPdl(launches, k0_scan, dim3(a.nimages), dim3(kThreads), 0, stream, a);
     if (e != cudaSuccess) return e;
     if (getenv("ROCJPEG_B200_DEBUG_SYNC")) {
         e = cudaStreamSynchronize(stream);
@@ -537,9 +537,9 @@ cudaError_t LaunchK0Destuff(const K0Args& a, cudaStream_t stream) {
         if (e != cudaSuccess) return e;
     }
     switch (a.sub_bytes) {
-        case 32: return LaunchPdl(k0_apply<32>, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
-        case 64: return LaunchPdl(k0_apply<64>, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
-        case 128: return LaunchPdl(k0_apply<128>, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
+        case 32: return LaunchPdl(launches, k0_apply<32>, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
+        case 64: return LaunchPdl(launches, k0_apply<64>, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
+        case 128: return LaunchPdl(launches, k0_apply<128>, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
         default: return cudaErrorInvalidValue;
     }
 }

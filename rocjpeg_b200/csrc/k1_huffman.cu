@@ -1366,67 +1366,69 @@ __global__ void k1_clear_short(K1Args a) {
 }
 
 template <int S>
-cudaError_t SyncImpl(const K1Args& a, int round, cudaStream_t stream, int max_iters = T + 1) {
+cudaError_t SyncImpl(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches, int max_iters = T + 1) {
     static_assert(S <= 128, "the packed decoder state holds bit positions below 2048");
     const size_t smem = sizeof(K1Smem<S>) + a.lut_smem_bytes;
     if (smem > 48 * 1024) return cudaErrorInvalidValue;   // 3 table pairs + the full second-level arena fit
-    if (round >= 0) return LaunchPdl(k1_sync<S>, dim3(a.total_ctas), dim3(T), smem, stream, a, round, max_iters);
-    return LaunchPdl(k1_write<S>, dim3(a.total_ctas), dim3(T), smem, stream, a);
+    if (round >= 0) return LaunchPdl(launches, k1_sync<S>, dim3(a.total_ctas), dim3(T), smem, stream, a, round, max_iters);
+    return LaunchPdl(launches, k1_write<S>, dim3(a.total_ctas), dim3(T), smem, stream, a);
 }
 
 }  // namespace
 
-cudaError_t LaunchK1Sync(const K1Args& a, int round, cudaStream_t stream, int max_iters) {
+cudaError_t LaunchK1Sync(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches, int max_iters) {
     if (a.total_ctas == 0) return cudaSuccess;
     if (max_iters <= 0) max_iters = T + 1;
     switch (a.sub_bytes) {
-        case 32: return SyncImpl<32>(a, round, stream, max_iters);
-        case 64: return SyncImpl<64>(a, round, stream, max_iters);
-        case 128: return SyncImpl<128>(a, round, stream, max_iters);
+        case 32: return SyncImpl<32>(a, round, stream, launches, max_iters);
+        case 64: return SyncImpl<64>(a, round, stream, launches, max_iters);
+        case 128: return SyncImpl<128>(a, round, stream, launches, max_iters);
         default: return cudaErrorInvalidValue;
     }
 }
 
-cudaError_t LaunchK1ClearShort(const K1Args& a, cudaStream_t stream) {
+cudaError_t LaunchK1ClearShort(const K1Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.nimages <= 0) return cudaSuccess;
     k1_clear_short<<<dim3((a.nimages + 255) / 256), dim3(256), 0, stream>>>(a);
-    return cudaGetLastError();
+    const cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) ++*launches;
+    return e;
 }
 
-cudaError_t LaunchK1Fused(const K1Args& a, cudaStream_t stream) {
+cudaError_t LaunchK1Fused(const K1Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_ctas == 0) return cudaSuccess;
     const int max_iters = T + 1;
     switch (a.sub_bytes) {
         case 32: { const size_t smem = sizeof(K1Smem<32>) + a.lut_smem_bytes; if (smem > 48 * 1024) return cudaErrorInvalidValue;
-                   return LaunchPdl(k1_fused<32>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
+                   return LaunchPdl(launches, k1_fused<32>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
         case 64: { const size_t smem = sizeof(K1Smem<64>) + a.lut_smem_bytes; if (smem > 48 * 1024) return cudaErrorInvalidValue;
-                   return LaunchPdl(k1_fused<64>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
+                   return LaunchPdl(launches, k1_fused<64>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
         case 128: { const size_t smem = sizeof(K1Smem<128>) + a.lut_smem_bytes; if (smem > 48 * 1024) return cudaErrorInvalidValue;
-                    return LaunchPdl(k1_fused<128>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
+                    return LaunchPdl(launches, k1_fused<128>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
         default: return cudaErrorInvalidValue;
     }
 }
 
-cudaError_t LaunchK1Write(const K1Args& a, cudaStream_t stream) {
+cudaError_t LaunchK1Write(const K1Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_ctas == 0) return cudaSuccess;
     if (!a.inline_scan) {
-        const cudaError_t e = LaunchPdl(k1_scan, dim3(a.nimages), dim3(kScanThreads), 0, stream, a);
+        const cudaError_t e = LaunchPdl(launches, k1_scan, dim3(a.nimages), dim3(kScanThreads), 0, stream, a);
         if (e != cudaSuccess) return e;
     }
     switch (a.sub_bytes) {
-        case 32: return SyncImpl<32>(a, -1, stream);
-        case 64: return SyncImpl<64>(a, -1, stream);
-        case 128: return SyncImpl<128>(a, -1, stream);
+        case 32: return SyncImpl<32>(a, -1, stream, launches);
+        case 64: return SyncImpl<64>(a, -1, stream, launches);
+        case 128: return SyncImpl<128>(a, -1, stream, launches);
         default: return cudaErrorInvalidValue;
     }
 }
 
-cudaError_t LaunchDcScan(const K1Args& a, cudaStream_t stream) {
+cudaError_t LaunchDcScan(const K1Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_dc_tiles == 0) return cudaSuccess;
-    if (a.dc_image) return LaunchPdl(dc_image, dim3(a.nimages), dim3(kDcImageThreads), 0, stream, a);
-    cudaError_t e = LaunchPdl(dc_sums, dim3(a.total_dc_tiles), dim3(kDcTileMcus), 0, stream, a);
-    if (e == cudaSuccess) e = LaunchPdl(dc_scan, dim3(a.nimages), dim3(kScanThreads), 0, stream, a);
-    if (e == cudaSuccess) e = LaunchPdl(dc_apply, dim3(a.total_dc_tiles), dim3(kDcTileMcus), 0, stream, a);
+    if (a.dc_image) return LaunchPdl(launches, dc_image, dim3(a.nimages), dim3(kDcImageThreads), 0, stream, a);
+    cudaError_t e = LaunchPdl(launches, dc_sums, dim3(a.total_dc_tiles), dim3(kDcTileMcus), 0, stream, a);
+    if (e == cudaSuccess) e = LaunchPdl(launches, dc_scan, dim3(a.nimages), dim3(kScanThreads), 0, stream, a);
+    if (e == cudaSuccess) e = LaunchPdl(launches, dc_apply, dim3(a.total_dc_tiles), dim3(kDcTileMcus), 0, stream, a);
     return e;
 }
 

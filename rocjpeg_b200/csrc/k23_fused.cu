@@ -370,10 +370,10 @@ __global__ void __launch_bounds__(kFThreads, 6) k23_warp(K23Args a) {
 
 }  // namespace
 
-cudaError_t LaunchK23Fused(const K23Args& a, cudaStream_t stream) {
+cudaError_t LaunchK23Fused(const K23Args& a, cudaStream_t stream, uint32_t* launches) {
     cudaError_t e = cudaSuccess;
-    if (a.total_tiles_w != 0) e = LaunchPdl(k23_warp, dim3(a.total_tiles_w), dim3(kFThreads), 0, stream, a);
-    if (e == cudaSuccess && a.total_tiles != 0) e = LaunchPdl(k23_fused, dim3(a.total_tiles), dim3(kFThreads), 0, stream, a);
+    if (a.total_tiles_w != 0) e = LaunchPdl(launches, k23_warp, dim3(a.total_tiles_w), dim3(kFThreads), 0, stream, a);
+    if (e == cudaSuccess && a.total_tiles != 0) e = LaunchPdl(launches, k23_fused, dim3(a.total_tiles), dim3(kFThreads), 0, stream, a);
     return e;
 }
 

@@ -172,9 +172,9 @@ __global__ void __launch_bounds__(kThreads, 8) k2_idct(K2Args a) {
 
 }  // namespace
 
-cudaError_t LaunchK2Idct(const K2Args& a, cudaStream_t stream) {
+cudaError_t LaunchK2Idct(const K2Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_tiles == 0) return cudaSuccess;
-    return LaunchPdl(k2_idct, dim3((a.total_tiles + kTilesPerCta - 1) / kTilesPerCta), dim3(kThreads), 0, stream, a);
+    return LaunchPdl(launches, k2_idct, dim3((a.total_tiles + kTilesPerCta - 1) / kTilesPerCta), dim3(kThreads), 0, stream, a);
 }
 
 // Forces the module holding this stage's kernels onto the device (CUDA loads lazily: the first launch

@@ -261,13 +261,13 @@ __global__ void __launch_bounds__(kThreads) k2_idct_1x1(K2Args a) {
 
 }  // namespace
 
-cudaError_t LaunchK2Scaled(const K2Args& a, int scale_denom, cudaStream_t stream) {
+cudaError_t LaunchK2Scaled(const K2Args& a, int scale_denom, cudaStream_t stream, uint32_t* launches) {
     if (a.total_tiles == 0) return cudaSuccess;
     const dim3 grid((a.total_tiles + kTilesPerCta - 1) / kTilesPerCta);
     switch (scale_denom) {
-        case 2: return LaunchPdl(k2_idct_4x4, grid, dim3(kThreads), 0, stream, a);
-        case 4: return LaunchPdl(k2_idct_2x2, grid, dim3(kThreads), 0, stream, a);
-        case 8: return LaunchPdl(k2_idct_1x1, grid, dim3(kThreads), 0, stream, a);
+        case 2: return LaunchPdl(launches, k2_idct_4x4, grid, dim3(kThreads), 0, stream, a);
+        case 4: return LaunchPdl(launches, k2_idct_2x2, grid, dim3(kThreads), 0, stream, a);
+        case 8: return LaunchPdl(launches, k2_idct_1x1, grid, dim3(kThreads), 0, stream, a);
         default: return cudaErrorInvalidValue;
     }
 }

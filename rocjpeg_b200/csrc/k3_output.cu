@@ -185,9 +185,9 @@ __global__ void __launch_bounds__(kThreads) k3_output(K3Args a) {
 
 }  // namespace
 
-cudaError_t LaunchK3Output(const K3Args& a, cudaStream_t stream) {
+cudaError_t LaunchK3Output(const K3Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_tiles == 0) return cudaSuccess;
-    return LaunchPdl(k3_output, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
+    return LaunchPdl(launches, k3_output, dim3(a.total_tiles), dim3(kThreads), 0, stream, a);
 }
 
 // Forces the module holding this stage's kernels onto the device (CUDA loads lazily: the first launch

@@ -10,6 +10,7 @@
 //      (k2_scaled.cu)   its reduced-size forms for decodes at 1/2, 1/4 and 1/8 scale
 //   K3 (k3_output.cu)   the post-processing kernels and copies of
 //                       src/rocjpeg_hip_kernels.cpp / src/rocjpeg_decoder.cpp:372-636
+// Every launcher adds the kernels it actually enqueues to *launches (a launcher with an empty grid enqueues none).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -38,7 +39,7 @@ __device__ __forceinline__ void PdlEntry() {
 }
 
 template <class... KArgs, class... Args>
-inline cudaError_t LaunchPdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
+inline cudaError_t LaunchPdl(uint32_t* launches, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = block;
@@ -49,7 +50,9 @@ inline cudaError_t LaunchPdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, si
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+    if (e == cudaSuccess) ++*launches;
+    return e;
 }
 #endif
 
@@ -96,11 +99,11 @@ struct GatherItem {
     uint32_t pad_;
 };
 // Per-tile prefix elements of the raw bytes already in the arena (cudaMemcpy uploads, resident re-runs) ...
-cudaError_t LaunchK0Reduce(const K0Args& a, cudaStream_t stream);
+cudaError_t LaunchK0Reduce(const K0Args& a, cudaStream_t stream, uint32_t* launches);
 // ... or computed on the way by the kernel that uploads them (items: device array, one per image).
-cudaError_t LaunchGatherReduce(const K0Args& a, const GatherItem* items, cudaStream_t stream);
+cudaError_t LaunchGatherReduce(const K0Args& a, const GatherItem* items, cudaStream_t stream, uint32_t* launches);
 // Scan over the tiles + scatter: destuffed bytes, restart intervals, segment table (two launches).
-cudaError_t LaunchK0Destuff(const K0Args& a, cudaStream_t stream);
+cudaError_t LaunchK0Destuff(const K0Args& a, cudaStream_t stream, uint32_t* launches);
 cudaError_t PreloadK0();
 
 struct K1Args {
@@ -146,15 +149,15 @@ struct K1Args {
 
 // Speculative decode + CTA-local synchronisation (round 0) or cross-CTA fix-up (round >= 1).
 // max_iters bounds the CTA-local fix-up loop (<= 0: until nothing changes).
-cudaError_t LaunchK1Sync(const K1Args& a, int round, cudaStream_t stream, int max_iters = 0);
+cudaError_t LaunchK1Sync(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches, int max_iters = 0);
 // Final pass: positions from the block counts, coefficients and DC differences written.
-cudaError_t LaunchK1Write(const K1Args& a, cudaStream_t stream);
+cudaError_t LaunchK1Write(const K1Args& a, cudaStream_t stream, uint32_t* launches);
 // Both in one kernel (batches whose pictures have at most 256 K1 CTAs, K1Args::fusable); counters[0] = CTA boundaries whose
 // handed-over state was not the owner's: non-zero -> run LaunchK1Sync rounds >= 1 and LaunchK1Write.
-cudaError_t LaunchK1Fused(const K1Args& a, cudaStream_t stream);
-cudaError_t LaunchK1ClearShort(const K1Args& a, cudaStream_t stream);   // before that fallback's LaunchK1Write
+cudaError_t LaunchK1Fused(const K1Args& a, cudaStream_t stream, uint32_t* launches);
+cudaError_t LaunchK1ClearShort(const K1Args& a, cudaStream_t stream, uint32_t* launches);   // before that fallback's LaunchK1Write
 // DC prediction: per-tile sums, then prefix; absolute DC written over the per-block differences.
-cudaError_t LaunchDcScan(const K1Args& a, cudaStream_t stream);
+cudaError_t LaunchDcScan(const K1Args& a, cudaStream_t stream, uint32_t* launches);
 
 struct K2Args {
     const ImageDesc* images;
@@ -168,11 +171,11 @@ struct K2Args {
     int nimages;
     uint32_t total_tiles;
 };
-cudaError_t LaunchK2Idct(const K2Args& a, cudaStream_t stream);
+cudaError_t LaunchK2Idct(const K2Args& a, cudaStream_t stream, uint32_t* launches);
 // Reduced-size IDCT (k2_scaled.cu) for the pictures decoded at scale 1 / scale_denom (2, 4 or 8): every block yields an
 // (8 / scale_denom)-sample square. Same tiles and arguments as LaunchK2Idct; planes, pitches, crop rectangle and the
 // caller's channels are in scaled units.
-cudaError_t LaunchK2Scaled(const K2Args& a, int scale_denom, cudaStream_t stream);
+cudaError_t LaunchK2Scaled(const K2Args& a, int scale_denom, cudaStream_t stream, uint32_t* launches);
 
 // K2 + K3 in one kernel for whole-picture RGB / RGB_PLANAR outputs (OutputDesc::fused): coefficients in, pixels out.
 struct K23Args {
@@ -185,7 +188,7 @@ struct K23Args {
     int nimages;
     uint32_t total_tiles, total_tiles_w;
 };
-cudaError_t LaunchK23Fused(const K23Args& a, cudaStream_t stream);
+cudaError_t LaunchK23Fused(const K23Args& a, cudaStream_t stream, uint32_t* launches);
 cudaError_t PreloadK23();
 
 struct K3Args {
@@ -196,7 +199,7 @@ struct K3Args {
     int nimages;
     uint32_t total_tiles;
 };
-cudaError_t LaunchK3Output(const K3Args& a, cudaStream_t stream);
+cudaError_t LaunchK3Output(const K3Args& a, cudaStream_t stream, uint32_t* launches);
 
 // Load the stages' kernels now instead of at their first launch.
 cudaError_t PreloadK1();

@@ -94,7 +94,6 @@ def main():
         ("lanes3", {"ROCJPEG_B200_LANES": "3"}, steps),
         ("lanes4_equal", {"ROCJPEG_B200_LANES": "4", "ROCJPEG_B200_SPLIT": "25,25,25,25"}, steps),
         ("lanes4_40_30_20_10", {"ROCJPEG_B200_LANES": "4", "ROCJPEG_B200_SPLIT": "40,30,20,10"}, steps),
-        ("lanes4_threads", {"ROCJPEG_B200_SUBMIT_THREADS": "1"}, steps),
         ("nomerge", {"ROCJPEG_B200_NO_MERGE": "1"}, steps),
         ("lanes4_15_30_30_25", {"ROCJPEG_B200_LANES": "4", "ROCJPEG_B200_SPLIT": "15,30,30,25"}, steps),
         ("lanes4_20_35_30_15", {"ROCJPEG_B200_LANES": "4", "ROCJPEG_B200_SPLIT": "20,35,30,15"}, steps),
