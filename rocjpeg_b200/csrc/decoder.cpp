@@ -723,38 +723,33 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     k0_.nimages = n;
     k0_.total_tiles = k0tile;
     k0_.sub_bytes = S;
-    const bool inline_scan_ok = EnvInt("ROCJPEG_B200_NO_INLINE_SCAN", 0) == 0;
     {
         uint32_t most_tiles = 0;
         for (int i = 0; i < n; i++) most_tiles = std::max(most_tiles, h_k0_tile0_[size_t(i) + 1] - h_k0_tile0_[size_t(i)]);
-        k0_.inline_scan = (most_tiles <= 32u && inline_scan_ok) ? 1 : 0;
+        k0_.inline_scan = (most_tiles <= 32u && EnvInt("ROCJPEG_B200_NO_INLINE_SCAN", 0) == 0) ? 1 : 0;
     }
     k1_.rec_fill_vecs = uint32_t((blk * sizeof(BlockRec) + 15) / 16);   // the slab leaves 256 bytes behind every array
     k1_.lut_smem_bytes = max_pairs * 2u * uint32_t(kFastSize) * 4u + max_sub * 4u;
     k1_.total_dc_tiles = dctile;
     k1_.sub_bytes = S;
-    {
-        uint32_t most = 0;
-        for (int i = 0; i < n; i++) most = std::max(most, h_img_cta0_[size_t(i) + 1] - h_img_cta0_[size_t(i)]);
-        k1_.inline_scan = (most <= 32u && inline_scan_ok) ? 1 : 0;
-        k1_.fusable = most <= uint32_t(std::max(0, EnvInt("ROCJPEG_B200_K1_FUSE_CTAS", 256))) ? 1 : 0;
-        uint32_t most_mcus = 0;
-        for (int i = 0; i < n; i++) most_mcus = std::max(most_mcus, uint32_t(h_images_[size_t(i)].total_mcus));
-        // one CTA per picture: a lone picture of 8000 MCUs is faster through the tiled kernels (0.013 against 0.06 ms
-        // for 1920x1080), a lane full of such pictures keeps every SM busy either way and saves two launches
-        const int dc_limit = EnvInt("ROCJPEG_B200_DC_IMAGE_MCUS", n >= 16 ? 2 * kDcImageMaxMcus : kDcImageMaxMcus);
-        k1_.dc_image = (most_mcus <= uint32_t(std::max(0, dc_limit)) && EnvInt("ROCJPEG_B200_NO_DC_IMAGE", 0) == 0) ? 1 : 0;
+    uint32_t most_ctas = 0, most_mcus = 0;
+    for (int i = 0; i < n; i++) {
+        most_ctas = std::max(most_ctas, h_img_cta0_[size_t(i) + 1] - h_img_cta0_[size_t(i)]);
+        most_mcus = std::max(most_mcus, uint32_t(h_images_[size_t(i)].total_mcus));
     }
     // Counting and write pass of the entropy stage in one kernel when no picture has more than 256 K1 CTAs (k1_huffman.cu:
     // k1_fused); ROCJPEG_B200_NO_K1_FUSE=1 or an explicit ROCJPEG_B200_SYNC_ROUNDS keep the separate kernels, with that
     // many k1_sync rounds launched up front.
     const char* rounds_env = std::getenv("ROCJPEG_B200_SYNC_ROUNDS");
     sync_rounds_ = std::min(std::max((rounds_env && *rounds_env) ? std::atoi(rounds_env) : 2, 1), kMaxSyncRounds);
-    k1_fused_ = !rounds_env && EnvInt("ROCJPEG_B200_NO_K1_FUSE", 0) == 0 && k1_.fusable && k1_.total_ctas != 0;
-    // ... and, for pictures small enough for dc_image, it integrates the DC differences itself (no DC launch behind it;
-    // ROCJPEG_B200_NO_K1_DC=1 keeps it). Not for larger ones: a CTA waits there for the picture's earlier CTAs to finish
-    // writing, and with the many CTAs of 4K pictures those waits hold SM slots the next wave needs (c4_dri 3.29 -> 3.65 ms)
-    k1_.k1_dc = k1_fused_ && k1_.dc_image && EnvInt("ROCJPEG_B200_NO_K1_DC", 0) == 0 ? 1 : 0;
+    const bool fusable = most_ctas <= 256u;
+    k1_fused_ = !rounds_env && EnvInt("ROCJPEG_B200_NO_K1_FUSE", 0) == 0 && fusable && k1_.total_ctas != 0;
+    // ... and, for pictures of up to kK1DcMaxMcus MCUs (twice that in a lane of 16 or more pictures; ROCJPEG_B200_DC_IMAGE_MCUS
+    // overrides the limit), it integrates the DC differences itself (no DC launch behind it; ROCJPEG_B200_NO_K1_DC=1 keeps
+    // it). Not for larger ones: a CTA waits there for the picture's earlier CTAs to finish writing, and with the many CTAs
+    // of 4K pictures those waits hold SM slots the next wave needs (c4_dri 3.29 -> 3.65 ms)
+    const int dc_limit = EnvInt("ROCJPEG_B200_DC_IMAGE_MCUS", n >= 16 ? 2 * kK1DcMaxMcus : kK1DcMaxMcus);
+    k1_.k1_dc = k1_fused_ && most_mcus <= uint32_t(std::max(0, dc_limit)) && EnvInt("ROCJPEG_B200_NO_K1_DC", 0) == 0 ? 1 : 0;
     k2_ = K2Args{};
     k2_.nimages = n;
     k2_.total_tiles = k2tile;

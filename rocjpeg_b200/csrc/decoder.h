@@ -62,8 +62,8 @@ enum StageId {
     kStageUpload = 0,   // descriptor block + entropy-coded bytes, host -> device
     kStageDestuff,      // K0: end of slice, destuffing, restart intervals, segment table (three launches)
     kStageSync,         // all k1_sync rounds
-    kStageWrite,        // (k1_scan +) k1_write
-    kStageDc,           // dc_image, or dc_sums + dc_scan + dc_apply
+    kStageWrite,        // k1_scan + k1_write
+    kStageDc,           // dc_sums + dc_scan + dc_apply (none when k1_fused integrates the DC)
     kStageIdct,         // k2_idct and the reduced-size k2_idct_4x4 / 2x2 / 1x1
     kStageOutput,       // k3_output
     kStageCount

@@ -30,21 +30,17 @@
 //                     last round; a non-zero value triggers more rounds
 //                     (correctness never depends on the stream synchronising).
 //   k1_scan           per image: exclusive prefix of the CTAs' block counts
-//                     (segmented at restart intervals) and entry counts. Not launched
-//                     when no picture has more than 32 CTAs: the write pass then sums
-//                     the picture's earlier partials itself.
+//                     (segmented at restart intervals) and entry counts.
 //   k1_write          the final decode: the image's sparse coefficient stream (one
 //                     32-bit (int16 value, zig-zag index) entry per symbol with
 //                     magnitude bits, eight per 256-bit store) and one 8-byte record
 //                     per block {where its entries end, DC difference}.
-//   k1_fused          counting and write pass in one kernel; for pictures dc_image would take, each CTA then also
+//   k1_fused          counting and write pass in one kernel; for pictures of up to kK1DcMaxMcus MCUs, each CTA then also
 //                     integrates the DC of its share of the picture's blocks (IntegrateDc) and no DC kernel runs.
-//   dc_image          pictures up to a few thousand MCUs: per-component, per-restart-
-//                     interval prefix sum of the DC differences, one CTA per picture,
-//                     one launch; the integrated DC replaces the difference in the
-//                     block's record, where K2 reads it.
 //   dc_sums / dc_scan / dc_apply
-//                     the same for large pictures, tiles of 256 MCUs over all SMs.
+//                     per-component, per-restart-interval prefix sum of the DC
+//                     differences in tiles of 256 MCUs over all SMs; the integrated DC
+//                     replaces the difference in the block's record, where K2 reads it.
 #include <cuda_runtime.h>
 
 #include <cstddef>
@@ -696,35 +692,10 @@ __device__ __forceinline__ void WriteBody(const K1Args& a, K1Smem<S>& sm, const 
                 carry_s[1] = ents;
             }
         }
-    } else if (!a.inline_scan) {
-        if (tid == 0) {
-            const uint2 cin = a.cta_carry[cta];
-            carry_s[0] = cin.x;
-            carry_s[1] = cin.y;
-        }
-    } else if (warp == 0) {
-        // at most 32 CTAs per image: one lane per earlier CTA of the image. Entries: plain sum. Blocks: the
-        // partials from the last CTA holding a restart-interval start on (its partial counts only the
-        // blocks after that start).
-        const uint32_t k = __ldg(a.img_cta0 + img) + uint32_t(lane);
-        uint2 part = make_uint2(0u, 0u);
-        uint32_t ents = 0;
-        if (k < cta) {
-            part = a.cta_partial[k];
-            ents = a.cta_entries[k];
-        }
-        const uint32_t starts = __ballot_sync(0xFFFFFFFFu, part.x != 0);
-        const int from = starts ? 31 - __clz(starts) : 0;
-        uint32_t cb = lane >= from ? part.y : 0u;
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) {
-            cb += __shfl_xor_sync(0xFFFFFFFFu, cb, d);
-            ents += __shfl_xor_sync(0xFFFFFFFFu, ents, d);
-        }
-        if (lane == 0) {
-            carry_s[0] = cb;
-            carry_s[1] = ents;
-        }
+    } else if (tid == 0) {
+        const uint2 cin = a.cta_carry[cta];
+        carry_s[0] = cin.x;
+        carry_s[1] = cin.y;
     }
     __syncthreads();
     if (tid == 0) {   // statistics: coefficient entries the batch writes (pads included), read back with the round counters
@@ -1006,8 +977,8 @@ __device__ __forceinline__ int LoadDc(const BlockRec* r) {
 }
 
 // k1_fused, after its write pass: the DC differences of blocks [lo, hi) of the picture (BlockPos) become absolute DC values,
-// the arithmetic of dc_image on a range that need not start on an MCU. Every record of the range is final once this CTA and
-// the one before it have written theirs: the first block's DC symbol may lie in the previous CTA, every other symbol of the
+// the arithmetic of dc_sums / dc_apply on a range that need not start on an MCU. Every record of the range is final once
+// this CTA and the one before it have written theirs: the first block's DC symbol may lie in the previous CTA, every other symbol of the
 // range lies in this one. Each thread sums a contiguous run; a CTA-wide segmented scan and a decoupled look-back over the
 // picture's earlier CTAs (their per-component sums after the last predictor reset, or the predictors leaving them once
 // known) give the predictors entering each run. Every wait is for a lower ticket, i.e. for a running CTA that itself
@@ -1281,83 +1252,6 @@ __global__ void __launch_bounds__(kDcTileMcus) dc_apply(K1Args a) {
               reset_here ? 0 : v2 + a2 - mcu.s2);
 }
 
-// Pictures of a few thousand MCUs (the 500x375 batches): the three launches above are three
-// latencies in a row for a few microseconds of work each. One CTA per picture does it all: chunks of
-// kDcImageThreads MCUs, a segmented scan per chunk, the chunk's last predictors carried to the next.
-constexpr int kDcImageThreads = 512;   // 64 registers per thread (an MCU's ten differences live in registers): two CTAs per SM
-
-__global__ void __launch_bounds__(kDcImageThreads) dc_image(K1Args a) {
-    PdlEntry();
-    constexpr int kWarps = kDcImageThreads / 32;
-    static_assert(kWarps <= 32, "the warp totals are scanned by one warp");
-    __shared__ int wsum[kWarps][3];    // per warp: value of its open segment at the warp's end
-    __shared__ int wflag[kWarps];      // the warp contains a predictor reset
-    __shared__ int wpre[kWarps][3];    // predictors entering the warp (from the chunk's earlier warps and the carry)
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const ImageDesc& im = a.images[blockIdx.x];
-    const int ri = im.restart_interval, bpm = im.bpm;
-    const uint32_t comp_bits = im.comp_bits;
-    const int64_t total = int64_t(im.total_mcus);
-    int c0 = 0, c1 = 0, c2 = 0;   // warp 0: predictors entering the chunk
-    for (int64_t base = 0; base < total; base += kDcImageThreads) {
-        const int64_t m = base + tid;
-        const bool active = m < total;
-        const bool reset_here = active && ResetAt(uint32_t(m), ri);
-        BlockRec* rec = a.blk_rec + im.blk0 + m * bpm;
-        McuDc mcu;
-        mcu.Load(rec, bpm, comp_bits, active);
-        // inclusive segmented scan of the per-MCU sums inside the warp
-        int v0 = mcu.s0, v1 = mcu.s1, v2 = mcu.s2;
-        uint32_t f = reset_here ? 1u : 0u;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const int p0 = __shfl_up_sync(0xFFFFFFFFu, v0, d);
-            const int p1 = __shfl_up_sync(0xFFFFFFFFu, v1, d);
-            const int p2 = __shfl_up_sync(0xFFFFFFFFu, v2, d);
-            const uint32_t pf = __shfl_up_sync(0xFFFFFFFFu, f, d);
-            if (lane >= d) {
-                if (!f) { v0 += p0; v1 += p1; v2 += p2; }
-                f |= pf;
-            }
-        }
-        __syncthreads();   // the previous chunk's readers are done
-        if (lane == 31) { wsum[warp][0] = v0; wsum[warp][1] = v1; wsum[warp][2] = v2; wflag[warp] = int(f); }
-        __syncthreads();
-        if (warp == 0) {
-            // the same scan over the 32 warp totals, with the chunk's carry in front
-            int t0 = 0, t1 = 0, t2 = 0;
-            uint32_t tf = 0;
-            if (lane < kWarps) { t0 = wsum[lane][0]; t1 = wsum[lane][1]; t2 = wsum[lane][2]; tf = uint32_t(wflag[lane]); }
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const int p0 = __shfl_up_sync(0xFFFFFFFFu, t0, d);
-                const int p1 = __shfl_up_sync(0xFFFFFFFFu, t1, d);
-                const int p2 = __shfl_up_sync(0xFFFFFFFFu, t2, d);
-                const uint32_t pf = __shfl_up_sync(0xFFFFFFFFu, tf, d);
-                if (lane >= d) {
-                    if (!tf) { t0 += p0; t1 += p1; t2 += p2; }
-                    tf |= pf;
-                }
-            }
-            if (!tf) { t0 += c0; t1 += c1; t2 += c2; }
-            int x0 = __shfl_up_sync(0xFFFFFFFFu, t0, 1), x1 = __shfl_up_sync(0xFFFFFFFFu, t1, 1), x2 = __shfl_up_sync(0xFFFFFFFFu, t2, 1);
-            if (lane == 0) { x0 = c0; x1 = c1; x2 = c2; }
-            if (lane < kWarps) { wpre[lane][0] = x0; wpre[lane][1] = x1; wpre[lane][2] = x2; }
-            c0 = __shfl_sync(0xFFFFFFFFu, t0, 31);
-            c1 = __shfl_sync(0xFFFFFFFFu, t1, 31);
-            c2 = __shfl_sync(0xFFFFFFFFu, t2, 31);
-        }
-        __syncthreads();
-        if (active) {
-            // exclusive prefix = predictor values entering this MCU
-            const bool open = (f == 0);   // no reset at or before this MCU inside its warp
-            const int p0 = v0 - mcu.s0 + (open ? wpre[warp][0] : 0), p1 = v1 - mcu.s1 + (open ? wpre[warp][1] : 0),
-                      p2 = v2 - mcu.s2 + (open ? wpre[warp][2] : 0);
-            mcu.Store(rec, bpm, comp_bits, reset_here ? 0 : p0, reset_here ? 0 : p1, reset_here ? 0 : p2);
-        }
-    }
-}
-
 // Before the separate kernels redo a batch the fused kernel mis-speculated on: what its write pass reported per picture
 // ("ran out of bytes") came from wrong start states.
 __global__ void k1_clear_short(K1Args a) {
@@ -1366,23 +1260,22 @@ __global__ void k1_clear_short(K1Args a) {
 }
 
 template <int S>
-cudaError_t SyncImpl(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches, int max_iters = T + 1) {
+cudaError_t SyncImpl(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches) {
     static_assert(S <= 128, "the packed decoder state holds bit positions below 2048");
     const size_t smem = sizeof(K1Smem<S>) + a.lut_smem_bytes;
     if (smem > 48 * 1024) return cudaErrorInvalidValue;   // 3 table pairs + the full second-level arena fit
-    if (round >= 0) return LaunchPdl(launches, k1_sync<S>, dim3(a.total_ctas), dim3(T), smem, stream, a, round, max_iters);
+    if (round >= 0) return LaunchPdl(launches, k1_sync<S>, dim3(a.total_ctas), dim3(T), smem, stream, a, round, T + 1);
     return LaunchPdl(launches, k1_write<S>, dim3(a.total_ctas), dim3(T), smem, stream, a);
 }
 
 }  // namespace
 
-cudaError_t LaunchK1Sync(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches, int max_iters) {
+cudaError_t LaunchK1Sync(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches) {
     if (a.total_ctas == 0) return cudaSuccess;
-    if (max_iters <= 0) max_iters = T + 1;
     switch (a.sub_bytes) {
-        case 32: return SyncImpl<32>(a, round, stream, launches, max_iters);
-        case 64: return SyncImpl<64>(a, round, stream, launches, max_iters);
-        case 128: return SyncImpl<128>(a, round, stream, launches, max_iters);
+        case 32: return SyncImpl<32>(a, round, stream, launches);
+        case 64: return SyncImpl<64>(a, round, stream, launches);
+        case 128: return SyncImpl<128>(a, round, stream, launches);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -1411,10 +1304,8 @@ cudaError_t LaunchK1Fused(const K1Args& a, cudaStream_t stream, uint32_t* launch
 
 cudaError_t LaunchK1Write(const K1Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_ctas == 0) return cudaSuccess;
-    if (!a.inline_scan) {
-        const cudaError_t e = LaunchPdl(launches, k1_scan, dim3(a.nimages), dim3(kScanThreads), 0, stream, a);
-        if (e != cudaSuccess) return e;
-    }
+    const cudaError_t e = LaunchPdl(launches, k1_scan, dim3(a.nimages), dim3(kScanThreads), 0, stream, a);
+    if (e != cudaSuccess) return e;
     switch (a.sub_bytes) {
         case 32: return SyncImpl<32>(a, -1, stream, launches);
         case 64: return SyncImpl<64>(a, -1, stream, launches);
@@ -1425,7 +1316,6 @@ cudaError_t LaunchK1Write(const K1Args& a, cudaStream_t stream, uint32_t* launch
 
 cudaError_t LaunchDcScan(const K1Args& a, cudaStream_t stream, uint32_t* launches) {
     if (a.total_dc_tiles == 0) return cudaSuccess;
-    if (a.dc_image) return LaunchPdl(launches, dc_image, dim3(a.nimages), dim3(kDcImageThreads), 0, stream, a);
     cudaError_t e = LaunchPdl(launches, dc_sums, dim3(a.total_dc_tiles), dim3(kDcTileMcus), 0, stream, a);
     if (e == cudaSuccess) e = LaunchPdl(launches, dc_scan, dim3(a.nimages), dim3(kScanThreads), 0, stream, a);
     if (e == cudaSuccess) e = LaunchPdl(launches, dc_apply, dim3(a.total_dc_tiles), dim3(kDcTileMcus), 0, stream, a);
@@ -1450,7 +1340,6 @@ cudaError_t PreloadK1() {
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, dc_sums);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, dc_scan);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, dc_apply);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, dc_image);
     return e;
 }
 

@@ -58,7 +58,7 @@ inline cudaError_t LaunchPdl(uint32_t* launches, void (*kernel)(KArgs...), dim3 
 
 constexpr int kK0TileBytes = 16384;  // raw bytes per destuffing tile (one CTA, 64 bytes per thread) = bytes per gather step
 constexpr int kK1Threads = 128;      // threads per CTA in K1, one subsequence each
-constexpr int kDcImageMaxMcus = 4096;   // pictures up to this many MCUs take the one-launch DC integration
+constexpr int kK1DcMaxMcus = 4096;   // k1_fused integrates the DC of pictures up to this many MCUs (x2 in lanes of 16+)
 // K1Args::halo leading threads of a CTA re-decode the previous CTA's last subsequences; the CTA owns the
 // kK1Threads - halo subsequences behind them (chosen per batch, decoder.cpp)
 constexpr int kDcTileMcus = 256;     // MCUs per DC-scan tile
@@ -139,20 +139,14 @@ struct K1Args {
     uint32_t lut_smem_bytes;      // shared memory for the Huffman tables: 4 KiB per table pair + the second-level arena (batch maximum)
     uint32_t rec_fill_vecs;       // 16-byte vectors of blk_rec that round 0 of k1_sync fills with 0xFF ("never decoded")
     int halo;                     // threads of a CTA that re-decode the subsequences before the CTA's own
-    int inline_scan;              // no image has more than 32 K1 CTAs: k1_write sums the partials of the image's earlier CTAs
-                                  // itself (one warp, one load each) and k1_scan is not launched
-    int fusable;                  // no image has more than 256 K1 CTAs: counting and write pass may run as one kernel (k1_fused)
-    int dc_image;                 // no image has more than kDcImageMaxMcus MCUs: one CTA per image integrates its DC
-                                  // differences in ONE launch (dc_image) instead of sums / scan / apply
     int k1_dc;                    // k1_fused integrates the DC differences itself: LaunchDcScan is not needed after it
 };
 
 // Speculative decode + CTA-local synchronisation (round 0) or cross-CTA fix-up (round >= 1).
-// max_iters bounds the CTA-local fix-up loop (<= 0: until nothing changes).
-cudaError_t LaunchK1Sync(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches, int max_iters = 0);
-// Final pass: positions from the block counts, coefficients and DC differences written.
+cudaError_t LaunchK1Sync(const K1Args& a, int round, cudaStream_t stream, uint32_t* launches);
+// Final pass: k1_scan (positions from the block counts), then k1_write (coefficients and DC differences written).
 cudaError_t LaunchK1Write(const K1Args& a, cudaStream_t stream, uint32_t* launches);
-// Both in one kernel (batches whose pictures have at most 256 K1 CTAs, K1Args::fusable); counters[0] = CTA boundaries whose
+// Both in one kernel (batches whose pictures have at most 256 K1 CTAs); counters[0] = CTA boundaries whose
 // handed-over state was not the owner's: non-zero -> run LaunchK1Sync rounds >= 1 and LaunchK1Write.
 cudaError_t LaunchK1Fused(const K1Args& a, cudaStream_t stream, uint32_t* launches);
 cudaError_t LaunchK1ClearShort(const K1Args& a, cudaStream_t stream, uint32_t* launches);   // before that fallback's LaunchK1Write

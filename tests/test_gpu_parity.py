@@ -159,13 +159,14 @@ def test_every_halo_width(dec, orc, halo, monkeypatch):
         gu.assert_same(got, want, f"{name} halo={halo}")
 
 
-@pytest.mark.parametrize("knobs", [{}, {"ROCJPEG_B200_NO_INLINE_SCAN": "1"}, {"ROCJPEG_B200_NO_DC_IMAGE": "1"},
-                                   {"ROCJPEG_B200_NO_INLINE_SCAN": "1", "ROCJPEG_B200_NO_DC_IMAGE": "1"}])
+@pytest.mark.parametrize("knobs", [{}, {"ROCJPEG_B200_NO_INLINE_SCAN": "1"}, {"ROCJPEG_B200_NO_K1_DC": "1"},
+                                   {"ROCJPEG_B200_NO_INLINE_SCAN": "1", "ROCJPEG_B200_NO_K1_DC": "1"}])
 def test_small_and_large_picture_scan_paths_agree(dec, orc, knobs, monkeypatch):
-    """Batches of small pictures fold the CTA-offset scan into the write pass and integrate the DC
-    differences in one launch per picture; large pictures (and the knobs here) take the separate scan
-    kernels. Both must be exact, with and without restart intervals, and a picture above the one-launch
-    limits (2048x1536 4:4:4: 49 152 MCUs, > 32 K1 CTAs) must leave the small-picture paths by itself."""
+    """Batches of small pictures fold the destuffing stage's tile scan into its scatter pass and integrate
+    the DC differences inside the fused entropy kernel; large pictures (and the knobs here) take the separate
+    scan kernels and the tiled DC kernels. Both must be exact, with and without restart intervals, and a
+    picture above the small-picture limits (2048x1536 4:4:4: 49 152 MCUs) must leave the small-picture paths
+    by itself."""
     for k, v in knobs.items():
         monkeypatch.setenv(k, v)
     for name in ("synth_420_500x375_dri7", "synth_444_500x375", "synth_422_500x375", "synth_400_333x211", "mug_422_crop_dri1"):

@@ -1,5 +1,5 @@
 """The fused entropy kernel (k1_fused) integrates the DC differences of its own share of each picture's blocks; the DC kernels
-(dc_image, or dc_sums / dc_scan / dc_apply) are then not launched. ROCJPEG_B200_NO_K1_DC=1 keeps them. Both schedules must
+(dc_sums / dc_scan / dc_apply) are then not launched. ROCJPEG_B200_NO_K1_DC=1 keeps them. Both schedules must
 give the same bytes and the same per-image status on every path that follows the entropy stage."""
 import os
 
@@ -108,7 +108,7 @@ def test_restart_intervals_and_crops_that_skip_them(dec, orc, css, S, monkeypatc
 
 
 def test_pictures_above_the_one_launch_dc_limit(dec, orc, monkeypatch):
-    """k1_fused integrates the DC of the pictures dc_image would take: up to 8192 MCUs in a batch of 16 or more (720x576
+    """k1_fused integrates the DC of pictures up to 4096 MCUs, up to 8192 MCUs in a batch of 16 or more (720x576
     4:4:4, 6480 MCUs), any size when ROCJPEG_B200_DC_IMAGE_MCUS raises that limit (2048x1536, 49 152 MCUs)."""
     mid = [datagen.make_jpeg(720, 576, "444", seed=60 + i, restart_mcus=(0, 45, 90)[i % 3]) for i in range(16)]
     on, off = _same_both_ways(dec, orc, mid, "rgb_planar", monkeypatch, "16 x 720x576")
