@@ -52,7 +52,7 @@ typedef struct {
     uint32_t truncated_images;                /* pictures of the last call whose scan ended before their last block */
     uint32_t pad_;
     uint64_t fused_blocks;                    /* blocks transformed by the fused IDCT + output kernel (whole-picture RGB / RGB_PLANAR):
-                                                 their planes never reach memory; ROCJPEG_B200_NO_FUSE=1 disables the fusion */
+                                                 their planes never reach memory */
 } RocJpegB200Stats;
 
 /* CUDA-event timing on a decoder handle: 0 off (default), 1 an event after every stage (stage_ms and total_ms;

@@ -423,10 +423,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
 
     any_direct_ = false;
     needs_planes_ = false;
-    const bool direct_ok = EnvInt("ROCJPEG_B200_NO_DIRECT", 0) == 0;
-    const bool fuse_ok = EnvInt("ROCJPEG_B200_NO_FUSE", 0) == 0;
     uint32_t k23tile = 0, k23tile_w = 0;
-    const bool warp_ok = EnvInt("ROCJPEG_B200_NO_WARP_FUSE", 0) == 0;
     k2_needed_ = false;
     uint64_t scan_off = 0, raw_off = 0, blk = 0, plane_off = 0, ent = 0, sub = 0;
     uint32_t dctile = 0, k2tile = 0, k3tile = 0, max_pairs = 1, max_sub = 0, k0tile = 0, nseg_total = 0;
@@ -638,10 +635,10 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
         const bool whole = od.x0 == 0 && od.y0 == 0 && od.w == out_w && od.h == out_h;
         const bool planar = od.fmt == FMT_Y || od.fmt == FMT_YUV_PLANAR ||
                             (od.fmt == FMT_NATIVE && (p.css == CSS_444 || p.css == CSS_440 || p.css == CSS_411 || p.css == CSS_400));
-        od.direct = (whole && planar && direct_ok && !(remote && remote[i])) ? 1 : 0;
+        od.direct = (whole && planar && !(remote && remote[i])) ? 1 : 0;
         // Whole-picture RGB / RGB_PLANAR: IDCT and colour conversion in one kernel, the planes never leave shared memory
         // (full size only: a scaled picture goes reduced-size IDCT -> plane arena -> output stage)
-        od.fused = (d == 1 && whole && fuse_ok && (od.fmt == FMT_RGB || od.fmt == FMT_RGB_PLANAR) && h_fused_.size() < 65535) ? 1 : 0;
+        od.fused = (d == 1 && whole && (od.fmt == FMT_RGB || od.fmt == FMT_RGB_PLANAR) && h_fused_.size() < 65535) ? 1 : 0;
         const bool tiles = !od.direct && !od.fused;
         od.tiles_x = tiles ? uint32_t((od.w + kK3TileW - 1) / kK3TileW) : 0u;
         od.tiles_y = tiles ? uint32_t((od.h + kK3TileH - 1) / kK3TileH) : 0u;
@@ -663,7 +660,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
             // destination rows all 4-byte aligned (every row takes the register path): the warp-per-column kernel
             bool aligned = (od.dst_pitch[0] & 3u) == 0;
             for (int c = 0; c < (od.fmt == FMT_RGB ? 1 : 3); c++) aligned = aligned && (reinterpret_cast<uintptr_t>(od.dst[c]) & 3u) == 0;
-            aligned = aligned && warp_ok && (fi.mpt / 8) * p.bpm <= 16;   // a warp's MCUs hold at most 16 blocks (k23_fused.cu)
+            aligned = aligned && (fi.mpt / 8) * p.bpm <= 16;   // a warp's MCUs hold at most 16 blocks (k23_fused.cu)
             // a destination on another GPU: the strip kernel's rows cross NVLink as 256-pixel segments, the warp kernel's as 32-byte ones
             if (remote && remote[i]) aligned = false;
             fi.tile0 = aligned ? k23tile_w : k23tile;
@@ -1471,9 +1468,8 @@ int Lane::CopyCoefficients(int image, int16_t* host_out, size_t count) {
     RJB_CUDA(cudaMemcpy(recs.data(), k1_.blk_rec + im.blk0, recs.size() * sizeof(BlockRec), cudaMemcpyDeviceToHost));
     RJB_CUDA(cudaMemcpy(ents.data(), k1_.entries + im.ent0, ents.size() * 4, cudaMemcpyDeviceToHost));
     for (size_t b = 0; b < recs.size(); b++) {
-        uint32_t e0 = b ? recs[b - 1].end : 0u, e1 = recs[b].end;   // a block's entries begin where its predecessor's end
-        if (e0 == kNoEntry || e1 == kNoEntry || e1 < e0 || e1 - e0 > 0xFFFFu || e1 > im.ent_cap) e0 = e1 = 0;   // as K2
-        for (uint32_t k = e0; k < e1; k++) tmp[b * 64 + kZz[CoefEntryPos(ents[k])]] = int16_t(ents[k] & 0xFFFFu);
+        const uint2 e = BlockEntryRange(b ? recs[b - 1].end : 0u, recs[b].end, im.ent_cap);
+        for (uint32_t k = e.x; k < e.y; k++) tmp[b * 64 + kZz[CoefEntryPos(ents[k])]] = int16_t(ents[k] & 0xFFFFu);
         tmp[b * 64] = recs[b].dc;   // integrated DC lives in the block's record
     }
     size_t base = 0;

@@ -26,36 +26,12 @@ constexpr int kMaxBlocks = 128;       // blocks of one strip: 32 MCUs x 4 (4:4:0
 constexpr int kLumaBytes = 16 * kStripW, kChromaBytes = 8 * kStripW;   // plane capacities: 16 rows of luma; 8 x 256 or 16 x 128 of chroma
 static_assert(kStripW == kTileW, "the row routines assume 8 samples per lane over the strip");
 
-// shared memory through 32-bit window addresses (computed once: the generic-pointer forms made the compiler rebuild
-// the window base in every iteration of the issue-bound IDCT loop)
-__device__ __forceinline__ uint32_t SharedU32(const void* p) {
-    uint32_t a = uint32_t(__cvta_generic_to_shared(p));
-    asm volatile("mov.u32 %0, %0;" : "+r"(a));   // opaque: keeps the address in a register instead of re-deriving the window base
-    return a;
-}
-__device__ __forceinline__ uint32_t Lds32(uint32_t a) {
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ uint4 Lds128(uint32_t a) {
-    uint4 v;
-    asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ void Sts32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ void Sts64(uint32_t a, uint32_t x, uint32_t y) { asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(a), "r"(x), "r"(y) : "memory"); }
-__device__ __forceinline__ void Sts128(uint32_t a, uint4 v) {
-    asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-
 __global__ void __launch_bounds__(kFThreads, 6) k23_fused(K23Args a) {
     PdlEntry();
-    constexpr int kRS = 12, kBS = 104;   // workspace strides as in k2_idct.cu (bank-conflict free column / row access)
     __shared__ __align__(16) int ws[32 * kBS];
     __shared__ __align__(16) uint8_t s_pl[kLumaBytes + 2 * kChromaBytes];
     __shared__ __align__(16) uint8_t s_buf[kFThreads / 32][kRowBuf];
-    __shared__ uint32_t s_tab[3][64];            // per component and zig-zag code: workspace byte offset | quantiser step << 16
+    __shared__ uint32_t s_tab[3][64];            // per component and zig-zag code: TabEntry
     // per block of the strip: {first entry, entries | component << 16 | valid << 24, dequantised DC, plane offset | pitch << 16}
     __shared__ __align__(16) uint4 s_meta[kMaxBlocks];
     __shared__ K3Job s_job;
@@ -93,11 +69,8 @@ __global__ void __launch_bounds__(kFThreads, 6) k23_fused(K23Args a) {
     }
     // quantiser / offset tables per component
     for (int idx = tid; idx < ncomp * 64; idx += kFThreads) {
-        const int c = idx >> 6, code = idx & 63;   // entries carry position + 1 (huff_core.cuh)
-        const int nat = kZigzag[(code + 63) & 63];
-        // (code 1 = position 0: DC-difference and pad entries; the block's integrated DC is stored with the zero fill, so these
-        // are parked in a padding word of the workspace's first row)
-        s_tab[c][code] = uint32_t(code == 1 ? 8 * 4 : ((nat >> 3) * kRS + (nat & 7)) * 4) | (uint32_t(__ldg(a.qtables + size_t(fi.qidx[c]) * 64 + nat)) << 16);
+        const int c = idx >> 6, code = idx & 63;
+        s_tab[c][code] = TabEntry(code, a.qtables + size_t(fi.qidx[c]) * 64);
     }
     // per block of the strip: its record (where its entries lie, integrated DC) and where its samples go
     if (tid < kMaxBlocks) {
@@ -109,19 +82,18 @@ __global__ void __launch_bounds__(kFThreads, 6) k23_fused(K23Args a) {
             const int H = fi.H[c];
             const size_t blk = size_t(mrow * fi.mcus_x + m0 + (bx >> fi.hshift[c])) * size_t(fi.bpm) + size_t(fi.first_blk[c] + v * H + (bx & (H - 1)));
             const uint2 r = __ldg(reinterpret_cast<const uint2*>(rec + blk));
-            uint32_t e0 = blk ? __ldg(&rec[blk - 1].end) : 0u, e1 = r.x;
-            if (e0 == kNoEntry || e1 == kNoEntry || e1 < e0 || e1 - e0 > 0xFFFFu || e1 > fi.ent_cap) e1 = e0 = 0;   // never decoded (as k2_idct.cu)
-            m.x = e0;
-            m.y = (e1 - e0) | (uint32_t(c) << 16) | (1u << 24);
+            const uint2 e = BlockEntryRange(blk ? __ldg(&rec[blk - 1].end) : 0u, r.x, fi.ent_cap);
+            m.x = e.x;
+            m.y = (e.y - e.x) | (uint32_t(c) << 16) | (1u << 24);
             m.z = uint32_t(int(int16_t(r.y & 0xFFFFu)) * int(__ldg(a.qtables + size_t(fi.qidx[c]) * 64)));   // integrated DC, dequantised
             m.w = (fi.base[c] + uint32_t(v * 8) * fi.pitch[c] + uint32_t(bx * 8)) | (fi.pitch[c] << 16);
         }
         s_meta[tid] = m;
     }
     __syncthreads();
-    // ---- IDCT: 32 blocks at a time, 8 threads per block (k2_idct.cu's arithmetic, samples to shared memory). The loop is
-    // issue bound: everything it touches is addressed through 32-bit shared-window addresses computed once, a block's
-    // description is one 128-bit load, and the trip count is the same for every warp.
+    // ---- IDCT: 32 blocks at a time, 8 threads per block, samples to shared memory. The loop is issue bound: everything it
+    // touches is addressed through 32-bit shared-window addresses computed once, a block's description is one 128-bit load,
+    // and the trip count is the same for every warp.
     const int b = tid >> 3, jj = tid & 7;
     const uint32_t my_sa = SharedU32(ws) + uint32_t(b * kBS * 4);
     const uint32_t row_sa = my_sa + uint32_t(jj * kRS * 4), col_sa = my_sa + uint32_t(jj * 4);
@@ -132,40 +104,10 @@ __global__ void __launch_bounds__(kFThreads, 6) k23_fused(K23Args a) {
 #pragma unroll 1
     for (; meta_sa < meta_end + uint32_t(b * 16); meta_sa += 32 * 16) {   // (same trip count for the 32 block slots: slot b's g runs b, b + 32, ...)
         const uint4 m = Lds128(meta_sa);
-        const uint32_t n = m.y & 0xFFFFu;
-        const uint32_t* ep = ent_j + m.x;
-        // four loads in flight per thread (32 entries per block) before the first is used
-        const uint32_t k = uint32_t(jj);
-        uint32_t e[4];
-#pragma unroll
-        for (int u = 0; u < 4; u++) e[u] = (k + 8u * u < n) ? __ldg(ep + 8 * u) : 0u;
-        Sts128(row_sa, make_uint4(jj == 0 ? m.z : 0u, 0u, 0u, 0u));   // zero fill; the integrated DC goes in with it
-        Sts128(row_sa + 16, make_uint4(0u, 0u, 0u, 0u));
-        __syncwarp();
-        const uint32_t tab_sa = tab_sa0 + ((m.y >> 8) & 0x300u);
-        auto put = [&](uint32_t en) {
-            const uint32_t t = Lds32(tab_sa + ((en >> 14) & 0xFCu));
-            Sts32(my_sa + (t & 0xFFFFu), uint32_t(int(int16_t(en & 0xFFFFu)) * int(t >> 16)));
-        };
-#pragma unroll
-        for (int u = 0; u < 4; u++)
-            if (k + 8u * u < n) put(e[u]);
-        for (uint32_t kk = k + 32u; kk < n; kk += 8) put(__ldg(ep + (kk - k)));
-        __syncwarp();
-        int in[8], out[8];
-#pragma unroll
-        for (int r = 0; r < 8; r++) in[r] = int(Lds32(col_sa + uint32_t(r * kRS * 4)));   // column jj
-        Islow8<11>(in, out, 1 << 10);
-#pragma unroll
-        for (int r = 0; r < 8; r++) Sts32(col_sa + uint32_t(r * kRS * 4), uint32_t(out[r]));
-        __syncwarp();
-        {
-            const uint4 lo = Lds128(row_sa), hi = Lds128(row_sa + 16);   // row jj
-            in[0] = int(lo.x); in[1] = int(lo.y); in[2] = int(lo.z); in[3] = int(lo.w);
-            in[4] = int(hi.x); in[5] = int(hi.y); in[6] = int(hi.z); in[7] = int(hi.w);
-            Islow8<18>(in, out, (1 << 17) + (128 << 18));
-            if (m.y >> 24) Sts64(pl_sa + (m.w & 0xFFFFu) + uint32_t(jj) * (m.w >> 16), PackSat4(out[0], out[1], out[2], out[3]), PackSat4(out[4], out[5], out[6], out[7]));
-        }
+        ScatterColumns(my_sa, row_sa, col_sa, jj, tab_sa0, (m.y >> 8) & 0x300u, ent_j + m.x, m.y & 0xFFFFu, m.z);
+        int out[8];
+        RowPass(row_sa, out);
+        if (m.y >> 24) Sts64(pl_sa + (m.w & 0xFFFFu) + uint32_t(jj) * (m.w >> 16), PackRow(out));
         __syncwarp();
     }
     __syncthreads();
@@ -209,14 +151,13 @@ constexpr int kWarpBlocks = 16;            // blocks under them at most ((2x2, 1
 constexpr int kWarpLuma = kWarpW * 16, kWarpChroma = 256;   // plane capacities: 32 x 16 luma; 32 x 8, 16 x 16 or 8 x 8 chroma
 
 struct __align__(16) WarpSmem {
-    int ws[4 * 104];                       // four blocks in flight (strides as above)
+    int ws[4 * kBS];                       // four blocks in flight
     uint4 meta[kWarpBlocks];
     uint8_t pl[kWarpLuma + 2 * kWarpChroma];
 };
 
 __global__ void __launch_bounds__(kFThreads, 6) k23_warp(K23Args a) {
     PdlEntry();
-    constexpr int kRS = 12, kBS = 104;
     __shared__ WarpSmem s_w[kFThreads / 32];
     __shared__ uint32_t s_tab[3][64];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -231,8 +172,7 @@ __global__ void __launch_bounds__(kFThreads, 6) k23_warp(K23Args a) {
         const int ncomp_g = gfi.ncomp;
         for (int idx = tid; idx < ncomp_g * 64; idx += kFThreads) {
             const int c = idx >> 6, code = idx & 63;
-            const int nat = kZigzag[(code + 63) & 63];
-            s_tab[c][code] = uint32_t(code == 1 ? 8 * 4 : ((nat >> 3) * kRS + (nat & 7)) * 4) | (uint32_t(__ldg(a.qtables + size_t(gfi.qidx[c]) * 64 + nat)) << 16);
+            s_tab[c][code] = TabEntry(code, a.qtables + size_t(gfi.qidx[c]) * 64);
         }
     }
     __syncthreads();
@@ -262,12 +202,11 @@ __global__ void __launch_bounds__(kFThreads, 6) k23_warp(K23Args a) {
                 const uint32_t blk = uint32_t(mrow * mcus_x + m0 + (bx >> (ci >> 24))) * uint32_t(fi.bpm) + ((ci >> 16) & 0xFFu) + uint32_t(v) * H + (uint32_t(bx) & (H - 1u));
                 const BlockRec* rp = a.blk_rec + fi.blk0 + blk;
                 const uint2 r = __ldg(reinterpret_cast<const uint2*>(rp));
-                uint32_t e0 = blk ? __ldg(&rp[-1].end) : 0u, e1 = r.x;
-                if (e0 == kNoEntry || e1 == kNoEntry || e1 < e0 || e1 - e0 > 0xFFFFu || e1 > fi.ent_cap) e1 = e0 = 0;   // never decoded
+                const uint2 e = BlockEntryRange(blk ? __ldg(&rp[-1].end) : 0u, r.x, fi.ent_cap);
                 const uint32_t pitch = uint32_t(8 * mpw) * H;                       // 32 for luma, 32 >> sx for chroma
                 const uint32_t base = c == 0 ? 0u : uint32_t(kWarpLuma + (c - 1) * kWarpChroma);
-                m.x = e0;
-                m.y = (e1 - e0) | (uint32_t(c) << 16) | (1u << 24);
+                m.x = e.x;
+                m.y = (e.y - e.x) | (uint32_t(c) << 16) | (1u << 24);
                 m.z = uint32_t(int(int16_t(r.y & 0xFFFFu)) * int(s_tab[c][1] >> 16));   // integrated DC, dequantised (code 1 = position 0)
                 m.w = (base + uint32_t(v * 8) * pitch + uint32_t(bx * 8)) | (pitch << 16);
             }
@@ -287,39 +226,10 @@ __global__ void __launch_bounds__(kFThreads, 6) k23_warp(K23Args a) {
 #pragma unroll 1
         for (; meta_sa < meta_end; meta_sa += 4 * 16) {
             const uint4 m = Lds128(meta_sa);
-            const uint32_t n = m.y & 0xFFFFu;
-            const uint32_t* ep = ent_j + m.x;
-            const uint32_t k = uint32_t(jj);
-            uint32_t e[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) e[u] = (k + 8u * u < n) ? __ldg(ep + 8 * u) : 0u;
-            Sts128(row_sa, make_uint4(jj == 0 ? m.z : 0u, 0u, 0u, 0u));
-            Sts128(row_sa + 16, make_uint4(0u, 0u, 0u, 0u));
-            __syncwarp();
-            const uint32_t tab_sa = tab_sa0 + ((m.y >> 8) & 0x300u);
-            auto put = [&](uint32_t en) {
-                const uint32_t tt = Lds32(tab_sa + ((en >> 14) & 0xFCu));
-                Sts32(my_sa + (tt & 0xFFFFu), uint32_t(int(int16_t(en & 0xFFFFu)) * int(tt >> 16)));
-            };
-#pragma unroll
-            for (int u = 0; u < 4; u++)
-                if (k + 8u * u < n) put(e[u]);
-            for (uint32_t kk = k + 32u; kk < n; kk += 8) put(__ldg(ep + (kk - k)));
-            __syncwarp();
-            int in[8], out[8];
-#pragma unroll
-            for (int r = 0; r < 8; r++) in[r] = int(Lds32(col_sa + uint32_t(r * kRS * 4)));
-            Islow8<11>(in, out, 1 << 10);
-#pragma unroll
-            for (int r = 0; r < 8; r++) Sts32(col_sa + uint32_t(r * kRS * 4), uint32_t(out[r]));
-            __syncwarp();
-            {
-                const uint4 lo = Lds128(row_sa), hi = Lds128(row_sa + 16);
-                in[0] = int(lo.x); in[1] = int(lo.y); in[2] = int(lo.z); in[3] = int(lo.w);
-                in[4] = int(hi.x); in[5] = int(hi.y); in[6] = int(hi.z); in[7] = int(hi.w);
-                Islow8<18>(in, out, (1 << 17) + (128 << 18));
-                if (m.y >> 24) Sts64(pl_sa + (m.w & 0xFFFFu) + uint32_t(jj) * (m.w >> 16), PackSat4(out[0], out[1], out[2], out[3]), PackSat4(out[4], out[5], out[6], out[7]));
-            }
+            ScatterColumns(my_sa, row_sa, col_sa, jj, tab_sa0, (m.y >> 8) & 0x300u, ent_j + m.x, m.y & 0xFFFFu, m.z);
+            int out[8];
+            RowPass(row_sa, out);
+            if (m.y >> 24) Sts64(pl_sa + (m.w & 0xFFFFu) + uint32_t(jj) * (m.w >> 16), PackRow(out));
             __syncwarp();
         }
     }

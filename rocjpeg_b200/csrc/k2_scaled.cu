@@ -102,16 +102,9 @@ __device__ __forceinline__ void ScaledBody(const K2Args& a) {
     // dump word for positions the transform ignores) and its quantiser step (high half)
     __shared__ uint32_t s_tab[kTilesPerCta][64];
     __shared__ uint32_t s_tile0[kSearchCache];
-    // per tile and block: {first entry, entries | valid << 24, dequantised integrated DC, -}
-    __shared__ __align__(16) uint4 s_meta[kTilesPerCta][kBlocksPerTile];
+    __shared__ __align__(16) uint4 s_meta[kTilesPerCta][kBlocksPerTile];   // per tile and block: TileBlockMeta
     const int tid = threadIdx.x;
-    const bool cached = a.nimages <= kSearchCache;
-    if (cached) {
-        for (int i = tid; i < a.nimages; i += kThreads) s_tile0[i] = __ldg(a.img_tile0 + i);
-        __syncthreads();
-    }
-    if (tid < kTilesPerCta) s_tile[tid] = ResolveTile<S>(a, cached ? s_tile0 : nullptr, blockIdx.x * kTilesPerCta + tid);
-    __syncthreads();
+    ResolveCtaTiles<S, kThreads, kTilesPerCta>(a, s_tile, s_tile0);
     for (int idx = tid; idx < kTilesPerCta * 64; idx += kThreads) {
         const int t = idx >> 6, code = idx & 63;   // entries carry position + 1 (huff_core.cuh)
         const TileInfo& ti = s_tile[t];
@@ -123,22 +116,10 @@ __device__ __forceinline__ void ScaledBody(const K2Args& a) {
             s_tab[t][code] = uint32_t(word * 4) | (uint32_t(__ldg(ti.qt + nat)) << 16);
         }
     }
-    // block records of all the CTA's tiles, as k2_idct
+    // block records of all the CTA's tiles
     for (int idx = tid; idx < kTilesPerCta * kBlocksPerTile; idx += kThreads) {
         const int t = idx >> 5, bb = idx & 31;
-        const TileInfo& ti = s_tile[t];
-        uint4 m = make_uint4(0u, 0u, 0u, 0u);
-        if (ti.nbx >= 0 && ti.direct != 2 && ti.bx0 + bb < ti.nbx) {
-            const int bx = ti.bx0 + bb;
-            const size_t blk = size_t(ti.row_mcu + uint32_t(bx >> ti.hshift)) * uint32_t(ti.bpm) + ti.k_row + uint32_t(bx & ti.hmask);
-            const uint2 r = __ldg(reinterpret_cast<const uint2*>(ti.rec + blk));
-            uint32_t e0 = blk ? __ldg(&ti.rec[blk - 1].end) : 0u, e1 = r.x;
-            if (e0 == kNoEntry || e1 == kNoEntry || e1 < e0 || e1 - e0 > 0xFFFFu || e1 > ti.ent_cap) e1 = e0 = 0;   // never decoded
-            m.x = e0;
-            m.y = (e1 - e0) | (1u << 24);
-            m.z = uint32_t(int(int16_t(r.y & 0xFFFFu)) * int(__ldg(ti.qt)));   // integrated DC, dequantised
-        }
-        s_meta[t][bb] = m;
+        s_meta[t][bb] = TileBlockMeta(s_tile[t], bb);
     }
     __syncthreads();
     const int group = tid / (kBlocksPerTile * kTpb), gt = tid % (kBlocksPerTile * kTpb);
@@ -238,13 +219,7 @@ __global__ void __launch_bounds__(kThreads) k2_idct_1x1(K2Args a) {
     __shared__ TileInfo s_tile[kTilesPerCta];
     __shared__ uint32_t s_tile0[kSearchCache];
     const int tid = threadIdx.x;
-    const bool cached = a.nimages <= kSearchCache;
-    if (cached) {
-        for (int i = tid; i < a.nimages; i += kThreads) s_tile0[i] = __ldg(a.img_tile0 + i);
-        __syncthreads();
-    }
-    if (tid < kTilesPerCta) s_tile[tid] = ResolveTile<1>(a, cached ? s_tile0 : nullptr, blockIdx.x * kTilesPerCta + tid);
-    __syncthreads();
+    ResolveCtaTiles<1, kThreads, kTilesPerCta>(a, s_tile, s_tile0);
     const int bb = tid & 31;
 #pragma unroll 1
     for (int it = tid >> 5; it < kTilesPerCta; it += kThreads / 32) {
@@ -252,8 +227,7 @@ __global__ void __launch_bounds__(kThreads) k2_idct_1x1(K2Args a) {
         if (ti.nbx < 0) break;
         const int bx = ti.bx0 + bb;
         if (ti.direct == 2 || bx >= ti.nbx) continue;
-        const size_t blk = size_t(ti.row_mcu + uint32_t(bx >> ti.hshift)) * uint32_t(ti.bpm) + ti.k_row + uint32_t(bx & ti.hmask);
-        const int dc = int(__ldg(&ti.rec[blk].dc)) * int(__ldg(ti.qt));
+        const int dc = int(__ldg(&ti.rec[TileBlock(ti, bx)].dc)) * int(__ldg(ti.qt));
         const uint32_t v = PackSat4((dc + 4 + (128 << 3)) >> 3, 0, 0, 0);
         if (!ti.direct || bx < ti.clip_w) ti.out[bx] = uint8_t(v);
     }

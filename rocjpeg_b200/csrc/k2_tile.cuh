@@ -1,37 +1,16 @@
-// k2_tile.cuh — what the IDCT kernels share: the tile -> picture / component resolution and the shared-memory
-// access helpers. The full-size kernel (k2_idct.cu) and the reduced-size kernels (k2_scaled.cu) cut a component
+// k2_tile.cuh — what the IDCT kernels share: the tile -> picture / component resolution and the records of a
+// tile's blocks. The full-size kernel (k2_idct.cu) and the reduced-size kernels (k2_scaled.cu) cut a component
 // into the same tiles: 32 horizontally adjacent blocks of one block row. They differ in how many samples a block
 // yields per row and column: S = 8 at full size, 8 / d at scale 1/d.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "idct_core.cuh"
 #include "stages.h"
 
 namespace rjb {
 namespace k2tile {
-
-// shared memory through 32-bit window addresses kept in registers (the generic-pointer forms made the compiler re-derive
-// the window base inside the issue-bound tile loop)
-__device__ __forceinline__ uint32_t SharedU32(const void* p) {
-    uint32_t a = uint32_t(__cvta_generic_to_shared(p));
-    asm volatile("mov.u32 %0, %0;" : "+r"(a));
-    return a;
-}
-__device__ __forceinline__ uint32_t Lds32(uint32_t a) {
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ uint4 Lds128(uint32_t a) {
-    uint4 v;
-    asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ void Sts32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ void Sts128(uint32_t a, uint4 v) {
-    asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
 
 constexpr int kBlocksPerTile = 32;
 constexpr int kSearchCache = 1024;   // image tile prefix entries searched in shared memory
@@ -147,6 +126,40 @@ __device__ __forceinline__ TileInfo ResolveTile(const K2Args& a, const uint32_t*
         t -= n;
     }
     return ti;
+}
+
+// The CTA's kTiles tiles, resolved into s_tile by its first kTiles threads (the image tile prefix searched in s_tile0
+// when it fits there); ends with the CTA synchronised.
+template <int S, int kThreads, int kTiles>
+__device__ __forceinline__ void ResolveCtaTiles(const K2Args& a, TileInfo* s_tile, uint32_t* s_tile0) {
+    const int tid = threadIdx.x;
+    const bool cached = a.nimages <= kSearchCache;
+    if (cached) {
+        for (int i = tid; i < a.nimages; i += kThreads) s_tile0[i] = __ldg(a.img_tile0 + i);
+        __syncthreads();
+    }
+    if (tid < kTiles) s_tile[tid] = ResolveTile<S>(a, cached ? s_tile0 : nullptr, blockIdx.x * kTiles + tid);
+    __syncthreads();
+}
+
+// decode-order index of the tile's block in block column bx
+__device__ __forceinline__ size_t TileBlock(const TileInfo& ti, int bx) {
+    return size_t(ti.row_mcu + uint32_t(bx >> ti.hshift)) * uint32_t(ti.bpm) + ti.k_row + uint32_t(bx & ti.hmask);
+}
+
+// Block bb of the tile for the transform loops: {first entry, entries | valid << 24, dequantised integrated DC, 0}; zero
+// past the component's right edge and in a tile with nothing to store
+__device__ __forceinline__ uint4 TileBlockMeta(const TileInfo& ti, int bb) {
+    uint4 m = make_uint4(0u, 0u, 0u, 0u);
+    if (ti.nbx >= 0 && ti.direct != 2 && ti.bx0 + bb < ti.nbx) {
+        const size_t blk = TileBlock(ti, ti.bx0 + bb);
+        const uint2 r = __ldg(reinterpret_cast<const uint2*>(ti.rec + blk));
+        const uint2 e = BlockEntryRange(blk ? __ldg(&ti.rec[blk - 1].end) : 0u, r.x, ti.ent_cap);
+        m.x = e.x;
+        m.y = (e.y - e.x) | (1u << 24);
+        m.z = uint32_t(int(int16_t(r.y & 0xFFFFu)) * int(__ldg(ti.qt)));   // integrated DC, dequantised
+    }
+    return m;
 }
 
 }  // namespace k2tile

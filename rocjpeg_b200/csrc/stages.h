@@ -77,6 +77,16 @@ struct BlockRec {
     int16_t pad_;
 };
 
+// A block's coefficient entries [x, y), from its predecessor's `end` (0 for block 0 of an image) and its own; empty for
+// a block no thread reached or one whose record a damaged stream left inconsistent. (A block of a valid stream has at
+// most 64 entries + 7 pads per subsequence boundary inside it; after a DAMAGED restart interval the first block of the
+// next one also owns the pad groups the counting pass reserved in vain, any number of them - they are skipped, not a
+// reason to drop the block; the count is 16 bits wide.)
+__host__ __device__ __forceinline__ uint2 BlockEntryRange(uint32_t e0, uint32_t e1, const uint32_t& ent_cap) {
+    if (e0 == kNoEntry || e1 == kNoEntry || e1 < e0 || e1 - e0 > 0xFFFFu || e1 > ent_cap) e1 = e0 = 0;
+    return make_uint2(e0, e1);
+}
+
 struct K0Args {
     const ImageDesc* images;      // device
     SegmentDesc* segments;        // device, written here: the batch's segment table

@@ -97,7 +97,6 @@ def main():
         ("nomerge", {"ROCJPEG_B200_NO_MERGE": "1"}, steps),
         ("lanes4_15_30_30_25", {"ROCJPEG_B200_LANES": "4", "ROCJPEG_B200_SPLIT": "15,30,30,25"}, steps),
         ("lanes4_20_35_30_15", {"ROCJPEG_B200_LANES": "4", "ROCJPEG_B200_SPLIT": "20,35,30,15"}, steps),
-        ("nofuse", {"ROCJPEG_B200_NO_FUSE": "1"}, steps),
         ("s64", {"ROCJPEG_B200_SUBSEQ": "64"}, steps),
         ("halo4", {"ROCJPEG_B200_HALO": "4"}, steps),
         ("halo8", {"ROCJPEG_B200_HALO": "8"}, steps),
