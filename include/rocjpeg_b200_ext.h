@@ -59,6 +59,19 @@ typedef struct {
  * the events keep neighbouring stages from overlapping), 2 first and last event only (total_ms).
  * Env ROCJPEG_B200_PROFILE sets the initial level. */
 RocJpegStatus rocJpegB200SetProfiling(RocJpegHandle handle, int enable);
+/* Colour convention of RGB and RGB_PLANAR outputs, per handle. It applies to every later rocJpegDecode,
+ * rocJpegDecodeBatched, rocJpegB200DecodeBatchedScaled and rocJpegB200Prepare[Scaled] on the handle (and to the other
+ * devices of a sharded call); rocJpegB200Run replays what Prepare captured.
+ *   ROCJPEG_B200_COLOR_REFERENCE (default): the reference's kernels, BT.709 full-range float and nearest-neighbour chroma;
+ *   ROCJPEG_B200_COLOR_LIBJPEG: libjpeg-turbo's default decode (what Pillow and torchvision's CPU decoder return), JFIF
+ *     integer colour and "fancy" (triangle) chroma upsampling, bit for bit at full size and at 1/2, 1/4, 1/8 except for
+ *     4:2:0 at a reduced size (libjpeg-turbo transforms that chroma at twice the luma size instead of upsampling it).
+ * NATIVE, YUV_PLANAR and Y outputs, and 4:0:0 pictures, are the same under both. An unknown value returns
+ * ROCJPEG_STATUS_INVALID_PARAMETER. Env ROCJPEG_B200_COLOR=libjpeg sets the initial convention at rocJpegCreate. */
+#define ROCJPEG_B200_COLOR_REFERENCE 0
+#define ROCJPEG_B200_COLOR_LIBJPEG 1
+RocJpegStatus rocJpegB200SetColorConvention(RocJpegHandle handle, int convention);
+RocJpegStatus rocJpegB200GetColorConvention(RocJpegHandle handle, int *convention);
 /* Statistics of the last rocJpegDecode / rocJpegDecodeBatched / rocJpegB200Run on this handle. */
 RocJpegStatus rocJpegB200GetStats(RocJpegHandle handle, RocJpegB200Stats *stats);
 

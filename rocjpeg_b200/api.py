@@ -102,8 +102,11 @@ EXT_EXPORTS = (
     "rocJpegB200GetScanStatus", "rocJpegB200GetDeviceSegment", "rocJpegB200ParseAndDecodeBatched",
     "rocJpegB200PlanShardsPinned", "rocJpegB200GetImageStatus", "rocJpegB200StreamLoadFiles",
     "rocJpegB200GetScaledImageInfo", "rocJpegB200DecodeBatchedScaled", "rocJpegB200PrepareScaled",
+    "rocJpegB200SetColorConvention", "rocJpegB200GetColorConvention",
 )
 SCALES = (1, 2, 4, 8)   # denominators of the reduced-size decodes
+COLOR_REFERENCE = 0   # RGB colour conventions (rocJpegB200SetColorConvention): the reference's kernels (default)
+COLOR_LIBJPEG = 1     # libjpeg-turbo's default decode: JFIF integer colour, fancy chroma upsampling
 
 _lib = None
 
@@ -136,6 +139,8 @@ def load_library() -> C.CDLL:
     L.rocJpegGetErrorName.argtypes = [i32]
     L.rocJpegGetErrorName.restype = C.c_char_p
     L.rocJpegB200SetProfiling.argtypes = [vp, i32]
+    L.rocJpegB200SetColorConvention.argtypes = [vp, i32]
+    L.rocJpegB200GetColorConvention.argtypes = [vp, C.POINTER(i32)]
     L.rocJpegB200GetStats.argtypes = [vp, C.POINTER(Stats)]
     L.rocJpegB200Prepare.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(RocJpegDecodeParams), C.POINTER(RocJpegImage)]
     L.rocJpegB200Run.argtypes = [vp]
@@ -406,6 +411,15 @@ class Decoder:
     def set_profiling(self, level):
         """0/False off, 1/True per-stage events, 2 first/last event only (total_ms)."""
         self.lib.rocJpegB200SetProfiling(self.handle, int(level))
+
+    def set_color_convention(self, convention: int):
+        """COLOR_REFERENCE or COLOR_LIBJPEG for every later RGB / RGB_PLANAR decode on this handle."""
+        _check(self.lib.rocJpegB200SetColorConvention(self.handle, int(convention)), "rocJpegB200SetColorConvention")
+
+    def color_convention(self) -> int:
+        c = C.c_int32()
+        _check(self.lib.rocJpegB200GetColorConvention(self.handle, C.byref(c)), "rocJpegB200GetColorConvention")
+        return c.value
 
     def stats(self) -> Stats:
         s = Stats()

@@ -257,6 +257,19 @@ RocJpegStatus rocJpegB200SetProfiling(RocJpegHandle handle, int enable) {
     return ROCJPEG_STATUS_SUCCESS;
 }
 
+RocJpegStatus rocJpegB200SetColorConvention(RocJpegHandle handle, int convention) {
+    if (handle == nullptr || (convention != ROCJPEG_B200_COLOR_REFERENCE && convention != ROCJPEG_B200_COLOR_LIBJPEG))
+        return ROCJPEG_STATUS_INVALID_PARAMETER;
+    static_cast<DecoderHandle*>(handle)->decoder->SetColorConvention(convention);
+    return ROCJPEG_STATUS_SUCCESS;
+}
+
+RocJpegStatus rocJpegB200GetColorConvention(RocJpegHandle handle, int* convention) {
+    if (handle == nullptr || convention == nullptr) return ROCJPEG_STATUS_INVALID_PARAMETER;
+    *convention = static_cast<DecoderHandle*>(handle)->decoder->color_convention();
+    return ROCJPEG_STATUS_SUCCESS;
+}
+
 RocJpegStatus rocJpegB200GetStats(RocJpegHandle handle, RocJpegB200Stats* stats) {
     if (handle == nullptr || stats == nullptr) return ROCJPEG_STATUS_INVALID_PARAMETER;
     const rjb::BatchStats& s = static_cast<DecoderHandle*>(handle)->decoder->stats();

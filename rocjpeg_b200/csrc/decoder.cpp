@@ -215,6 +215,10 @@ int Decoder::Initialize() {
     RJB_CUDA(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
     RJB_CUDA(cudaStreamCreateWithPriority(&upload_stream_, cudaStreamNonBlocking, prio_hi));
     profiling_ = EnvInt("ROCJPEG_B200_PROFILE", 0);
+    {   // ROCJPEG_B200_COLOR=libjpeg: callers that cannot reach the extension API (the reference's samples) decode RGB as libjpeg-turbo does
+        const char* c = std::getenv("ROCJPEG_B200_COLOR");
+        color_ = (c && std::strcmp(c, "libjpeg") == 0) ? kColorLibjpeg : kColorReference;
+    }
     strict_status_ = EnvInt("ROCJPEG_B200_STRICT", 1) != 0;
     // everything a first decode would otherwise pay for: kernel modules, the lanes' streams and events
     RJB_CUDA(PreloadK0());
@@ -253,9 +257,15 @@ int Decoder::Initialize() {
             (void)cudaGetLastError();
         }
         peer->profiling_ = profiling_;
+        peer->color_ = color_;
         peers_.push_back(std::move(peer));
     }
     return kSuccess;
+}
+
+void Decoder::SetColorConvention(int convention) {
+    color_ = convention;
+    for (auto& peer : peers_) peer->SetColorConvention(convention);
 }
 
 namespace {
@@ -423,6 +433,7 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
 
     any_direct_ = false;
     needs_planes_ = false;
+    jfif_ = params.color == kColorLibjpeg && (params.output_format == FMT_RGB || params.output_format == FMT_RGB_PLANAR);
     uint32_t k23tile = 0, k23tile_w = 0;
     k2_needed_ = false;
     uint64_t scan_off = 0, raw_off = 0, blk = 0, plane_off = 0, ent = 0, sub = 0;
@@ -579,7 +590,10 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
             if (p.restart_interval > 0 && cw > 0 && chh > 0 && cw <= uint32_t(out_w) && chh <= uint32_t(out_h) &&
                 params.crop_top >= 0 && params.crop_bottom <= out_h && im.mcus_y > 0) {
                 const int mcu_h = 8 * std::max(1, p.ncomp == 1 ? 1 : p.vmax) / d;   // MCU rows in output rows
-                const uint64_t row_lo = uint64_t(params.crop_top / mcu_h), row_hi = uint64_t((params.crop_bottom - 1) / mcu_h);
+                // (k3_jfif: fancy upsampling reads the chroma row on each side of the crop, the rows of the IDCT stage's widened rectangle)
+                const int halo = jfif_ ? (p.css == CSS_440 || p.css == CSS_420 ? 2 : 1) : 0;
+                const int top = std::max(0, int(params.crop_top) - halo), bottom = std::min(out_h, int(params.crop_bottom) + halo);
+                const uint64_t row_lo = uint64_t(top / mcu_h), row_hi = uint64_t((bottom - 1) / mcu_h);
                 const uint64_t ri = uint64_t(p.restart_interval);
                 const uint64_t k_lo = row_lo * uint64_t(im.mcus_x) / ri, k_hi = ((row_hi + 1) * uint64_t(im.mcus_x) - 1) / ri;
                 im.seg_keep_lo = uint32_t(k_lo > 0 ? k_lo - 1 : 0);
@@ -638,7 +652,21 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
         od.direct = (whole && planar && !(remote && remote[i])) ? 1 : 0;
         // Whole-picture RGB / RGB_PLANAR: IDCT and colour conversion in one kernel, the planes never leave shared memory
         // (full size only: a scaled picture goes reduced-size IDCT -> plane arena -> output stage)
-        od.fused = (d == 1 && whole && (od.fmt == FMT_RGB || od.fmt == FMT_RGB_PLANAR) && h_fused_.size() < 65535) ? 1 : 0;
+        // (not under the libjpeg colour convention: k3_jfif's upsampling needs chroma across the fused kernel's strips)
+        od.fused = (!jfif_ && d == 1 && whole && (od.fmt == FMT_RGB || od.fmt == FMT_RGB_PLANAR) && h_fused_.size() < 65535) ? 1 : 0;
+        od.jfif = jfif_ ? 1 : 0;
+        od.pic_w = out_w;
+        od.pic_h = out_h;
+        od.upsample = UP_REPLICATE;
+        if (jfif_ && p.ncomp == 3) {
+            // jinit_upsampler (jdsample.c): fancy only with transforms larger than 1x1 (do_fancy needs min_DCT_scaled_size > 1);
+            // h2v1 / h2v2 fancy need a downsampled width > 2; every other ratio (4:4:4, 4:1:1) replicates
+            const int hr = p.hmax / p.hs[1], vr = p.vmax / p.vs[1];
+            const int cw = (out_w + hr - 1) / hr;
+            if (d < 8 && hr == 2 && vr == 1 && cw > 2) od.upsample = UP_H2V1;
+            else if (d < 8 && hr == 1 && vr == 2) od.upsample = UP_H1V2;
+            else if (d < 8 && hr == 2 && vr == 2 && cw > 2) od.upsample = UP_H2V2;
+        }
         const bool tiles = !od.direct && !od.fused;
         od.tiles_x = tiles ? uint32_t((od.w + kK3TileW - 1) / kK3TileW) : 0u;
         od.tiles_y = tiles ? uint32_t((od.h + kK3TileH - 1) / kK3TileH) : 0u;
@@ -992,7 +1020,7 @@ int Lane::LaunchDownstream(bool integrate_dc, const std::function<cudaError_t(in
     if (st != kSuccess) return st;
     RJB_CUDA(mark(6));
     RJB_CUDA(LaunchK23Fused(k23_, stream_, &stats_.kernel_launches));
-    RJB_CUDA(LaunchK3Output(k3_, stream_, &stats_.kernel_launches));
+    RJB_CUDA(jfif_ ? LaunchK3Jfif(k3_, stream_, &stats_.kernel_launches) : LaunchK3Output(k3_, stream_, &stats_.kernel_launches));
     RJB_CUDA(mark(7));
     RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
     RJB_CUDA(cudaMemcpyAsync(h_counters_.data() + 256, k0_.status, h_images_.size() * sizeof(ScanStatus), cudaMemcpyDeviceToHost, stream_));
@@ -1144,6 +1172,8 @@ int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodePar
     }
     if (params.output_format < FMT_NATIVE || params.output_format > FMT_RGB_PLANAR)
         return Fail(kInvalidParameter, "unknown output format");
+    DecodeParams lane_params = params;
+    lane_params.color = color_;
     Split(streams, n);
     for (int l = 0; l < active_lanes_; l++) {
         const int st = lanes_[l].Create(device_id_, sm_count_, l < 4);
@@ -1173,7 +1203,7 @@ int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodePar
         Lane& lane = lanes_[l];
         const int first = chunk_first_[l], cnt = chunk_first_[l + 1] - first;
         lane.set_host_mark(0, NowMs());
-        int st = lane.Build(streams + first, cnt, params, dsts + first, remote ? remote + first : nullptr);
+        int st = lane.Build(streams + first, cnt, lane_params, dsts + first, remote ? remote + first : nullptr);
         if (st == kSuccess) st = launch ? lane.LaunchAll(true, profiling_, upload_stream_) : lane.Upload(upload_stream_);
         if (st != kSuccess) {
             for (int k = 0; k < active_lanes_; k++) lanes_[k].Sync();   // do not leave work in flight behind an error (the failed lane's included)

@@ -33,7 +33,11 @@ namespace rjb {
 struct DecodeParams {
     int32_t output_format;
     int16_t crop_left, crop_top, crop_right, crop_bottom;
+    int32_t color = 0;   // kColor*: the handle's colour convention (not part of RocJpegDecodeParams)
 };
+// Colour conventions of RGB / RGB_PLANAR (ROCJPEG_B200_COLOR_* of include/rocjpeg_b200_ext.h)
+constexpr int kColorReference = 0;   // the reference's kernels: BT.709 full-range float, nearest-neighbour chroma
+constexpr int kColorLibjpeg = 1;     // libjpeg-turbo's default decode: JFIF integer colour, fancy upsampling (k3_jfif.cu)
 struct DestImage {
     uint8_t* channel[4];
     uint32_t pitch[4];
@@ -194,6 +198,7 @@ class Lane {
     K2Args k2s_[kScaledKernels] = {};   // reduced-size IDCT: the pictures of scale 1/2, 1/4, 1/8
     K3Args k3_ = {};
     K23Args k23_ = {};
+    bool jfif_ = false;           // the output stage is k3_jfif (RGB / RGB_PLANAR under the libjpeg colour convention)
     bool k2_needed_ = true;       // some image of the lane is not served by the fused kernel
     bool any_direct_ = false, needs_planes_ = false;
     // The kernel schedule, fixed by Build: how the entropy-coded bytes are uploaded (the gather kernel also leaves the
@@ -245,6 +250,9 @@ class Decoder {
     int CopySegment(int image, uint32_t segment, uint8_t* host_out, size_t capacity, uint32_t* nbytes);   // destuffed by K0
     int GetScanStatus(int image, ScanStatus* out);
     void SetProfiling(int level) { profiling_ = level; }   // 0 off, 1 per-stage events, 2 first/last event only
+    // kColor*: applies to every later decode and Prepare on this handle, the peers of a sharded call included
+    void SetColorConvention(int convention);
+    int color_convention() const { return color_; }
     const BatchStats& stats() const { return stats_; }
     const std::string& last_error() const { return err_; }
     int device_id() const { return device_id_; }
@@ -270,6 +278,7 @@ class Decoder {
     bool initialized_ = false, prepared_ = false;
     bool strict_status_ = true;   // ROCJPEG_B200_STRICT=0: truncated scans do not change the return code
     int profiling_ = 0;
+    int color_ = kColorReference;
     std::mutex mutex_;
     std::string err_;
     int sm_count_ = 0;

@@ -138,7 +138,13 @@ struct OutputDesc {
     uint32_t tiles_x, tiles_y;
     int32_t direct;          // the IDCT stage stores this image's planes straight into dst (planar formats, no crop): no output tiles
     int32_t fused;           // whole-picture RGB / RGB_PLANAR: the fused IDCT + output kernel serves it (no IDCT tiles' output, no output tiles)
+    int32_t jfif;            // RGB / RGB_PLANAR under the libjpeg colour convention: k3_jfif serves it, and a crop needs the chroma around it
+    int32_t upsample;        // UpsampleMode of k3_jfif
+    int32_t pic_w, pic_h;    // the picture's size at its scale (the crop rectangle lies inside it): the upsampling's edges
 };
+
+// Chroma upsampling of k3_jfif.cu: the method libjpeg-turbo's jinit_upsampler (jdsample.c) picks for the component ratio.
+enum UpsampleMode : int32_t { UP_REPLICATE = 0, UP_H2V1 = 1, UP_H1V2 = 2, UP_H2V2 = 3 };
 
 // Everything the fused IDCT + output kernel (k23_fused.cu) needs about one picture, prepared on the host so that a CTA
 // starts from one record instead of deriving it (a quarter of the kernel's time when thread 0 did: profiles/r02_*).

@@ -97,8 +97,17 @@ __device__ __forceinline__ TileInfo ResolveTile(const K2Args& a, const uint32_t*
                 // samples under the crop rectangle, so blocks outside it are not transformed at all.
                 const int sx = comp == 0 ? 0 : im.css == CSS_411 ? 2 : (im.css == CSS_422 || im.css == CSS_420) ? 1 : 0;
                 const int sy = (comp != 0 && (im.css == CSS_440 || im.css == CSS_420)) ? 1 : 0;
-                const int bx_lo = (od.x0 >> sx) >> kLogS, bx_hi = ((od.x0 + od.w - 1) >> sx) >> kLogS;
-                const int by_lo = (od.y0 >> sy) >> kLogS, by_hi = ((od.y0 + od.h - 1) >> sy) >> kLogS;
+                int x_lo = od.x0, x_hi = od.x0 + od.w - 1, y_lo = od.y0, y_hi = od.y0 + od.h - 1;
+                if (od.jfif) {
+                    // fancy upsampling (k3_jfif.cu) reads one chroma sample beyond the crop on each side: the rectangle
+                    // widened by one chroma sample, clamped to the picture
+                    const int hx = im.css == CSS_411 ? 4 : (im.css == CSS_422 || im.css == CSS_420) ? 2 : 1;
+                    const int hy = (im.css == CSS_440 || im.css == CSS_420) ? 2 : 1;
+                    x_lo = max(0, x_lo - hx); x_hi = min(od.pic_w - 1, x_hi + hx);
+                    y_lo = max(0, y_lo - hy); y_hi = min(od.pic_h - 1, y_hi + hy);
+                }
+                const int bx_lo = (x_lo >> sx) >> kLogS, bx_hi = (x_hi >> sx) >> kLogS;
+                const int by_lo = (y_lo >> sy) >> kLogS, by_hi = (y_hi >> sy) >> kLogS;
                 if (by < by_lo || by > by_hi || ti.bx0 > bx_hi || ti.bx0 + kBlocksPerTile - 1 < bx_lo) ti.direct = 2;
             }
             if (od.direct && !a.force_planes) {

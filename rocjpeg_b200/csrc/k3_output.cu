@@ -196,6 +196,7 @@ cudaError_t PreloadK3() {
     cudaFuncAttributes at;
     cudaError_t e = cudaSuccess;
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k3_output);
+    if (e == cudaSuccess) e = PreloadK3Jfif();
     return e;
 }
 

@@ -400,6 +400,8 @@ __device__ __forceinline__ void FlushShifted(const uint8_t* buf, uint8_t* dst, i
     if (done + lane < n) dst[done + lane] = buf[done + lane];
 }
 
+__device__ __forceinline__ void StoreRgb8Staged(const K3Job& j, uint8_t* buf, int y, int lane, int n, const Rgb8& o);
+
 // One output row segment like RowRgbFast (same preconditions on the source: (x0 + xt) % 8 == 0), any destination alignment.
 // buf: per-warp staging, 16-byte aligned, at least 3 * (kTileW + 16) bytes.
 template <int SX, bool SM>
@@ -431,6 +433,14 @@ __device__ __forceinline__ void RowRgbStaged(const K3Job& j, int sy, bool gray, 
             o = Convert8<SX>(yy, uu, vv);
         }
     }
+    StoreRgb8Staged(j, buf, y, lane, n, o);
+}
+
+// The store half of RowRgbStaged: the lane's 8 converted pixels (the first n of them; none when n <= 0) of output row y,
+// every lane of the warp calling, written out at the destination's alignment. Also the store of k3_jfif.cu's rows whose
+// destination is not 4-byte aligned.
+__device__ __forceinline__ void StoreRgb8Staged(const K3Job& j, uint8_t* buf, int y, int lane, int n, const Rgb8& o) {
+    const int nx = j.nx, xt = j.xt;
     constexpr int kPlane = kTileW + 16;   // staged bytes per plane (+ the words FlushShifted reads past the end)
     if (j.fmt == FMT_RGB) {
         if (n > 0) {

@@ -204,6 +204,9 @@ struct K3Args {
     uint32_t total_tiles;
 };
 cudaError_t LaunchK3Output(const K3Args& a, cudaStream_t stream, uint32_t* launches);
+// The output stage of RGB / RGB_PLANAR under the libjpeg colour convention (k3_jfif.cu): same tiles and arguments.
+cudaError_t LaunchK3Jfif(const K3Args& a, cudaStream_t stream, uint32_t* launches);
+cudaError_t PreloadK3Jfif();   // part of PreloadK3
 
 // Load the stages' kernels now instead of at their first launch.
 cudaError_t PreloadK1();
