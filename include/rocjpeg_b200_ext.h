@@ -11,6 +11,7 @@
  *     device-resident throughput ("inputs already in HBM") can be timed apart
  *     from the host->device copy;
  *   - decodes at 1/2, 1/4 and 1/8 scale (reduced-size IDCT, as libjpeg's scale_denom);
+ *   - decodes resized to a requested size as Pillow's Image.resize does it;
  *   - per-stage CUDA-event timings and batch statistics for the roofline report;
  *   - parser taps (host only; usable without a GPU).
  * Plain C ABI: pointers and sizes only.
@@ -103,6 +104,46 @@ RocJpegStatus rocJpegB200DecodeBatchedScaled(RocJpegHandle handle, RocJpegStream
                                              const RocJpegDecodeParams *decode_params, const int32_t *scale_denoms, RocJpegImage *destinations);
 RocJpegStatus rocJpegB200PrepareScaled(RocJpegHandle handle, RocJpegStreamHandle *jpeg_stream_handles, int batch_size,
                                        const RocJpegDecodeParams *decode_params, const int32_t *scale_denoms, RocJpegImage *destinations);
+
+/* Decode straight to a requested size, resampled as Pillow does (Image.resize), on the GPU behind the decode. Per picture:
+ *   1. decode exactly as rocJpegB200DecodeBatchedScaled would: the handle's colour convention, at 1/scale_denom, the crop
+ *      rectangle of decode_params in the scaled picture's coordinates;
+ *   2. resize that picture to width x height with Pillow's Image.resize((width, height), filter), byte for byte: Pillow's
+ *      double-precision weights rounded to 22-bit fixed point, a horizontal then a vertical pass of int32 multiply-adds with
+ *      the clipped 8-bit intermediate in between (Pillow's Resample.c).
+ * With a crop the result is img.crop(box).resize(size, filter): torchvision's resized_crop on a PIL image.
+ * Output formats at the requested size: RGB (interleaved, channel[0]), RGB_PLANAR (three planes, all with pitch[0]), Y
+ * (luma only: Pillow's "L" mode). Any pitch of at least the row's bytes, any base alignment. NATIVE and YUV_PLANAR,
+ * filter 0 (NEAREST) or any other unknown filter, a width or height of 0 or above 65535, a denominator outside
+ * {1, 2, 4, 8}, a null channel or a pitch below the row's bytes return ROCJPEG_STATUS_INVALID_PARAMETER before anything
+ * runs. Per-image status, BAD_JPEG and ROCJPEG_B200_STRICT behave as for rocJpegDecodeBatched; a truncated picture is
+ * resized from what its decode produced. The decoded pictures pass through a device arena the handle keeps (grow-only).
+ * A resized call runs on the handle's own device: on a sharded handle (ROCJPEG_B200_DEVICES) it is not split, and a
+ * destination on another device returns ROCJPEG_STATUS_INVALID_PARAMETER. target_dimension stays unread.
+ *   rocJpegB200DecodeBatchedResized: resize[i] for picture i;
+ *   rocJpegB200PrepareResized: rocJpegB200Prepare with resizes; rocJpegB200Run replays it unchanged;
+ *   rocJpegB200ResizeCoefficients (host only): Pillow's coefficients of one axis, as the passes apply them.
+ *     *ksize = taps per output sample (2 ceil(support) + 1); bounds[2 i] = first input sample of output sample i,
+ *     bounds[2 i + 1] = how many it reads; taps[i * ksize + t] = their fixed-point weights, rows padded with zeros.
+ *     bounds and taps NULL: only *ksize. capacity (in taps) below out_size * ksize: INVALID_PARAMETER. */
+#define ROCJPEG_B200_FILTER_LANCZOS 1 /* Pillow's Image.Resampling values */
+#define ROCJPEG_B200_FILTER_BILINEAR 2
+#define ROCJPEG_B200_FILTER_BICUBIC 3
+#define ROCJPEG_B200_FILTER_BOX 4
+#define ROCJPEG_B200_FILTER_HAMMING 5
+typedef struct {
+    uint32_t width, height; /* size of the output, >= 1 each */
+    int32_t filter;         /* ROCJPEG_B200_FILTER_* */
+    int32_t scale_denom;    /* 1, 2, 4, 8: reduced-size IDCT before the resize (as rocJpegB200DecodeBatchedScaled) */
+} RocJpegB200Resize;
+RocJpegStatus rocJpegB200DecodeBatchedResized(RocJpegHandle handle, RocJpegStreamHandle *jpeg_stream_handles, int batch_size,
+                                              const RocJpegDecodeParams *decode_params, const RocJpegB200Resize *resize,
+                                              RocJpegImage *destinations);
+RocJpegStatus rocJpegB200PrepareResized(RocJpegHandle handle, RocJpegStreamHandle *jpeg_stream_handles, int batch_size,
+                                        const RocJpegDecodeParams *decode_params, const RocJpegB200Resize *resize,
+                                        RocJpegImage *destinations);
+RocJpegStatus rocJpegB200ResizeCoefficients(uint32_t in_size, uint32_t out_size, int filter, int32_t *bounds, int32_t *taps,
+                                            size_t capacity, int32_t *ksize);
 
 /* Timing-harness helper: exactly the caller's loop of the reference's batched sample - rocJpegStreamParse(datas[i],
  * lengths[i], handles[i]) for every image, then one rocJpegDecodeBatched - issued from C. *parse_seconds (optional) = wall

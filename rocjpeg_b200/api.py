@@ -63,6 +63,11 @@ class Stats(C.Structure):
     ]
 
 
+class ResizeSpec(C.Structure):
+    """RocJpegB200Resize: output size, FILTER_*, scale denominator of one picture of a resized decode."""
+    _fields_ = [("width", C.c_uint32), ("height", C.c_uint32), ("filter", C.c_int32), ("scale_denom", C.c_int32)]
+
+
 class StreamInfo(C.Structure):
     _fields_ = [
         ("width", C.c_int32), ("height", C.c_int32), ("num_components", C.c_int32), ("chroma_subsampling", C.c_int32),
@@ -103,10 +108,14 @@ EXT_EXPORTS = (
     "rocJpegB200PlanShardsPinned", "rocJpegB200GetImageStatus", "rocJpegB200StreamLoadFiles",
     "rocJpegB200GetScaledImageInfo", "rocJpegB200DecodeBatchedScaled", "rocJpegB200PrepareScaled",
     "rocJpegB200SetColorConvention", "rocJpegB200GetColorConvention",
+    "rocJpegB200DecodeBatchedResized", "rocJpegB200PrepareResized", "rocJpegB200ResizeCoefficients",
 )
 SCALES = (1, 2, 4, 8)   # denominators of the reduced-size decodes
 COLOR_REFERENCE = 0   # RGB colour conventions (rocJpegB200SetColorConvention): the reference's kernels (default)
 COLOR_LIBJPEG = 1     # libjpeg-turbo's default decode: JFIF integer colour, fancy chroma upsampling
+# Resampling filters of the resized decodes (rocJpegB200DecodeBatchedResized): Pillow's Image.Resampling values
+FILTER_LANCZOS, FILTER_BILINEAR, FILTER_BICUBIC, FILTER_BOX, FILTER_HAMMING = 1, 2, 3, 4, 5
+FILTERS = (FILTER_LANCZOS, FILTER_BILINEAR, FILTER_BICUBIC, FILTER_BOX, FILTER_HAMMING)
 
 _lib = None
 
@@ -147,6 +156,9 @@ def load_library() -> C.CDLL:
     L.rocJpegB200GetScaledImageInfo.argtypes = [vp, vp, i32, C.POINTER(C.c_uint8), C.POINTER(i32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]
     L.rocJpegB200DecodeBatchedScaled.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(RocJpegDecodeParams), C.POINTER(C.c_int32), C.POINTER(RocJpegImage)]
     L.rocJpegB200PrepareScaled.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(RocJpegDecodeParams), C.POINTER(C.c_int32), C.POINTER(RocJpegImage)]
+    L.rocJpegB200DecodeBatchedResized.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(RocJpegDecodeParams), C.POINTER(ResizeSpec), C.POINTER(RocJpegImage)]
+    L.rocJpegB200PrepareResized.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(RocJpegDecodeParams), C.POINTER(ResizeSpec), C.POINTER(RocJpegImage)]
+    L.rocJpegB200ResizeCoefficients.argtypes = [C.c_uint32, C.c_uint32, i32, vp, vp, C.c_size_t, C.POINTER(C.c_int32)]
     L.rocJpegB200GetCoefficients.argtypes = [vp, i32, vp, C.c_size_t]
     L.rocJpegB200GetPlanes.argtypes = [vp, i32, vp, C.c_size_t]
     L.rocJpegB200StreamGetInfo.argtypes = [vp, C.POINTER(StreamInfo)]
@@ -192,6 +204,21 @@ def plan_shards_pinned(costs, fixed, num_devices: int):
     out = np.zeros(len(c), dtype=np.int32)
     _check(load_library().rocJpegB200PlanShardsPinned(c.ctypes.data, f.ctypes.data, len(c), num_devices, out.ctypes.data), "rocJpegB200PlanShardsPinned")
     return out
+
+
+def resize_coefficients(in_size: int, out_size: int, filt: int):
+    """rocJpegB200ResizeCoefficients: Pillow's coefficients of one axis as the resize passes apply them.
+    Returns (bounds int32 (out_size, 2): first input sample and count per output sample, taps int32 (out_size, ksize))."""
+    import numpy as np
+
+    L = load_library()
+    ks = C.c_int32()
+    _check(L.rocJpegB200ResizeCoefficients(in_size, out_size, filt, None, None, 0, C.byref(ks)), "rocJpegB200ResizeCoefficients")
+    bounds = np.zeros((out_size, 2), dtype=np.int32)
+    taps = np.zeros((out_size, ks.value), dtype=np.int32)
+    _check(L.rocJpegB200ResizeCoefficients(in_size, out_size, filt, bounds.ctypes.data, taps.ctypes.data, taps.size, C.byref(ks)),
+           "rocJpegB200ResizeCoefficients")
+    return bounds, taps
 
 
 def load_files(streams, paths, io_threads: int = 0):
@@ -376,6 +403,30 @@ class Decoder:
         rectangle are in scaled units (scaled_image_info). Returns RocJpegStatus."""
         hs, imgs, n, _ = streams if dests is None else self.make_batch(streams, dests)
         return self.lib.rocJpegB200DecodeBatchedScaled(self.handle, hs, n, C.byref(params), self._scales(scales, n), imgs)
+
+    @staticmethod
+    def _resizes(sizes, filters, scales, n):
+        """RocJpegB200Resize array: sizes[i] = (width, height); filters / scales one per picture or one for all."""
+        if len(sizes) != n:
+            raise ValueError(f"{len(sizes)} sizes for {n} pictures")
+        filters = list(filters) if isinstance(filters, (list, tuple)) else [filters] * n
+        scales = [1] * n if scales is None else (list(scales) if isinstance(scales, (list, tuple)) else [scales] * n)
+        arr = (ResizeSpec * n)()
+        for i in range(n):
+            arr[i].width, arr[i].height = int(sizes[i][0]), int(sizes[i][1])
+            arr[i].filter, arr[i].scale_denom = int(filters[i]), int(scales[i])
+        return arr
+
+    def decode_batched_resized(self, streams, params: RocJpegDecodeParams, dests, sizes, filters, scales=None) -> int:
+        """rocJpegB200DecodeBatchedResized: picture i decoded (at 1/scales[i], cropped by params) and resized to sizes[i] =
+        (width, height) with filters[i] exactly as Pillow's Image.resize. dests are at the resized size. Returns RocJpegStatus."""
+        hs, imgs, n, _ = streams if dests is None else self.make_batch(streams, dests)
+        return self.lib.rocJpegB200DecodeBatchedResized(self.handle, hs, n, C.byref(params), self._resizes(sizes, filters, scales, n), imgs)
+
+    def prepare_resized(self, streams, params: RocJpegDecodeParams, dests, sizes, filters, scales=None) -> int:
+        """rocJpegB200PrepareResized: the resized decode made resident; run() replays it."""
+        hs, imgs, n, _ = self.make_batch(streams, dests)
+        return self.lib.rocJpegB200PrepareResized(self.handle, hs, n, C.byref(params), self._resizes(sizes, filters, scales, n), imgs)
 
     def make_sources(self, addresses, lengths):
         """Argument arrays (data pointers, lengths) for parse_and_decode_batched."""

@@ -322,6 +322,65 @@ RocJpegStatus rocJpegB200PrepareScaled(RocJpegHandle handle, RocJpegStreamHandle
     }
 }
 
+namespace {
+// The resized calls: denominators and (size, filter) per picture out of RocJpegB200Resize; prepare = rocJpegB200PrepareResized.
+RocJpegStatus DecodeResized(RocJpegHandle handle, RocJpegStreamHandle* jpeg_stream_handles, int batch_size, const RocJpegDecodeParams* decode_params,
+                            const RocJpegB200Resize* resize, RocJpegImage* destinations, bool prepare) {
+    if (handle == nullptr || jpeg_stream_handles == nullptr || decode_params == nullptr || resize == nullptr || destinations == nullptr ||
+        batch_size < 0 || (prepare && batch_size == 0))
+        return ROCJPEG_STATUS_INVALID_PARAMETER;
+    auto h = static_cast<DecoderHandle*>(handle);
+    try {
+        std::vector<const rjb::StreamParser*> streams;
+        int st = CollectStreams(jpeg_stream_handles, batch_size, &streams);
+        if (st != 0) return RocJpegStatus(st);
+        std::vector<int32_t> denoms(static_cast<size_t>(batch_size));
+        std::vector<rjb::ResizeSpec> specs(static_cast<size_t>(batch_size));
+        for (int i = 0; i < batch_size; i++) {
+            denoms[size_t(i)] = resize[i].scale_denom;
+            specs[size_t(i)] = rjb::ResizeSpec{resize[i].width, resize[i].height, resize[i].filter};
+        }
+        std::vector<rjb::DestImage> dsts;
+        st = ToDests(destinations, batch_size, denoms.data(), &dsts);
+        if (st != 0) return RocJpegStatus(st);
+        if (const char* why = rjb::CheckResizeArgs(ToParams(decode_params), batch_size, dsts.data(), specs.data())) {
+            h->CaptureError(why);
+            return ROCJPEG_STATUS_INVALID_PARAMETER;
+        }
+        st = prepare ? h->decoder->Prepare(streams.data(), batch_size, ToParams(decode_params), dsts.data(), specs.data())
+                     : h->decoder->Decode(streams.data(), batch_size, ToParams(decode_params), dsts.data(), specs.data());
+        if (st != 0) h->CaptureError(h->decoder->last_error());
+        return RocJpegStatus(st);
+    } catch (const std::exception& e) {
+        h->CaptureError(e.what());
+        ERR(e.what());
+        return ROCJPEG_STATUS_RUNTIME_ERROR;
+    }
+}
+}  // namespace
+
+RocJpegStatus rocJpegB200DecodeBatchedResized(RocJpegHandle handle, RocJpegStreamHandle* jpeg_stream_handles, int batch_size,
+                                              const RocJpegDecodeParams* decode_params, const RocJpegB200Resize* resize, RocJpegImage* destinations) {
+    return DecodeResized(handle, jpeg_stream_handles, batch_size, decode_params, resize, destinations, false);
+}
+
+RocJpegStatus rocJpegB200PrepareResized(RocJpegHandle handle, RocJpegStreamHandle* jpeg_stream_handles, int batch_size,
+                                        const RocJpegDecodeParams* decode_params, const RocJpegB200Resize* resize, RocJpegImage* destinations) {
+    return DecodeResized(handle, jpeg_stream_handles, batch_size, decode_params, resize, destinations, true);
+}
+
+RocJpegStatus rocJpegB200ResizeCoefficients(uint32_t in_size, uint32_t out_size, int filter, int32_t* bounds, int32_t* taps, size_t capacity,
+                                            int32_t* ksize) {
+    if (ksize == nullptr || !rjb::ValidFilter(filter) || in_size < 1 || out_size < 1 || in_size > rjb::kMaxResizeSize ||
+        out_size > rjb::kMaxResizeSize)
+        return ROCJPEG_STATUS_INVALID_PARAMETER;
+    *ksize = rjb::ResizeTaps(in_size, out_size, filter);
+    if (bounds == nullptr && taps == nullptr) return ROCJPEG_STATUS_SUCCESS;
+    if (bounds == nullptr || taps == nullptr || capacity < size_t(out_size) * size_t(*ksize)) return ROCJPEG_STATUS_INVALID_PARAMETER;
+    rjb::ResizeCoefficients(in_size, out_size, filter, bounds, taps);
+    return ROCJPEG_STATUS_SUCCESS;
+}
+
 RocJpegStatus rocJpegB200Run(RocJpegHandle handle) {
     if (handle == nullptr) return ROCJPEG_STATUS_INVALID_PARAMETER;
     auto h = static_cast<DecoderHandle*>(handle);

@@ -227,6 +227,7 @@ int Decoder::Initialize() {
     RJB_CUDA(PreloadK2Scaled());
     RJB_CUDA(PreloadK3());
     RJB_CUDA(PreloadK23());
+    RJB_CUDA(PreloadK4());
     for (int l = 1; l < 4; l++) {   // the lanes a call uses by default; the others (ROCJPEG_B200_LANES > 4) are created on demand
         st = lanes_[l].Create(device_id_, sm_count_);
         if (st != kSuccess) return Fail(st, lanes_[l].last_error());
@@ -381,9 +382,19 @@ static uint64_t OutputBytes(int css, int fmt, int W, int H) {
     }
 }
 
-int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const uint8_t* remote) {
-    if (params.output_format < FMT_NATIVE || params.output_format > FMT_RGB_PLANAR)
+int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& call_params, const DestImage* dsts, const uint8_t* remote,
+                const ResizeSpec* resize) {
+    if (call_params.output_format < FMT_NATIVE || call_params.output_format > FMT_RGB_PLANAR)
         return Fail(kInvalidParameter, "unknown output format");
+    DecodeParams params = call_params;
+    h_resize_.clear();
+    k4_ = K4Args{};
+    if (resize) {   // decode into the resize arena (RGB_PLANAR as interleaved RGB: the same pixels), resize from there
+        const int st = PlanResize(streams, n, call_params, dsts, resize);
+        if (st != kSuccess) return st;
+        dsts = h_resize_dsts_.data();
+        if (params.output_format == FMT_RGB_PLANAR) params.output_format = FMT_RGB;
+    }
     h_images_.assign(size_t(n), ImageDesc{});
     h_outputs_.assign(size_t(n), OutputDesc{});
     h_img_cta0_.assign(size_t(n) + 1, 0);
@@ -790,12 +801,118 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& p
     k23_.nimages = n;
     k23_.total_tiles = k23tile;
     k23_.total_tiles_w = k23tile_w;
+    if (!h_resize_.empty()) {
+        k4_.njobs = n;
+        k4_.h_tiles = h_rh_tile0_[size_t(n)];
+        k4_.v_tiles = h_rv_tile0_[size_t(n)];
+        stats_.output_bytes = 0;   // what reaches the caller's buffers: the resized pictures
+        for (const ResizeJob& j : h_resize_) stats_.output_bytes += uint64_t(j.out_w) * uint64_t(j.out_h) * uint64_t(j.ch);
+    }
+    return kSuccess;
+}
+
+int Lane::PlanResize(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const ResizeSpec* resize) {
+    h_resize_.assign(size_t(n), ResizeJob{});
+    h_resize_coef_.clear();
+    h_resize_dsts_.assign(size_t(n), DestImage{});
+    h_rh_tile0_.assign(size_t(n) + 1, 0);
+    h_rv_tile0_.assign(size_t(n) + 1, 0);
+    // tables de-duplicated by (in size, out size, filter): a batch of equal-sized pictures carries one per axis
+    struct Table {
+        uint32_t in, out;
+        int filter, ksize;
+        uint32_t off;
+    };
+    std::vector<Table> tables;
+    auto table = [&](uint32_t in, uint32_t out, int filter, int32_t* ksize) -> uint32_t {
+        for (const Table& t : tables)
+            if (t.in == in && t.out == out && t.filter == filter) {
+                *ksize = t.ksize;
+                return t.off;
+            }
+        const uint32_t off = uint32_t(h_resize_coef_.size());
+        // an axis that keeps its size (a pass Pillow skips): the identity, one tap of weight 1 << 22
+        const int ks = in == out ? 1 : ResizeTaps(in, out, filter);
+        h_resize_coef_.resize(size_t(off) + 2 * size_t(out) + size_t(out) * size_t(ks), 0);
+        int32_t* bounds = &h_resize_coef_[off];
+        int32_t* taps = bounds + 2 * size_t(out);
+        if (in == out) {
+            for (uint32_t i = 0; i < out; i++) {
+                bounds[2 * i] = int32_t(i);
+                bounds[2 * i + 1] = 1;
+                taps[i] = 1 << kResamplePrecision;
+            }
+        } else {
+            ResizeCoefficients(in, out, filter, bounds, taps);
+        }
+        h_resize_coef_.resize(AlignUp(h_resize_coef_.size(), 2));   // the next table's int2 bounds 8-byte aligned
+        tables.push_back(Table{in, out, filter, ks, off});
+        *ksize = ks;
+        return off;
+    };
+    const int fmt = params.output_format;
+    const int ch = fmt == FMT_Y ? 1 : 3;
+    std::vector<size_t> src_off(static_cast<size_t>(n)), tmp_off(static_cast<size_t>(n));
+    size_t arena = 0;
+    uint32_t htile = 0, vtile = 0;
+    for (int i = 0; i < n; i++) {
+        const ParsedJpeg& p = streams[i]->parsed();
+        const int d = dsts[i].scale_denom;
+        // the decoded picture: the crop rectangle (in scaled units) or the whole scaled picture (Build's ROI rule)
+        int w = (p.width + d - 1) / d, h = (p.height + d - 1) / d;
+        const uint32_t rw = uint32_t(int(params.crop_right) - int(params.crop_left));
+        const uint32_t rh = uint32_t(int(params.crop_bottom) - int(params.crop_top));
+        if (rw > 0 && rh > 0 && rw <= uint32_t(w) && rh <= uint32_t(h)) {
+            w = int(rw);
+            h = int(rh);
+        }
+        ResizeJob& j = h_resize_[size_t(i)];
+        j.in_w = w;
+        j.out_w = int32_t(resize[i].width);
+        j.out_h = int32_t(resize[i].height);
+        j.ch = ch;
+        j.fmt = fmt;
+        j.h_coef = table(uint32_t(w), resize[i].width, resize[i].filter, &j.h_ksize);
+        j.v_coef = table(uint32_t(h), resize[i].height, resize[i].filter, &j.v_ksize);
+        const int32_t* vb = &h_resize_coef_[j.v_coef];
+        j.y0 = vb[0];
+        j.rows = vb[2 * (j.out_h - 1)] + vb[2 * (j.out_h - 1) + 1] - j.y0;
+        // (pitches are multiples of 64: whole-picture RGB keeps the fused kernel's aligned path; 64 bytes of slack behind
+        // each region cover the 24-byte loads of the vertical pass's ragged last lane)
+        j.src_pitch = uint32_t(AlignUp(size_t(w) * ch, 64));
+        src_off[size_t(i)] = arena;
+        arena = AlignUp(arena + size_t(j.src_pitch) * size_t(h) + 64, 256);
+        j.tmp_pitch = uint32_t(AlignUp(size_t(j.out_w) * ch, 64));
+        tmp_off[size_t(i)] = arena;
+        arena = AlignUp(arena + size_t(j.tmp_pitch) * size_t(j.rows) + 64, 256);
+        for (int c = 0; c < 3; c++) j.dst[c] = dsts[i].channel[c];
+        j.dst_pitch = dsts[i].pitch[0];
+        const uint32_t tiles_x = uint32_t(j.out_w + kResizeTileW - 1) / kResizeTileW;
+        h_rh_tile0_[size_t(i)] = htile;
+        h_rv_tile0_[size_t(i)] = vtile;
+        htile += tiles_x * uint32_t((j.rows + kResizeRowsH - 1) / kResizeRowsH);
+        vtile += tiles_x * uint32_t(j.out_h);
+    }
+    h_rh_tile0_[size_t(n)] = htile;
+    h_rv_tile0_[size_t(n)] = vtile;
+    RJB_CUDA(d_resize_.Reserve(arena));
+    uint8_t* base = d_resize_.as<uint8_t>();
+    for (int i = 0; i < n; i++) {
+        ResizeJob& j = h_resize_[size_t(i)];
+        j.src = base + src_off[size_t(i)];
+        j.tmp = base + tmp_off[size_t(i)];
+        DestImage& di = h_resize_dsts_[size_t(i)];
+        di.channel[0] = base + src_off[size_t(i)];
+        di.pitch[0] = j.src_pitch;
+        di.scale_denom = dsts[i].scale_denom;
+    }
     return kSuccess;
 }
 
 // Descriptor block: one pinned host buffer mirrored by one device buffer, one copy.
 struct Lane::Layout {
-    size_t images, outputs, cta0, k0tile0, dctile0, k2tile0, k2stile0[kScaledKernels], k3tile0, fused, tile_img, tile_img_w, gather, luts, qtables, total;
+    size_t images, outputs, cta0, k0tile0, dctile0, k2tile0, k2stile0[kScaledKernels], k3tile0, fused, tile_img, tile_img_w, gather, luts, qtables,
+        rjobs, rcoef, rh_tile0, rv_tile0, total;
 };
 
 int Lane::Upload(cudaStream_t up) {
@@ -818,6 +935,11 @@ int Lane::Upload(cudaStream_t up) {
     L.gather = place(n * sizeof(GatherItem));
     L.luts = place(h_lut_ptrs_.size() * sizeof(HuffLutSet));
     L.qtables = place(h_qtables_.size() * 2);
+    const size_t nr = h_resize_.size();   // resized calls: jobs, tables and tile starts of the resize passes
+    L.rjobs = place(nr * sizeof(ResizeJob));
+    L.rcoef = place(nr ? h_resize_coef_.size() * 4 : 0);
+    L.rh_tile0 = place(nr ? (nr + 1) * 4 : 0);
+    L.rv_tile0 = place(nr ? (nr + 1) * 4 : 0);
     L.total = o;
     uint8_t* h = h_desc_.Reserve(L.total);
     if (!h) return Fail(kOutOfMemory, "descriptor staging");
@@ -835,6 +957,12 @@ int Lane::Upload(cudaStream_t up) {
     std::memcpy(h + L.gather, h_gather_.data(), n * sizeof(GatherItem));
     for (size_t s = 0; s < h_lut_ptrs_.size(); s++) std::memcpy(h + L.luts + s * sizeof(HuffLutSet), h_lut_ptrs_[s], sizeof(HuffLutSet));
     std::memcpy(h + L.qtables, h_qtables_.data(), h_qtables_.size() * 2);
+    if (nr) {
+        std::memcpy(h + L.rjobs, h_resize_.data(), nr * sizeof(ResizeJob));
+        std::memcpy(h + L.rcoef, h_resize_coef_.data(), h_resize_coef_.size() * 4);
+        std::memcpy(h + L.rh_tile0, h_rh_tile0_.data(), (nr + 1) * 4);
+        std::memcpy(h + L.rv_tile0, h_rv_tile0_.data(), (nr + 1) * 4);
+    }
     desc_bytes_ = L.total;
 
     // One device allocation per lane (grow-only): the first call of a handle - the only one the
@@ -911,6 +1039,10 @@ int Lane::Upload(cudaStream_t up) {
     k23_.qtables = k2_.qtables;
     k23_.entries = k1_.entries;
     k23_.blk_rec = k1_.blk_rec;
+    k4_.jobs = reinterpret_cast<const ResizeJob*>(d + L.rjobs);
+    k4_.coef = reinterpret_cast<const int32_t*>(d + L.rcoef);
+    k4_.h_tile0 = reinterpret_cast<const uint32_t*>(d + L.rh_tile0);
+    k4_.v_tile0 = reinterpret_cast<const uint32_t*>(d + L.rv_tile0);
 
     // Uploads of all lanes go through ONE stream, in lane order: the first chunk gets the whole
     // PCIe link and its kernels start while the next chunks are still in flight.
@@ -1021,6 +1153,7 @@ int Lane::LaunchDownstream(bool integrate_dc, const std::function<cudaError_t(in
     RJB_CUDA(mark(6));
     RJB_CUDA(LaunchK23Fused(k23_, stream_, &stats_.kernel_launches));
     RJB_CUDA(jfif_ ? LaunchK3Jfif(k3_, stream_, &stats_.kernel_launches) : LaunchK3Output(k3_, stream_, &stats_.kernel_launches));
+    RJB_CUDA(LaunchK4Resize(k4_, stream_, &stats_.kernel_launches));   // resized calls (part of the output stage's interval)
     RJB_CUDA(mark(7));
     RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
     RJB_CUDA(cudaMemcpyAsync(h_counters_.data() + 256, k0_.status, h_images_.size() * sizeof(ScanStatus), cudaMemcpyDeviceToHost, stream_));
@@ -1150,7 +1283,41 @@ int Decoder::Split(const StreamParser* const* streams, int n) {
     return active_lanes_;
 }
 
-int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, bool launch, const uint8_t* remote) {
+const char* CheckResizeArgs(const DecodeParams& params, int n, const DestImage* dsts, const ResizeSpec* resize) {
+    const int fmt = params.output_format;
+    if (fmt != FMT_RGB && fmt != FMT_RGB_PLANAR && fmt != FMT_Y) return "a resized decode writes RGB, RGB_PLANAR or Y";
+    for (int i = 0; i < n; i++) {
+        const ResizeSpec& r = resize[i];
+        if (!ValidFilter(r.filter)) return "unknown resampling filter";
+        if (r.width < 1 || r.height < 1 || r.width > kMaxResizeSize || r.height > kMaxResizeSize) return "resized size out of range";
+        if (!ValidScale(dsts[i].scale_denom)) return "scale denominator must be 1, 2, 4 or 8";
+        const int planes = fmt == FMT_RGB_PLANAR ? 3 : 1;
+        for (int c = 0; c < planes; c++)
+            if (!dsts[i].channel[c]) return "null destination channel";
+        if (dsts[i].pitch[0] < uint64_t(r.width) * (fmt == FMT_RGB ? 3u : 1u)) return "destination pitch below the row's bytes";
+    }
+    return nullptr;
+}
+
+int Decoder::CheckResize(int n, const DecodeParams& params, const DestImage* dsts) {
+    if (peers_.empty()) return kSuccess;
+    uintptr_t range_base = 0;
+    size_t range_size = 0;
+    int range_dev = -1;
+    const int planes = params.output_format == FMT_RGB_PLANAR ? 3 : 1;
+    for (int i = 0; i < n; i++) {
+        for (int c = 0; c < planes; c++) {
+            const uintptr_t ptr = reinterpret_cast<uintptr_t>(dsts[i].channel[c]);
+            if (!(range_size != 0 && ptr >= range_base && ptr - range_base < range_size))
+                range_dev = DeviceOfPointer(dsts[i].channel[c], &range_base, &range_size);
+            if (range_dev >= 0 && range_dev != device_id_) return Fail(kInvalidParameter, "resized destination on another device");
+        }
+    }
+    return kSuccess;
+}
+
+int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, bool launch, const uint8_t* remote,
+                      const ResizeSpec* resize) {
     // validate the whole batch before anything is launched: an error leaves every destination untouched
     for (int i = 0; i < n; i++) {
         if (!streams[i]) return Fail(kInvalidParameter, "null stream handle in batch");
@@ -1172,6 +1339,10 @@ int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodePar
     }
     if (params.output_format < FMT_NATIVE || params.output_format > FMT_RGB_PLANAR)
         return Fail(kInvalidParameter, "unknown output format");
+    if (resize) {
+        const int st = CheckResize(n, params, dsts);
+        if (st != kSuccess) return st;
+    }
     DecodeParams lane_params = params;
     lane_params.color = color_;
     Split(streams, n);
@@ -1203,7 +1374,7 @@ int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodePar
         Lane& lane = lanes_[l];
         const int first = chunk_first_[l], cnt = chunk_first_[l + 1] - first;
         lane.set_host_mark(0, NowMs());
-        int st = lane.Build(streams + first, cnt, lane_params, dsts + first, remote ? remote + first : nullptr);
+        int st = lane.Build(streams + first, cnt, lane_params, dsts + first, remote ? remote + first : nullptr, resize ? resize + first : nullptr);
         if (st == kSuccess) st = launch ? lane.LaunchAll(true, profiling_, upload_stream_) : lane.Upload(upload_stream_);
         if (st != kSuccess) {
             for (int k = 0; k < active_lanes_; k++) lanes_[k].Sync();   // do not leave work in flight behind an error (the failed lane's included)
@@ -1262,17 +1433,17 @@ void Decoder::Aggregate() {
     }
 }
 
-int Decoder::Decode(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts) {
+int Decoder::Decode(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const ResizeSpec* resize) {
     std::lock_guard<std::mutex> lock(mutex_);
     if (!initialized_) return Fail(kNotInitialized, "decoder not initialised");
     if (!streams || !dsts || n < 0) return kInvalidParameter;
     if (n == 0) return kSuccess;
     sharded_ = false;
-    if (!peers_.empty() && n >= 2) return DecodeSharded(streams, n, params, dsts);
+    if (!peers_.empty() && n >= 2 && !resize) return DecodeSharded(streams, n, params, dsts);
     DeviceGuard guard(device_id_);
     prepared_ = false;
     const auto t0 = std::chrono::steady_clock::now();
-    int st = BuildAll(streams, n, params, dsts, true);
+    int st = BuildAll(streams, n, params, dsts, true, nullptr, resize);
     if (st != kSuccess) return st;
     const auto t1 = std::chrono::steady_clock::now();
     st = FinishAll();
@@ -1387,13 +1558,13 @@ int Decoder::DecodeSharded(const StreamParser* const* streams, int n, const Deco
     return status;
 }
 
-int Decoder::Prepare(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts) {
+int Decoder::Prepare(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const ResizeSpec* resize) {
     std::lock_guard<std::mutex> lock(mutex_);
     if (!initialized_) return Fail(kNotInitialized, "decoder not initialised");
     if (!streams || !dsts || n <= 0) return kInvalidParameter;
     DeviceGuard guard(device_id_);
     prepared_ = false;
-    int st = BuildAll(streams, n, params, dsts, false);
+    int st = BuildAll(streams, n, params, dsts, false, nullptr, resize);
     if (st != kSuccess) return st;
     for (int l = 0; l < active_lanes_; l++) {
         st = lanes_[l].Sync();

@@ -24,6 +24,7 @@
 
 #include "device_types.h"
 #include "jpeg_parser.h"
+#include "resample.h"
 #include "stages.h"
 
 namespace rjb {
@@ -46,6 +47,15 @@ struct DestImage {
 constexpr int kScaledKernels = 3;   // reduced-size IDCT kernels: scale 1/2, 1/4, 1/8
 inline bool ValidScale(int d) { return d == 1 || d == 2 || d == 4 || d == 8; }
 inline int ScaleIndex(int d) { return d == 2 ? 0 : d == 4 ? 1 : 2; }   // d > 1: index of its reduced-size kernel
+// Size and filter of one picture of a resized decode (RocJpegB200Resize without the denominator, which DestImage carries)
+struct ResizeSpec {
+    uint32_t width, height;   // 1 .. kMaxResizeSize
+    int32_t filter;           // ResampleFilter (resample.h)
+};
+
+// The argument checks of a resized decode that need no device: formats (RGB, RGB_PLANAR, Y), filters, sizes, denominators,
+// destination channels and pitches. nullptr when they hold, else why not (INVALID_PARAMETER).
+const char* CheckResizeArgs(const DecodeParams& params, int n, const DestImage* dsts, const ResizeSpec* resize);
 
 class DeviceBuffer {
   public:
@@ -133,7 +143,10 @@ class Lane {
     int Create(int device_id, int sm_count, bool prealloc = true);
     // remote[i] != 0: image i's destination lives on another GPU (stores go over NVLink: rows through the output stage, not the
     // IDCT stage's scattered block stores); nullptr: all local
-    int Build(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const uint8_t* remote = nullptr);
+    // resize != nullptr (one per picture): the pictures are decoded into the lane's resize arena and resized from there into
+    // dsts (RGB_PLANAR is decoded interleaved, the vertical pass writes the planes)
+    int Build(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const uint8_t* remote = nullptr,
+              const ResizeSpec* resize = nullptr);
     int Upload(cudaStream_t upload_stream);   // nullptr: use the lane's own stream
     int LaunchAll(bool include_upload, int profiling, cudaStream_t upload_stream);
     int Finish(int profiling);
@@ -161,6 +174,8 @@ class Lane {
     // Everything after the entropy stage: DC integration (integrate_dc), IDCT, fused IDCT + output, output stage, then
     // the counters and per-image status back to the host. mark(i) runs after stage i - 1 (LaunchAll's stage events).
     int LaunchDownstream(bool integrate_dc, const std::function<cudaError_t(int)>& mark);
+    // the resize jobs and tables of a resized call, the arena they live in, and the decode's destinations inside it
+    int PlanResize(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const ResizeSpec* resize);
 
     bool created_ = false;
     std::string err_;
@@ -198,6 +213,12 @@ class Lane {
     K2Args k2s_[kScaledKernels] = {};   // reduced-size IDCT: the pictures of scale 1/2, 1/4, 1/8
     K3Args k3_ = {};
     K23Args k23_ = {};
+    K4Args k4_ = {};
+    std::vector<ResizeJob> h_resize_;          // resized calls: one job per picture (empty otherwise)
+    std::vector<int32_t> h_resize_coef_;       // their tables (K4Args::coef)
+    std::vector<uint32_t> h_rh_tile0_, h_rv_tile0_;
+    std::vector<DestImage> h_resize_dsts_;     // where the decode writes each picture: the resize arena
+    DeviceBuffer d_resize_;                    // decoded pictures + intermediate rows (grow-only)
     bool jfif_ = false;           // the output stage is k3_jfif (RGB / RGB_PLANAR under the libjpeg colour convention)
     bool k2_needed_ = true;       // some image of the lane is not served by the fused kernel
     bool any_direct_ = false, needs_planes_ = false;
@@ -240,10 +261,11 @@ class Decoder {
     int Initialize();   // RocJpegStatus
     // scale_denom > 1: the sizes a decode at that scale writes (rocJpegB200GetScaledImageInfo)
     int GetImageInfo(const StreamParser* s, uint8_t* ncomp, int32_t* css, uint32_t* widths, uint32_t* heights, int scale_denom = 1);
-    int Decode(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts);
+    // resize != nullptr: rocJpegB200DecodeBatchedResized (one spec per picture; never sharded: the handle's own device)
+    int Decode(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const ResizeSpec* resize = nullptr);
 
     // Extension entry points (include/rocjpeg_b200_ext.h)
-    int Prepare(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts);
+    int Prepare(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const ResizeSpec* resize = nullptr);
     int Run();          // launch all stages for the prepared batch and synchronise
     int CopyCoefficients(int image, int16_t* host_out, size_t count);   // component-major raster layout
     int CopyPlanes(int image, uint8_t* host_out, size_t count);
@@ -268,7 +290,11 @@ class Decoder {
     int Wait();
     int Fail(int status, const std::string& why);
     int Split(const StreamParser* const* streams, int n);
-    int BuildAll(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, bool launch, const uint8_t* remote = nullptr);
+    int BuildAll(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, bool launch, const uint8_t* remote = nullptr,
+                 const ResizeSpec* resize = nullptr);
+    // the device check of a resized call (its arguments passed CheckResizeArgs in the C ABI): on a sharded handle every
+    // destination must live on this handle's own device
+    int CheckResize(int n, const DecodeParams& params, const DestImage* dsts);
     int FinishAll();
     void Aggregate();
     // image index of the last call -> the decoder (this or a peer) and lane that holds it, index inside the lane

@@ -208,6 +208,36 @@ cudaError_t LaunchK3Output(const K3Args& a, cudaStream_t stream, uint32_t* launc
 cudaError_t LaunchK3Jfif(const K3Args& a, cudaStream_t stream, uint32_t* launches);
 cudaError_t PreloadK3Jfif();   // part of PreloadK3
 
+// K4 (k4_resize.cu): Pillow's resize of decoded pictures (rocJpegB200DecodeBatchedResized). The decode writes each
+// picture into the lane's resize arena; the horizontal pass turns the source rows the vertical pass reads into
+// intermediate rows of the output width (8 bits, clipped, as Pillow does), the vertical pass writes the caller's buffers.
+constexpr int kResizeThreads = 256;
+constexpr int kResizeTileW = 256;           // output samples per tile (horizontal pass: per warp; vertical: 8 per lane of a warp)
+constexpr int kResizeRowsH = kResizeThreads / 32;   // intermediate rows per tile of the horizontal pass (one per warp)
+struct ResizeJob {
+    const uint8_t* src;       // decoded picture (arena): in_w x in_h samples of `ch` bytes, rows 64-byte aligned
+    uint8_t* tmp;             // intermediate (arena): `rows` rows of out_w samples, rows 64-byte aligned
+    uint8_t* dst[3];          // the caller's channels (RGB: dst[0]; RGB_PLANAR: three planes with dst_pitch; Y: dst[0])
+    uint32_t src_pitch, tmp_pitch, dst_pitch;
+    int32_t in_w, out_w, out_h;
+    int32_t ch;               // bytes per sample of src and tmp: 3 (RGB, RGB_PLANAR) or 1 (Y)
+    int32_t fmt;              // FMT_RGB, FMT_RGB_PLANAR or FMT_Y
+    int32_t y0, rows;         // source rows y0 .. y0 + rows - 1 feed the vertical pass (Pillow's ybox)
+    uint32_t h_coef, v_coef;  // tables in K4Args::coef: out_size int2 bounds (first sample, count), then out_size x ksize taps
+    int32_t h_ksize, v_ksize;
+};
+struct K4Args {
+    const ResizeJob* jobs;
+    const int32_t* coef;          // the lane's tables, de-duplicated by (in size, out size, filter)
+    const uint32_t* h_tile0;      // njobs + 1: first horizontal tile of each job (a tile = kResizeTileW samples of kResizeRowsH rows)
+    const uint32_t* v_tile0;      // njobs + 1: first vertical tile of each job (a tile = one warp)
+    int njobs;
+    uint32_t h_tiles, v_tiles;
+};
+// Both passes, one launch each (none without jobs).
+cudaError_t LaunchK4Resize(const K4Args& a, cudaStream_t stream, uint32_t* launches);
+cudaError_t PreloadK4();
+
 // Load the stages' kernels now instead of at their first launch.
 cudaError_t PreloadK1();
 cudaError_t PreloadK2();
