@@ -129,6 +129,13 @@ cudaError_t DeviceBuffer::Reserve(size_t bytes) {
         return e;
     }
     cap_ = want;
+    if (const int poison = PoisonByte(); poison >= 0) {
+        // (the lanes' streams are non-blocking and do not wait for the legacy stream: the fill must be done before
+        // anything is enqueued on them, Lane::Create's counter memset included)
+        e = cudaMemset(ptr_, poison, want);
+        if (e == cudaSuccess) e = cudaDeviceSynchronize();
+        return e;
+    }
     return cudaSuccess;
 }
 

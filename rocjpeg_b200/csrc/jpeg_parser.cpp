@@ -32,6 +32,11 @@ inline uint32_t Rd16(const uint8_t* p) { return (uint32_t(p[0]) << 8) | p[1]; }
 inline size_t Align16(size_t v) { return (v + 15) & ~size_t(15); }
 }  // namespace
 
+int PoisonByte() {
+    const char* v = std::getenv("ROCJPEG_B200_POISON");
+    return (v && *v) ? int(std::strtol(v, nullptr, 0) & 0xFF) : -1;
+}
+
 // ------------------------------------------------------------ StagingBuffer
 
 StagingBuffer::~StagingBuffer() { Release(); }
@@ -71,6 +76,7 @@ uint8_t* StagingBuffer::Reserve(size_t bytes) {
     }
     ptr_ = static_cast<uint8_t*>(p);
     cap_ = want;
+    if (const int poison = PoisonByte(); poison >= 0) std::memset(ptr_, poison, cap_);
     return ptr_;
 }
 
@@ -84,6 +90,11 @@ inline int Log2Ceil(size_t v) {
     int l = 0;
     while ((size_t(1) << l) < v) l++;
     return l;
+}
+
+inline uint8_t* Poisoned(void* p, size_t bytes) {   // a block recycled from the free list too (ROCJPEG_B200_POISON)
+    if (const int poison = PoisonByte(); p && poison >= 0) std::memset(p, poison, bytes);
+    return static_cast<uint8_t*>(p);
 }
 }  // namespace
 
@@ -102,7 +113,7 @@ uint8_t* PinnedPool::Alloc(size_t bytes, size_t* cap, bool* pinned) {
         uint8_t* p = free_[size_t(cls)].back();
         free_[size_t(cls)].pop_back();
         *pinned = true;
-        return p;
+        return Poisoned(p, want);
     }
     if (!no_driver_ && slab_left_ < want) {
         // the tail of the old slab is abandoned (at most half of it, the slabs double)
@@ -128,13 +139,13 @@ uint8_t* PinnedPool::Alloc(size_t bytes, size_t* cap, bool* pinned) {
         slab_ += want;
         slab_left_ -= want;
         *pinned = true;
-        return p;
+        return Poisoned(p, want);
     }
     // no CUDA driver (host-only unit tests) or page-locking failed: pageable memory, decode still works from it
     void* p = nullptr;
     if (posix_memalign(&p, 4096, want) != 0) p = nullptr;
     *pinned = false;
-    return static_cast<uint8_t*>(p);
+    return Poisoned(p, want);
 }
 
 void PinnedPool::Free(uint8_t* p, size_t cap, bool pinned) {

@@ -35,6 +35,12 @@
 
 namespace rjb {
 
+// ROCJPEG_B200_POISON=<byte> (test knob; decimal or 0x..): every device arena and every grant of page-locked staging is
+// filled with that byte before first use, so that a kernel reading memory no call wrote shows in the output instead of
+// finding cudaMalloc's zeros or an earlier call's values. -1 when unset. Read at each allocation, so a test can set it
+// before creating a handle.
+int PoisonByte();
+
 // Grow-only host buffer; page-locked (cudaHostAlloc, portable + mapped) when a
 // CUDA driver is present, plain aligned memory otherwise (CPU-only unit tests).
 class StagingBuffer {

@@ -14,10 +14,8 @@ def roi_dims(orc, info, crop):
     return rc, w, h
 
 
-def alloc_outputs(orc, info, fmt, crop, pitch_pad=0, misalign=0):
-    """Returns (dest list for api.Decoder, torch buffers, pitches, shapes)."""
-    import torch
-
+def output_layout(orc, info, fmt, crop, pitch_pad=0):
+    """(shapes, pitches) of the destination channels of one picture: (rows, valid bytes per row) and the pitch of each."""
     shapes = oracle.output_shapes(info, fmt, crop, orc)
     pitches = [rb + pitch_pad for (_, rb) in shapes]
     css = oracle.CSS[info.css]
@@ -25,6 +23,14 @@ def alloc_outputs(orc, info, fmt, crop, pitch_pad=0, misalign=0):
         pitches[2] = pitches[1]          # U and V share pitch[1] (src/rocjpeg_decoder.cpp:589-597)
     if fmt == "rgb_planar":
         pitches[1] = pitches[2] = pitches[0]
+    return shapes, pitches
+
+
+def alloc_outputs(orc, info, fmt, crop, pitch_pad=0, misalign=0):
+    """Returns (dest list for api.Decoder, torch buffers, pitches, shapes)."""
+    import torch
+
+    shapes, pitches = output_layout(orc, info, fmt, crop, pitch_pad)
     bufs, dest = [], []
     for (rows, _), p in zip(shapes, pitches):
         t = torch.full((rows * p + misalign + 64,), FILL, dtype=torch.uint8, device="cuda")
