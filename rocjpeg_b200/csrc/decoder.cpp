@@ -183,10 +183,22 @@ int Lane::Sync() {
     return kSuccess;
 }
 
+int Lane::WaitEvent(cudaEvent_t ev) {
+    RJB_CUDA(cudaStreamWaitEvent(stream_, ev, 0));
+    return kSuccess;
+}
+
 Decoder::Decoder(int backend, int device_id) : backend_(backend), device_id_(device_id) {}
 
 Decoder::~Decoder() {   // lanes release their own streams, events and arenas
+    if (ev_caller_) cudaEventDestroy(ev_caller_);
     if (upload_stream_) cudaStreamDestroy(upload_stream_);
+}
+
+int Decoder::RecordCaller() {
+    DeviceGuard guard(device_id_);
+    RJB_CUDA(cudaEventRecord(ev_caller_, cudaStreamLegacy));
+    return kSuccess;
 }
 
 int Decoder::Fail(int status, const std::string& why) {
@@ -221,6 +233,7 @@ int Decoder::Initialize() {
     int prio_lo = 0, prio_hi = 0;
     RJB_CUDA(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
     RJB_CUDA(cudaStreamCreateWithPriority(&upload_stream_, cudaStreamNonBlocking, prio_hi));
+    RJB_CUDA(cudaEventCreateWithFlags(&ev_caller_, cudaEventDisableTiming));
     profiling_ = EnvInt("ROCJPEG_B200_PROFILE", 0);
     {   // ROCJPEG_B200_COLOR=libjpeg: callers that cannot reach the extension API (the reference's samples) decode RGB as libjpeg-turbo does
         const char* c = std::getenv("ROCJPEG_B200_COLOR");
@@ -1306,7 +1319,7 @@ const char* CheckResizeArgs(const DecodeParams& params, int n, const DestImage* 
     return nullptr;
 }
 
-int Decoder::CheckResize(int n, const DecodeParams& params, const DestImage* dsts) {
+int Decoder::CheckOwnDevice(int n, const DecodeParams& params, const DestImage* dsts) {
     if (peers_.empty()) return kSuccess;
     uintptr_t range_base = 0;
     size_t range_size = 0;
@@ -1317,7 +1330,7 @@ int Decoder::CheckResize(int n, const DecodeParams& params, const DestImage* dst
             const uintptr_t ptr = reinterpret_cast<uintptr_t>(dsts[i].channel[c]);
             if (!(range_size != 0 && ptr >= range_base && ptr - range_base < range_size))
                 range_dev = DeviceOfPointer(dsts[i].channel[c], &range_base, &range_size);
-            if (range_dev >= 0 && range_dev != device_id_) return Fail(kInvalidParameter, "resized destination on another device");
+            if (range_dev >= 0 && range_dev != device_id_) return Fail(kInvalidParameter, "destination on another device (a call that is not sharded)");
         }
     }
     return kSuccess;
@@ -1346,8 +1359,8 @@ int Decoder::BuildAll(const StreamParser* const* streams, int n, const DecodePar
     }
     if (params.output_format < FMT_NATIVE || params.output_format > FMT_RGB_PLANAR)
         return Fail(kInvalidParameter, "unknown output format");
-    if (resize) {
-        const int st = CheckResize(n, params, dsts);
+    if (!remote) {   // (a sharded call's share: remote[] says which destinations live on another device)
+        const int st = CheckOwnDevice(n, params, dsts);
         if (st != kSuccess) return st;
     }
     DecodeParams lane_params = params;
@@ -1450,7 +1463,11 @@ int Decoder::Decode(const StreamParser* const* streams, int n, const DecodeParam
     DeviceGuard guard(device_id_);
     prepared_ = false;
     const auto t0 = std::chrono::steady_clock::now();
-    int st = BuildAll(streams, n, params, dsts, true, nullptr, resize);
+    // the uploads wait for the caller's work on the legacy default stream; every lane waits for its upload
+    int st = RecordCaller();
+    if (st != kSuccess) return st;
+    RJB_CUDA(cudaStreamWaitEvent(upload_stream_, ev_caller_, 0));
+    st = BuildAll(streams, n, params, dsts, true, nullptr, resize);
     if (st != kSuccess) return st;
     const auto t1 = std::chrono::steady_clock::now();
     st = FinishAll();
@@ -1524,6 +1541,23 @@ int Decoder::DecodeSharded(const StreamParser* const* streams, int n, const Deco
         sub_dsts[d].push_back(dsts[i]);
         sub_remote[d].push_back(uint8_t(int(d) != owner[size_t(i)] ? 1 : 0));
     }
+    // Every device that holds destinations marks the caller's work on its legacy default stream; the uploads of every
+    // device that decodes a share (and behind them its lanes) wait for all those marks - a peer storing into this
+    // device's buffers included.
+    std::vector<cudaEvent_t> caller;
+    for (int d = 0; d < ndev; d++) {
+        if (std::find(owner.begin(), owner.end(), d) == owner.end()) continue;
+        Decoder* dec = d == 0 ? this : peers_[size_t(d - 1)].get();
+        const int st = dec->RecordCaller();
+        if (st != kSuccess) return Fail(st, dec->last_error());
+        caller.push_back(dec->ev_caller_);
+    }
+    for (int d = 0; d < ndev; d++) {
+        if (sub_streams[size_t(d)].empty()) continue;
+        Decoder* dec = d == 0 ? this : peers_[size_t(d - 1)].get();
+        DeviceGuard guard(dec->device_id_);
+        for (cudaEvent_t ev : caller) RJB_CUDA(cudaStreamWaitEvent(dec->upload_stream_, ev, 0));
+    }
     // enqueue everything on every device - one submitter thread per device, the caller's thread taking
     // this handle's device - then join: the devices run concurrently
     int status = kSuccess;
@@ -1585,8 +1619,12 @@ int Decoder::Run() {
     std::lock_guard<std::mutex> lock(mutex_);
     if (!initialized_ || !prepared_) return Fail(kNotInitialized, "no prepared batch");
     DeviceGuard guard(device_id_);
+    // nothing is uploaded: every lane waits for the caller's work on the legacy default stream itself
+    int st = RecordCaller();
+    if (st != kSuccess) return st;
     for (int l = 0; l < active_lanes_; l++) {
-        int st = lanes_[l].LaunchAll(false, profiling_, nullptr);
+        st = lanes_[l].WaitEvent(ev_caller_);
+        if (st == kSuccess) st = lanes_[l].LaunchAll(false, profiling_, nullptr);
         if (st != kSuccess) return Fail(st, lanes_[l].last_error());
     }
     return FinishAll();

@@ -151,6 +151,7 @@ class Lane {
     int LaunchAll(bool include_upload, int profiling, cudaStream_t upload_stream);
     int Finish(int profiling);
     int Sync();
+    int WaitEvent(cudaEvent_t ev);   // the lane's later work waits for `ev`
     int CopyCoefficients(int image, int16_t* host_out, size_t count);
     int CopyPlanes(int image, uint8_t* host_out, size_t count);
     int CopySegment(int image, uint32_t segment, uint8_t* host_out, size_t capacity, uint32_t* nbytes);
@@ -288,13 +289,15 @@ class Decoder {
     int DecodeSharded(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts);
     int Submit(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, const uint8_t* remote);   // async part
     int Wait();
+    int RecordCaller();   // ev_caller_ on this device's legacy default stream, behind what the caller enqueued there so far
     int Fail(int status, const std::string& why);
     int Split(const StreamParser* const* streams, int n);
     int BuildAll(const StreamParser* const* streams, int n, const DecodeParams& params, const DestImage* dsts, bool launch, const uint8_t* remote = nullptr,
                  const ResizeSpec* resize = nullptr);
-    // the device check of a resized call (its arguments passed CheckResizeArgs in the C ABI): on a sharded handle every
-    // destination must live on this handle's own device
-    int CheckResize(int n, const DecodeParams& params, const DestImage* dsts);
+    // the device check of a call that is not sharded (one picture, a resized call, Prepare): on a sharded handle every
+    // destination must live on this handle's own device - the call writes from that device only, after the caller's work
+    // on that device's legacy default stream only
+    int CheckOwnDevice(int n, const DecodeParams& params, const DestImage* dsts);
     int FinishAll();
     void Aggregate();
     // image index of the last call -> the decoder (this or a peer) and lane that holds it, index inside the lane
@@ -310,6 +313,10 @@ class Decoder {
     int sm_count_ = 0;
     Lane lanes_[kMaxLanes];
     cudaStream_t upload_stream_ = nullptr;   // all host->device traffic, serialised in lane order
+    // Recorded on the device's legacy default stream at the start of a call that writes the caller's memory; the call's
+    // work waits for it. The lanes' and the upload stream are non-blocking, so without it a decode would overwrite a
+    // destination that work the caller has already enqueued there (a framework's default stream) still writes or reads.
+    cudaEvent_t ev_caller_ = nullptr;
     int active_lanes_ = 0;
     int chunk_first_[kMaxLanes + 1] = {};   // image range of each lane's chunk
     BatchStats stats_;

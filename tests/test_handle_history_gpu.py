@@ -162,8 +162,8 @@ def stream(data):
 
 
 class Call:
-    """One entry (or a decoy of it) with its destinations. They are allocated here, before any call: torch.full runs on
-    torch's stream, which the library's non-blocking streams do not wait for - allocate, synchronise, then call."""
+    """One entry (or a decoy of it) with its destinations. They are allocated here, before any call, and the callers
+    synchronise before calling (test_stream_order_gpu.py tests the call's own ordering after torch's default stream)."""
 
     def __init__(self, orc, e, datas=None, crop=None):
         import torch
