@@ -806,6 +806,18 @@ int Lane::Build(const StreamParser* const* streams, int n, const DecodeParams& c
     // of 4K pictures those waits hold SM slots the next wave needs (c4_dri 3.29 -> 3.65 ms)
     const int dc_limit = EnvInt("ROCJPEG_B200_DC_IMAGE_MCUS", n >= 16 ? 2 * kK1DcMaxMcus : kK1DcMaxMcus);
     k1_.k1_dc = k1_fused_ && most_mcus <= uint32_t(std::max(0, dc_limit)) && EnvInt("ROCJPEG_B200_NO_K1_DC", 0) == 0 ? 1 : 0;
+    // ... and destuffs the raw bytes itself (k1_huffman.cu: StageInline), so that no K0 runs, when every picture is one restart
+    // interval (no DRI) whose buffer ends in the FF D9 that closes its scan - what encoders write. Whatever else the bytes
+    // hold that only K0 handles (a marker before that FF D9, a truncated interval) makes the lane redo the decode on K0's
+    // clean stream (Finish). ROCJPEG_B200_NO_INLINE_DESTUFF=1 keeps K0.
+    inline_destuff_ = k1_fused_ && EnvInt("ROCJPEG_B200_NO_INLINE_DESTUFF", 0) == 0;
+    for (int i = 0; i < n && inline_destuff_; i++) {
+        const ImageDesc& im = h_images_[size_t(i)];
+        const RawScan& rs = streams[i]->raw();
+        inline_destuff_ = im.restart_interval == 0 && im.nseg == 1 && rs.nbytes >= 3 && rs.host[rs.nbytes - 2] == 0xFF &&
+                          rs.host[rs.nbytes - 1] == 0xD9;
+    }
+    k1_.inline_destuff = inline_destuff_ ? 1 : 0;
     k2_ = K2Args{};
     k2_.nimages = n;
     k2_.total_tiles = k2tile;
@@ -1020,6 +1032,7 @@ int Lane::Upload(cudaStream_t up) {
     k1_.img_cta0 = reinterpret_cast<const uint32_t*>(d + L.cta0);
     k1_.img_dctile0 = reinterpret_cast<const uint32_t*>(d + L.dctile0);
     k1_.scan = base + o_scan;
+    k1_.raw = k0_.raw;
     k1_.luts = reinterpret_cast<const HuffLutSet*>(d + L.luts);
     k1_.state = reinterpret_cast<uint32_t*>(base + o_state);
     k1_.used = reinterpret_cast<uint32_t*>(base + o_used);
@@ -1141,10 +1154,14 @@ int Lane::LaunchAll(bool include_upload, int profiling_, cudaStream_t up) {
     }
     // "published" flags of the CTAs, the ticket counter, the CTAs' DC flags
     if (k1_fused_) RJB_CUDA(cudaMemsetAsync(k1_.cta_flag, 0, size_t(k1_.total_ctas) * 8 + 4, stream_));
-    // K0: end of slice, destuffing, restart intervals -> clean stream + segment table, all on the device
-    if (!(include_upload && upload_by_ == kUploadGather))   // cudaMemcpy upload, or a resident batch run again: the reduction is its own launch
-        RJB_CUDA(LaunchK0Reduce(k0_, stream_, &stats_.kernel_launches));
-    RJB_CUDA(LaunchK0Destuff(k0_, stream_, &stats_.kernel_launches));
+    // K0: end of slice, destuffing, restart intervals -> clean stream + segment table, all on the device (inline
+    // destuffing: k1_fused does it, and the taps that need the clean stream run K0 when asked)
+    if (!inline_destuff_) {
+        if (!(include_upload && upload_by_ == kUploadGather))   // cudaMemcpy upload, or a resident batch run again: the reduction is its own launch
+            RJB_CUDA(LaunchK0Reduce(k0_, stream_, &stats_.kernel_launches));
+        RJB_CUDA(LaunchK0Destuff(k0_, stream_, &stats_.kernel_launches));
+    }
+    clean_valid_ = !inline_destuff_;
     RJB_CUDA(mark(2));
     if (k1_fused_) {
         RJB_CUDA(LaunchK1Fused(k1_, stream_, &stats_.kernel_launches));
@@ -1202,11 +1219,23 @@ int Lane::Finish(int profiling_) {
         // The stream did not re-synchronise within the rounds launched up front: keep
         // going until a round changes nothing at any CTA boundary, then redo everything
         // downstream of the synchronisation.
+        // (inline destuffing: the count also holds what only K0 handles - K0 runs now, and the entropy stage starts over
+        // from round 0 on its clean stream)
+        K1Args k1 = k1_;
+        k1.inline_destuff = 0;
+        if (inline_destuff_) {
+            RJB_CUDA(LaunchK0Reduce(k0_, stream_, &stats_.kernel_launches));
+            RJB_CUDA(LaunchK0Destuff(k0_, stream_, &stats_.kernel_launches));
+            clean_valid_ = true;
+            RJB_CUDA(cudaMemsetAsync(k1.counters, 0, 4, stream_));
+            RJB_CUDA(LaunchK1Sync(k1, 0, stream_, &stats_.kernel_launches));
+            last = 0;
+        }
         uint32_t guard = 0;
         for (;;) {
             uint32_t slot = std::min<uint32_t>(last + 1, kMaxSyncRounds - 1);
-            RJB_CUDA(cudaMemsetAsync(k1_.counters + slot, 0, 4, stream_));
-            RJB_CUDA(LaunchK1Sync(k1_, int(slot), stream_, &stats_.kernel_launches));
+            RJB_CUDA(cudaMemsetAsync(k1.counters + slot, 0, 4, stream_));
+            RJB_CUDA(LaunchK1Sync(k1, int(slot), stream_, &stats_.kernel_launches));
             RJB_CUDA(cudaMemcpyAsync(h_counters_.data(), k1_.counters, 256, cudaMemcpyDeviceToHost, stream_));
             RJB_CUDA(cudaStreamSynchronize(stream_));
             stats_.sync_rounds++;
@@ -1215,9 +1244,9 @@ int Lane::Finish(int profiling_) {
             if (++guard > k1_.total_ctas + 2) return Fail(kExecutionFailed, "entropy decoder failed to converge");
         }
         RJB_CUDA(cudaMemsetAsync(k1_.blk_rec, 0xFF, coef_blocks_ * sizeof(BlockRec), stream_));
-        RJB_CUDA(cudaMemsetAsync(k1_.counters + 2 * kMaxSyncRounds, 0, 4, stream_));   // the first write pass counted its entries already
-        RJB_CUDA(LaunchK1ClearShort(k1_, stream_, &stats_.kernel_launches));   // ... and may have reported pictures short that are not
-        RJB_CUDA(LaunchK1Write(k1_, stream_, &stats_.kernel_launches));
+        RJB_CUDA(cudaMemsetAsync(k1.counters + 2 * kMaxSyncRounds, 0, 4, stream_));   // the first write pass counted its entries already
+        RJB_CUDA(LaunchK1ClearShort(k1, stream_, &stats_.kernel_launches));   // ... and may have reported pictures short that are not
+        RJB_CUDA(LaunchK1Write(k1, stream_, &stats_.kernel_launches));
         // k1_write leaves DC differences, also where k1_fused had integrated them; no stage events (the host waited in between)
         const int st = LaunchDownstream(true, [](int) { return cudaSuccess; });
         if (st != kSuccess) return st;
@@ -1688,6 +1717,17 @@ int Lane::CopySegment(int image, uint32_t segment, uint8_t* host_out, size_t cap
     if (segment >= im.nseg) return kInvalidParameter;
     SegmentDesc sd;
     RJB_CUDA(cudaStreamSynchronize(stream_));
+    if (!clean_valid_) {
+        // inline destuffing left no clean stream: K0 makes it now, the status words stay those of the decode
+        std::vector<ScanStatus> keep(h_images_.size());
+        uint32_t launches = 0;
+        RJB_CUDA(cudaMemcpy(keep.data(), k0_.status, keep.size() * sizeof(ScanStatus), cudaMemcpyDeviceToHost));
+        RJB_CUDA(LaunchK0Reduce(k0_, stream_, &launches));
+        RJB_CUDA(LaunchK0Destuff(k0_, stream_, &launches));
+        RJB_CUDA(cudaMemcpyAsync(k0_.status, keep.data(), keep.size() * sizeof(ScanStatus), cudaMemcpyHostToDevice, stream_));
+        RJB_CUDA(cudaStreamSynchronize(stream_));
+        clean_valid_ = true;
+    }
     RJB_CUDA(cudaMemcpy(&sd, k1_.segments + im.seg0 + segment, sizeof(sd), cudaMemcpyDeviceToHost));
     *nbytes = sd.nbytes;
     if (host_out) {

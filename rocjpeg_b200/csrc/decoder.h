@@ -227,6 +227,8 @@ class Lane {
     // destuffing pass's per-tile prefix elements), and k1_fused or `sync_rounds_` k1_sync rounds up front + k1_write.
     enum UploadBy { kUploadPerPicture, kUploadRuns, kUploadGather } upload_by_ = kUploadPerPicture;
     bool k1_fused_ = false;
+    bool inline_destuff_ = false;   // k1_fused destuffs the raw bytes itself, no K0 runs (chosen by Build, replayed by every Run)
+    bool clean_valid_ = false;      // the clean stream and the segment table hold the current batch (K0 ran)
     int sync_rounds_ = 2;
     size_t scan_bytes_ = 0, raw_bytes_ = 0, coef_blocks_ = 0, entry_count_ = 0, plane_bytes_ = 0, nsub_total_ = 0;
     uint32_t nseg_total_ = 0;

@@ -232,8 +232,10 @@ __device__ __forceinline__ uint32_t DecodeCount(uint32_t slot_sa, const LutView&
     }
     const uint32_t nb = ln.Blocks(), acc = ln.acc;
     *nnz_out = (((acc >> 11) & 0x3FFu) + 7u) & ~7u;   // a thread's run of the entry stream is padded to whole 32-byte stores
-    // bits consumed past the end (meaningful when the end is word-aligned, i.e. whenever a successor exists)
-    return PackState(acc & 63u, int((uint32_t(StateC(key)) + nb) % uint32_t(bpm)), int((acc >> 21) & 63u), nb > 0xFFFFu ? 0xFFFFu : nb);
+    // bits consumed past the end: the loop stops at the end rounded up to a whole word, the successor starts at the end
+    // itself (they differ for the inline-destuffed subsequences of k1_fused, whose ends fall on any byte; for the others
+    // only in a restart interval's last subsequence, which hands over nothing)
+    return PackState(((acc & 63u) + ((0u - end_bit) & 31u)) & 63u, int((uint32_t(StateC(key)) + nb) % uint32_t(bpm)), int((acc >> 21) & 63u), nb > 0xFFFFu ? 0xFFFFu : nb);
 }
 
 // Per-thread description of its subsequence. Subsequence g of an image covers bytes [g S, (g+1) S) of the
@@ -250,7 +252,24 @@ struct Sub {
     uint64_t start;    // byte offset of the subsequence in the scan arena
 };
 
-template <int S>
+// Segment k of the batch. Inline destuffing (no K0 ran, the table is not written): the picture's one restart interval,
+// measured in raw bytes up to the FF D9 that ends the caller's buffer; subsequence g of the picture then covers raw bytes
+// [g S, (g+1) S) of its entropy-coded data, and StageInline turns them into at most S destuffed bytes. (INL: compiled for
+// inline destuffing - the instance of k1_fused that LaunchK1Fused picks when K1Args::inline_destuff is set; every other
+// kernel, and k1_fused for the lanes that keep K0, has none of it.)
+template <bool INL>
+__device__ __forceinline__ SegmentDesc SegmentOf(const K1Args& a, const ImageDesc& im, uint32_t k) {
+    if (!INL) return a.segments[k];
+    SegmentDesc sd;
+    sd.data_off = im.data_off;
+    sd.nbytes = im.raw_len - 2u;
+    sd.sub0 = im.sub0;
+    sd.blk_first = 0;
+    sd.blk_count = im.nblocks;
+    return sd;
+}
+
+template <int S, bool INL>
 __device__ __forceinline__ Sub Locate(const K1Args& a, const ImageDesc& im, int64_t gi, bool use_cache) {
     Sub s;
     s.in_range = s.active = gi >= int64_t(im.sub0) && gi < int64_t(im.sub0) + int64_t(im.nsub);
@@ -272,7 +291,7 @@ __device__ __forceinline__ Sub Locate(const K1Args& a, const ImageDesc& im, int6
         }
         k = im.seg0 + lo;
     }
-    const SegmentDesc sd = a.segments[k];
+    const SegmentDesc sd = SegmentOf<INL>(a, im, k);
     const uint32_t j = g - sd.sub0;
     const uint32_t nchunks = (sd.nbytes + S - 1) / S;
     s.seg = k;
@@ -360,20 +379,123 @@ __device__ __forceinline__ void StageSlotVec(uint32_t* slot, const uint8_t* src,
     if (v != K1Smem<S>::kSlotVecs - 1) w[3] = ByteSwap32(q.w);
 }
 
+// Inline destuffing (K1Args::inline_destuff, k1_fused only): slot j receives raw bytes [j S, j S + S + 4) of the picture's
+// entropy-coded data (aligned 16-byte loads shifted by raw_skip), then each thread destuffs its own slot in place by K0's
+// rules (k0_core.cuh: ClassifyPiece): FF 00 -> FF, FF FF -> fill; a slot without FF stays as it is. The data end at the FF D9
+// that ends the caller's buffer. Behind each slot's destuffed bytes go the picture's next destuffed bytes - the look-ahead
+// of a symbol that crosses the slot's end, taken from the next slot once it is compacted, for the CTA's last slot from the
+// raw bytes behind it - and zeros behind the data's end, as K0 leaves them. What only K0 handles - a marker before that
+// FF D9, a picture without destuffed bytes, a slot too short to serve its neighbour's look-ahead - counts in counters[0]:
+// the host then redoes the lane on K0's clean stream (Lane::Finish). me.end_bit becomes the slot's destuffed length; the
+// result is where the picture's real bytes end in the slot's buffer, in bits (past its end when they do not end there).
 template <int S>
-__device__ __forceinline__ LutView StageCta(K1Smem<S>& sm, uint32_t* lut, const K1Args& a, const ImageDesc& im, const Sub& me) {
+__device__ __forceinline__ uint32_t StageInline(K1Smem<S>& sm, const K1Args& a, const ImageDesc& im, Sub& me) {
+    constexpr int kStride = K1Smem<S>::kSlotStride, V = S / 16 + 1;
+    const int tid = threadIdx.x;
+    const uint8_t* const raw = a.raw + im.raw_off;   // 16-byte aligned; the data start raw_skip bytes in
+    const uint32_t skip = im.raw_skip, q = skip >> 2, r = 8u * (skip & 3u), data_end = im.raw_len - 2u;
+    const uint32_t st = sm.start[tid];
+    const uint32_t prev = (me.active && st > 0u) ? uint32_t(__ldg(raw + skip + st - 1u)) : 0u;   // a stuffing 00 may open the slot
+    for (int idx = tid; idx < T * V; idx += T) {
+        const int slot = idx / V, v = idx - slot * V;
+        const uint32_t so = sm.start[slot];
+        if (so == ~0u) continue;
+        const uint4* src = reinterpret_cast<const uint4*>(raw + so) + v;
+        const uint4 x = __ldg(src), y = __ldg(src + 1);
+        // words q .. q + 4 of x:y hold the vector's 16 bytes shifted by raw_skip (+ 4 bytes)
+        const uint32_t w0 = q == 0u ? x.x : q == 1u ? x.y : q == 2u ? x.z : x.w;
+        const uint32_t w1 = q == 0u ? x.y : q == 1u ? x.z : q == 2u ? x.w : y.x;
+        uint32_t* w = sm.words + slot * kStride + v * 4;
+        w[0] = ByteSwap32(__funnelshift_r(w0, w1, r));
+        if (v != V - 1) {   // (the last vector: only its first word, which holds the byte after the slot)
+            const uint32_t w2 = q == 0u ? x.z : q == 1u ? x.w : q == 2u ? y.x : y.y;
+            const uint32_t w3 = q == 0u ? x.w : q == 1u ? y.x : q == 2u ? y.y : y.z;
+            const uint32_t w4 = q == 0u ? y.x : q == 1u ? y.y : q == 2u ? y.z : y.w;
+            w[1] = ByteSwap32(__funnelshift_r(w1, w2, r));
+            w[2] = ByteSwap32(__funnelshift_r(w2, w3, r));
+            w[3] = ByteSwap32(__funnelshift_r(w3, w4, r));
+        }
+    }
+    __syncthreads();
+    uint8_t* const b = reinterpret_cast<uint8_t*>(sm.words + tid * kStride);   // byte i of the stream at b[i ^ 3] (big-endian words)
+    uint32_t c = 0;
+    bool bad = false;
+    if (me.active) {
+        const uint32_t n = min(uint32_t(S), data_end - st);   // raw bytes of the slot before the data's end
+        uint32_t i = prev == 0xFFu ? 0u : n;                  // first byte that is not kept in place
+        for (int k = 0; k < S / 4 && i == n; k++) {
+            if (uint32_t(4 * k) >= n) break;
+            uint32_t x = sm.words[tid * kStride + k];
+            if (uint32_t(4 * k + 4) > n) x &= ~(0xFFFFFFFFu >> (8u * (n - uint32_t(4 * k))));
+            const uint32_t m = __vcmpeq4(x, 0xFFFFFFFFu);
+            if (m) i = uint32_t(4 * k) + uint32_t(__clz(m) >> 3);
+        }
+        c = i;
+        uint32_t p = i ? uint32_t(b[(i - 1u) ^ 3u]) : prev;
+        for (; i < n; i++) {
+            const uint32_t x = b[i ^ 3u];
+            const uint32_t nx = i + 1u < n ? uint32_t(b[(i + 1u) ^ 3u]) : (st + n < data_end ? uint32_t(b[n ^ 3u]) : 0xFFu);
+            if (x == 0xFFu && nx != 0u && nx != 0xFFu) bad = true;   // a marker before the buffer's final FF D9
+            if (x != 0xFFu ? p != 0xFFu : nx == 0u) b[(c++) ^ 3u] = uint8_t(x);
+            p = x;
+        }
+        if (c < 16u && (!me.last || c == 0u)) bad = true;
+        me.end_bit = c * 8u;
+    }
+    sm.endbit[tid] = c * 8u;
+    __syncthreads();
+    uint32_t real = 0;   // bytes of the picture's data in the look-ahead
+    if (me.active && tid < T - 1) {
+        const uint8_t* nb = reinterpret_cast<const uint8_t*>(sm.words + (tid + 1) * kStride);
+        const uint32_t cn = sm.endbit[tid + 1] >> 3, e = ((c + 3u) & ~3u) + 12u;
+        for (uint32_t i = c, k = 0; i < e; i++, k++) b[i ^ 3u] = k < cn ? nb[k ^ 3u] : uint8_t(0);
+        real = min(e - c, cn);
+    }
+    if (tid >= T - 32) {   // the last warp: the look-ahead of the CTA's last slot, from the 32 raw bytes behind it
+        const uint32_t sl = sm.start[T - 1];
+        if (sl != ~0u) {
+            const uint32_t lane = uint32_t(tid & 31), cl = sm.endbit[T - 1] >> 3, pos = sl + S + lane;
+            const uint32_t x = pos < data_end ? uint32_t(__ldg(raw + skip + pos)) : 0u;
+            uint32_t nx = __shfl_down_sync(0xFFFFFFFFu, x, 1), p = __shfl_up_sync(0xFFFFFFFFu, x, 1);
+            if (pos + 1u >= data_end) nx = 0xFFu;
+            else if (lane == 31u) nx = __ldg(raw + skip + pos + 1u);
+            if (lane == 0u) p = __ldg(raw + skip + pos - 1u);
+            const bool keep = pos < data_end && (x != 0xFFu ? p != 0xFFu : nx == 0u);
+            const uint32_t km = __ballot_sync(0xFFFFFFFFu, keep), at = __popc(km & ((1u << lane) - 1u)), tot = __popc(km);
+            const uint32_t want = ((cl + 3u) & ~3u) + 12u - cl;
+            uint8_t* lb = reinterpret_cast<uint8_t*>(sm.words + (T - 1) * kStride);
+            if (keep && at < want) lb[(cl + at) ^ 3u] = uint8_t(x);
+            if (lane >= tot && lane < want) lb[(cl + lane) ^ 3u] = 0;
+            if (lane == 0u && tot < want && sl + S + 32u < data_end) bad = true;
+            if (tid == T - 1) real = min(want, tot);
+        }
+    }
+    if (bad) atomicAdd(&a.counters[0], 1u);
+    return me.active ? 8u * (c + real) : 0u;
+}
+
+template <int S, bool INL>
+__device__ __forceinline__ LutView StageCta(K1Smem<S>& sm, uint32_t* lut, const K1Args& a, const ImageDesc& im, Sub& me) {
     const int tid = threadIdx.x;
     sm.start[tid] = me.active ? uint32_t(me.start - im.data_off) : ~0u;
     const LutView lv = StageTables<S>(lut, sm.sched, sm.pair_tab, a, im);
     __syncthreads();
-    constexpr int V = K1Smem<S>::kSlotVecs;
-    for (int idx = tid; idx < T * V; idx += T) {
-        const int slot = idx / V, v = idx - slot * V;
-        const uint32_t st = sm.start[slot];
-        if (st == ~0u) continue;
-        StageSlotVec<S>(sm.words + slot * K1Smem<S>::kSlotStride, a.scan + im.data_off + st, v);
+    uint32_t data_bits = 0;
+    if (INL) {
+        data_bits = StageInline<S>(sm, a, im, me);
+    } else {
+        constexpr int V = K1Smem<S>::kSlotVecs;
+        for (int idx = tid; idx < T * V; idx += T) {
+            const int slot = idx / V, v = idx - slot * V;
+            const uint32_t st = sm.start[slot];
+            if (st == ~0u) continue;
+            StageSlotVec<S>(sm.words + slot * K1Smem<S>::kSlotStride, a.scan + im.data_off + st, v);
+        }
     }
     __syncthreads();
+    // (the staging offsets are not needed any more: the end of the slot's data, as 8 x the shared address of its first
+    // word + 64 + its length in bits, for WriteBody's check)
+    if (INL) sm.start[tid] = 8u * SharedAddr(sm.words + tid * K1Smem<S>::kSlotStride) + 64u + data_bits;
     return lv;
 }
 
@@ -397,7 +519,7 @@ struct SyncOut {
 };
 
 // FUSED: round 0 inside k1_fused - the per-round counter counts nothing here (k1_fused counts boundary mismatches itself).
-template <int S, bool FUSED>
+template <int S, bool FUSED, bool INL>
 __device__ __forceinline__ SyncOut SyncBody(const K1Args& a, K1Smem<S>& sm, uint32_t* lut, int round, int max_iters, const uint32_t cta) {
     SyncOut so;
     so.live = false;
@@ -408,7 +530,7 @@ __device__ __forceinline__ SyncOut SyncBody(const K1Args& a, K1Smem<S>& sm, uint
     const int64_t gi = int64_t(cta) * TO + tid - H;
     const uint32_t g = uint32_t(gi);
     const bool owned = tid >= H;
-    Sub me = Locate<S>(a, im, gi, round > 0);
+    Sub me = Locate<S, INL>(a, im, gi, round > 0);
     if (round > 0 && !owned) me.active = false;   // later rounds read the owner's state instead of a halo
     if (round == 0 && owned && me.in_range) a.sub_seg[g] = me.seg;
     if (round == 0) {
@@ -433,7 +555,7 @@ __device__ __forceinline__ SyncOut SyncBody(const K1Args& a, K1Smem<S>& sm, uint
             old_out = out;
         }
     }
-    const LutView lv = StageCta<S>(sm, lut, a, im, me);
+    const LutView lv = StageCta<S, INL>(sm, lut, a, im, me);
     const int bpm = im.bpm;
     const uint32_t slots_sa = SharedAddr(sm.words);
     const uint32_t sched_sa = SharedAddr(sm.sched);
@@ -542,7 +664,7 @@ __global__ void __launch_bounds__(T) k1_sync(K1Args a, int round, int max_iters)
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint32_t* const lut = reinterpret_cast<uint32_t*>(smem_raw);
     K1Smem<S>& sm = *reinterpret_cast<K1Smem<S>*>(smem_raw + a.lut_smem_bytes);
-    (void)SyncBody<S, false>(a, sm, lut, round, max_iters, blockIdx.x);
+    (void)SyncBody<S, false, false>(a, sm, lut, round, max_iters, blockIdx.x);
 }
 
 // ---------------------------------------------------------------- k1_scan
@@ -614,9 +736,10 @@ __global__ void __launch_bounds__(kScanThreads) k1_scan(K1Args a) {
 // before it), the interval's end for one behind the interval's data, the picture's end for one behind the picture.
 // Clamped so that the split points never decrease, whatever a damaged stream made of the counts.
 constexpr int kDcPosSlot = 32;   // K1Smem::scratch words holding the range (IntegrateDc)
+template <bool INL>
 __device__ __forceinline__ uint32_t BlockPos(const K1Args& a, const ImageDesc& im, const Sub& s, uint32_t excl) {
     if (!s.in_range) return im.nblocks;
-    const SegmentDesc& sd = a.segments[s.seg];
+    const SegmentDesc sd = SegmentOf<INL>(a, im, s.seg);
     const uint32_t p = sd.blk_first + (!s.active ? sd.blk_count : s.first ? 0u : min(excl, sd.blk_count));
     return min(p, im.nblocks);
 }
@@ -625,7 +748,7 @@ __device__ __forceinline__ uint32_t BlockPos(const K1Args& a, const ImageDesc& i
 // state. FUSED (k1_fused): the same CTA has just synchronised - what enters it from the picture's earlier CTAs is read
 // from their partials as soon as each has published them (`cta_flag`), and the state handed over at the CTA boundary is
 // checked against the owner's.
-template <int S, bool FUSED>
+template <int S, bool FUSED, bool INL>
 __device__ __forceinline__ void WriteBody(const K1Args& a, K1Smem<S>& sm, const LutView& lv, uint32_t img, const ImageDesc& im, const Sub& me,
                                           uint32_t st, uint32_t my_nnz, uint32_t key, const uint32_t cta) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -725,7 +848,7 @@ __device__ __forceinline__ void WriteBody(const K1Args& a, K1Smem<S>& sm, const 
     // two threads' runs or two restart intervals is zero padding (position 0, which K2 overwrites
     // with the DC). No clearing, no read-modify-write, no ownership hand-over: a thread decodes
     // exactly the symbols that start inside its subsequence, as in the counting passes.
-    const SegmentDesc sd = a.segments[me.seg];
+    const SegmentDesc sd = SegmentOf<INL>(a, im, me.seg);
     const uint32_t blk0 = sd.blk_first + excl, limit = sd.blk_first + sd.blk_count;
     // running pointers: the current block's record {end-of-entries index, DC} and the next 32-byte
     // entry group of this thread's run; the run never leaves its reservation [n, n_end), the
@@ -794,10 +917,23 @@ __device__ __forceinline__ void WriteBody(const K1Args& a, K1Smem<S>& sm, const 
             ln.CommitWrite(nxt, rp, n, rp_stop, dcv, has_dc);
             if (ln.acc & kAccStop) break;
         }
+        // Inline destuffing: the symbol that ended the picture's last block must end inside the picture's data. Behind
+        // them a thread reads zeros, and how many zero bits it reads before it stops depends on the layout (K0's decode
+        // of the same bytes may come out short where this one did not): counters[0], the host redoes the lane on K0's
+        // stream. A complete scan ends its last block inside its data.
+        // (the read position is 8 wp + (acc & 31) - 64 bits from the slot's start: wp is the address of the word after the
+        // next; sm.start holds the end of the data in the same terms, StageCta)
+        if (INL && uint32_t(reinterpret_cast<uintptr_t>(rp)) == rp_stop && (ln.wp << 3) + (ln.acc & 31u) > sm.start[tid])
+            atomicAdd(&a.counters[0], 1u);
     }
     // per-image status (read back by the host with the round counters): the interval ran out of bytes before its last
     // block (truncated or damaged scan)
-    if (me.last && blk0 < limit && uint32_t(rp - recs) < limit) atomicOr(&a.status[img].flags, kDecodeShort);
+    // (inline destuffing: what the decode found past the data's end depends on the subsequence layout - the host redoes the
+    // picture on K0's layout, counters[0])
+    if (me.last && blk0 < limit && uint32_t(rp - recs) < limit) {
+        atomicOr(&a.status[img].flags, kDecodeShort);
+        if (INL) atomicAdd(&a.counters[0], 1u);
+    }
     // a block still in progress whose DC symbol was ours: the thread that ends it stores only the end index
     if (has_dc && (ln.acc & kAccZMask) != 0 && blk0 < limit && me.end_bit != 0) rp->dc = int16_t(dcv);
     if (n & 7u) {   // last, partial group: padded with entries for position 0, which K2 overwrites with the DC anyway
@@ -832,14 +968,14 @@ __global__ void __launch_bounds__(T) k1_write(K1Args a) {
     const int H = a.halo, TO = T - H;
     const int64_t gi = int64_t(cta) * TO + tid - H;
     const uint32_t g = uint32_t(gi);
-    Sub me = Locate<S>(a, im, gi, true);
+    Sub me = Locate<S, false>(a, im, gi, true);
     if (tid < H) me.active = false;   // halo slots belong to the previous CTA
-    const LutView lv = StageCta<S>(sm, lut, a, im, me);
+    const LutView lv = StageCta<S, false>(sm, lut, a, im, me);
     const uint32_t st = me.active ? a.state[g] : 0;
     const uint32_t my_nnz = me.active ? a.nnz[g] : 0;
     uint32_t key = 0;
     if (me.active && !me.first) key = StateKey(a.state[g - 1]);
-    WriteBody<S, false>(a, sm, lv, img, im, me, st, my_nnz, key, cta);
+    WriteBody<S, false, false>(a, sm, lv, img, im, me, st, my_nnz, key, cta);
 }
 
 // ---------------------------------------------------------------- k1_fused
@@ -853,12 +989,12 @@ __global__ void __launch_bounds__(T) k1_write(K1Args a) {
 // in counters[0], and the host then falls back to the separate kernels for the batch (none on the benchmark batches,
 // forced in tests with ROCJPEG_B200_HALO=1). With K1Args::k1_dc the CTA then turns the DC differences of its share of the
 // picture's blocks into absolute DC values (IntegrateDc), and no DC kernel follows.
-template <int S>
+template <int S, bool INL>
 __device__ void IntegrateDc(const K1Args& a, uint32_t* scratch, uint32_t img, uint32_t cta);
 
 // (the register cap replaces __launch_bounds__(T), which cannot be combined with it: the DC integration behind the write
 // loop would otherwise raise the kernel from the decode loops' 46 registers to 48)
-template <int S>
+template <int S, bool INL>
 __global__ void __maxnreg__(46) k1_fused(K1Args a, int max_iters) {
     PdlEntry();
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -871,7 +1007,11 @@ __global__ void __maxnreg__(46) k1_fused(K1Args a, int max_iters) {
     if (tid == 0) s_ticket = atomicAdd(a.cta_flag + a.total_ctas, 1u);
     __syncthreads();
     const uint32_t cta = s_ticket;
-    SyncOut so = SyncBody<S, true>(a, sm, lut, 0, max_iters, cta);
+    SyncOut so = SyncBody<S, true, INL>(a, sm, lut, 0, max_iters, cta);
+    // inline destuffing, no K0 ran: the picture's first CTA writes its status - a restart interval that ends at the FF D9
+    // closing the buffer - before any CTA of the picture may OR into it (they all wait for its flag below first)
+    if (INL && tid == 0 && cta == __ldg(a.img_cta0 + so.img))
+        a.status[so.img] = ScanStatus{1u, a.images[so.img].raw_len - 2u, 0u, 0u};
     if (tid == 0) s_img = so.img;
     // this CTA's counts and states are in global memory: let the picture's later CTAs see them
     __threadfence();
@@ -890,7 +1030,7 @@ __global__ void __maxnreg__(46) k1_fused(K1Args a, int max_iters) {
     }
     Sub me = so.me;
     if (tid < H) me.active = false;   // halo slots belong to the previous CTA
-    WriteBody<S, true>(a, sm, so.lv, so.img, im, me, me.active ? so.state : 0u, me.active ? so.nnz : 0u, so.used, cta);
+    WriteBody<S, true, INL>(a, sm, so.lv, so.img, im, me, me.active ? so.state : 0u, me.active ? so.nnz : 0u, so.used, cta);
     if (a.k1_dc) {
         // (ticket and picture re-read from shared memory: kept in registers across the write loop they cost two)
         const uint32_t c = *static_cast<volatile uint32_t*>(&s_ticket);
@@ -898,7 +1038,7 @@ __global__ void __maxnreg__(46) k1_fused(K1Args a, int max_iters) {
         __threadfence();
         __syncthreads();
         if (tid == 0) asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(a.cta_flag + c), "r"(2u) : "memory");
-        IntegrateDc<S>(a, sm.scratch, *static_cast<volatile uint32_t*>(&s_img), c);
+        IntegrateDc<S, INL>(a, sm.scratch, *static_cast<volatile uint32_t*>(&s_img), c);
     }
 }
 
@@ -983,7 +1123,7 @@ __device__ __forceinline__ int LoadDc(const BlockRec* r) {
 // picture's earlier CTAs (their per-component sums after the last predictor reset, or the predictors leaving them once
 // known) give the predictors entering each run. Every wait is for a lower ticket, i.e. for a running CTA that itself
 // waits only for lower tickets.
-template <int S>
+template <int S, bool INL>
 __device__ void IntegrateDc(const K1Args& a, uint32_t* scratch, uint32_t img, uint32_t cta) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int kW = T / 32;
@@ -997,10 +1137,10 @@ __device__ void IntegrateDc(const K1Args& a, uint32_t* scratch, uint32_t img, ui
         const uint32_t enter = scratch[3 * kW];
         const int64_t gi = int64_t(cta) * (T - H) + tid - H;
         if (tid == H) {
-            scratch[kDcPosSlot] = BlockPos(a, im, Locate<S>(a, im, gi, false), enter);
+            scratch[kDcPosSlot] = BlockPos<INL>(a, im, Locate<S, INL>(a, im, gi, false), enter);
         } else {
             const uint2 part = a.cta_partial[cta];
-            scratch[kDcPosSlot + 1] = BlockPos(a, im, Locate<S>(a, im, gi + 1, false), part.y + (part.x ? 0u : enter));
+            scratch[kDcPosSlot + 1] = BlockPos<INL>(a, im, Locate<S, INL>(a, im, gi + 1, false), part.y + (part.x ? 0u : enter));
         }
     }
     if (tid == 0 && cta != first) {
@@ -1293,11 +1433,14 @@ cudaError_t LaunchK1Fused(const K1Args& a, cudaStream_t stream, uint32_t* launch
     const int max_iters = T + 1;
     switch (a.sub_bytes) {
         case 32: { const size_t smem = sizeof(K1Smem<32>) + a.lut_smem_bytes; if (smem > 48 * 1024) return cudaErrorInvalidValue;
-                   return LaunchPdl(launches, k1_fused<32>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
+                   return LaunchPdl(launches, a.inline_destuff ? k1_fused<32, true> : k1_fused<32, false>, dim3(a.total_ctas), dim3(T), smem,
+                                    stream, a, max_iters); }
         case 64: { const size_t smem = sizeof(K1Smem<64>) + a.lut_smem_bytes; if (smem > 48 * 1024) return cudaErrorInvalidValue;
-                   return LaunchPdl(launches, k1_fused<64>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
+                   return LaunchPdl(launches, a.inline_destuff ? k1_fused<64, true> : k1_fused<64, false>, dim3(a.total_ctas), dim3(T), smem,
+                                    stream, a, max_iters); }
         case 128: { const size_t smem = sizeof(K1Smem<128>) + a.lut_smem_bytes; if (smem > 48 * 1024) return cudaErrorInvalidValue;
-                    return LaunchPdl(launches, k1_fused<128>, dim3(a.total_ctas), dim3(T), smem, stream, a, max_iters); }
+                    return LaunchPdl(launches, a.inline_destuff ? k1_fused<128, true> : k1_fused<128, false>, dim3(a.total_ctas), dim3(T), smem,
+                                    stream, a, max_iters); }
         default: return cudaErrorInvalidValue;
     }
 }
@@ -1333,9 +1476,12 @@ cudaError_t PreloadK1() {
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_write<128>);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_write<64>);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_write<32>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<128>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<64>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<32>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<128, false>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<128, true>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<64, false>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<64, true>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<32, false>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_fused<32, true>);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, k1_scan);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, dc_sums);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&at, dc_scan);

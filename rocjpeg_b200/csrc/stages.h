@@ -122,6 +122,7 @@ struct K1Args {
     const uint32_t* img_cta0;     // device, nimages + 1 entries: first K1 CTA of each image
     const uint32_t* img_dctile0;  // device, nimages + 1 entries: first DC tile of each image
     const uint8_t* scan;          // device scan arena
+    const uint8_t* raw;           // device raw arena (inline_destuff: the subsequences are staged from here)
     const HuffLutSet* luts;       // device
     uint32_t* state;              // per subsequence: packed out-state | blocks << 16
     uint32_t* used;               // per subsequence: key of the in-state its state was decoded from
@@ -150,6 +151,8 @@ struct K1Args {
     uint32_t rec_fill_vecs;       // 16-byte vectors of blk_rec that round 0 of k1_sync fills with 0xFF ("never decoded")
     int halo;                     // threads of a CTA that re-decode the subsequences before the CTA's own
     int k1_dc;                    // k1_fused integrates the DC differences itself: LaunchDcScan is not needed after it
+    int inline_destuff;           // k1_fused destuffs the raw bytes itself (no K0 ran): every picture is one restart interval
+                                  // whose data end where the caller's buffer ends in FF D9 (k1_huffman.cu: StageInline)
 };
 
 // Speculative decode + CTA-local synchronisation (round 0) or cross-CTA fix-up (round >= 1).
